@@ -213,6 +213,26 @@ def headline_config(T, V, n_total, chunk):
             "the 1.5 MB mesh is re-read per view by design" % (V * 28 * RES * RES / 1e9)}
 
 
+DUMP_SAMPLE_PIXELS = 1 << 19
+
+
+def dump_outputs(out_dir, z, col, nrm):
+    """--dump-outputs: the buffers the timed render_views steps left for their caller (z [V,H,W], colour and normals
+    [V,H,W,3], float32) as .npy files, so that two builds can be compared output for output.  The whole batch is 3.7 GB at
+    V = 128, so what is written is view 0 in full (<name>_view0.npy, 29 MB) and the same pixels of every view at
+    DUMP_SAMPLE_PIXELS flat indices into [V,H,W] drawn without replacement by numpy's default_rng(0), in ascending order
+    (<name>_sample.npy, 15 MB).  Only rank 0 writes, and rank 0 renders orbit views 0, N, 2N, ... of the N * V-view orbit
+    (N = ranks, V = --views): dumps compare output for output when they were taken with the same N and V."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = z.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_SAMPLE_PIXELS, n), replace=False))
+    didx = torch.from_numpy(idx).to(z.device)
+    for name, t in (("z", z), ("color", col), ("normals", nrm)):
+        np.save(os.path.join(out_dir, f"{name}_view0.npy"), t[0].cpu().numpy())
+        np.save(os.path.join(out_dir, f"{name}_sample.npy"), t.reshape(n, -1)[didx].squeeze(-1).cpu().numpy())
+
+
 def sample_view_indices(n_total, count=8):
     """Views k * n_total / count: an evenly spread sample of the orbit (frames of different view angles cost differently)."""
     return [(k * n_total) // count for k in range(count)]
@@ -360,6 +380,8 @@ def run_gpu_arm(args):
         clocks.sample_now()      # the GPU is still inside the timed steps here (launches are asynchronous)
         barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, z, col, nrm)
     k_launches, k_ms = f.profile_read()
     f.profile(False)
     launches = f.launch_count - launches0
@@ -949,7 +971,7 @@ def measure_workload(args, workload, world, rank, local, dev, cpu_threads=None, 
         torch.cuda.synchronize()
 
     f.clear(); f.render_arrays(dv, dc, dn); f.device_buffers()       # sizes the workspace, checks the pair list
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     for _ in range(3):
         step()
     barrier()
@@ -1180,7 +1202,15 @@ def main():
                          "rank 0's frame over NVLink (sharding.PeerFrame), and the value is frames/s complete on rank 0")
     ap.add_argument("--budget-s", type=float, default=float(os.environ.get("CRB_BENCH_BUDGET_S", "720")),
                     help="watchdog: leave (rank 0 printing the headline it has) after this many seconds; 0 = off")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one rendered (z, colour, normals: view 0 whole and a seeded "
+                         "pixel sample of all views) as float32 .npy files into DIR; rank 0 writes its own views, so compare "
+                         "dumps taken with the same number of ranks and --views")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "trex_1024_orbit"):
+        ap.error("--dump-outputs applies to the headline run (--impl b200, --workload trex_1024_orbit)")
     if args.budget_s > 0:
         start_watchdog(args.budget_s)
     if args.impl == "reference":

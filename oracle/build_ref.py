@@ -3,7 +3,7 @@
 TEST / BASELINE INFRASTRUCTURE ONLY -- nothing in the product package imports this.
 
 What it does (SURVEY.md section 8c recipe, BASELINE.md section 3 step 1):
-  * reads the reference tree where it lies (default /root/reference, read-only),
+  * reads the reference tree where it lies (the argument, else CRB_REFERENCE_SRC; read-only),
   * mirrors the `crender` package (+ the `objects/` assets the README flow needs) into the git-ignored
     build directory oracle/_ref/ -- a build output, never committed,
   * applies the two BUILD-ONLY changes the reference needs to compile with gcc:
@@ -48,11 +48,13 @@ def built(dst=DST):
             and any(n.startswith("math_utils.") and n.endswith(".so") for n in names))
 
 
-def build(src="/root/reference", dst=DST, force=False):
+def build(src=None, dst=DST, force=False):
+    """src: a checkout of the reference (default: the CRB_REFERENCE_SRC environment variable)."""
     if built(dst) and not force:
         return dst
-    if not os.path.isdir(os.path.join(src, "crender")):
-        raise FileNotFoundError(f"reference tree not found at {src}")
+    src = src or os.environ.get("CRB_REFERENCE_SRC")
+    if not src or not os.path.isdir(os.path.join(src, "crender")):
+        raise FileNotFoundError(f"no reference checkout at {src!r} (pass its path or set CRB_REFERENCE_SRC)")
     if os.path.isdir(dst):
         shutil.rmtree(dst)
     os.makedirs(dst)
@@ -82,4 +84,5 @@ def build(src="/root/reference", dst=DST, force=False):
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv))
+    paths = [a for a in sys.argv[1:] if a != "--force"]      # usage: build_ref.py [REFERENCE_CHECKOUT] [--force]
+    print(build(paths[0] if paths else None, force="--force" in sys.argv))

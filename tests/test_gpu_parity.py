@@ -11,6 +11,10 @@ from conftest import GOLDEN, TriModel, bits_equal, case_model, random_scene
 
 pytestmark = pytest.mark.gpu
 CHECKS = json.load(open(os.path.join(GOLDEN, "checksums.json")))
+def seeded(key):
+    """What the reference computed on the seeded inputs below (tests/golden/make_golden_seeded.py)."""
+    with open(os.path.join(GOLDEN, "seeded_checksums.json")) as fh:
+        return json.load(fh)[key]
 
 
 def sha(a):
@@ -783,77 +787,81 @@ def test_deferred_join_batches_match_joined_batches(Filler, trex):
     assert int((z < 1e5).sum()) > 100 and torch.equal(o2["z"].view(torch.int32), want[0]["z"].view(torch.int32))
 
 
-def test_reference_renderer_flow_with_the_drop_in_filler(Filler, trex, capfd):
-    """The run.py flow (run.py:20-26) with the reference's OWN Renderer and GuroIllumination classes driving this filler
-    (crender/cy/renderer.py:42-49: render_model, in-place illumination on the live views, get_color_buffer), next to
-    the same flow on the reference's own Cython filler: the images written by cv2.imwrite would be byte-identical."""
+def flow_sums(image, filler):
+    """Checksums of what run.py takes from one Renderer.render: the lit colour buffer, the uint8 image cv2.imwrite would
+    write (run.py:26), and the filler's normals and depth."""
+    z = filler.get_z_buffer()
+    return {"covered": int((z < 1e5).sum()), "image": sha(image), "u8": sha(image[::-1].astype("uint8")),
+            "normals": sha(filler.get_normals_buffer()), "z": sha(z)}
+
+
+def _reference_flow_classes():
+    """The reference's own Renderer / illumination / filler / iterator classes where oracle/_ref is present, else None."""
     from oracle import build_ref
     if not build_ref.built():
-        pytest.skip("oracle/_ref (reference Cython build) not present")
+        return None
     import sys
     from conftest import ROOT
     ref = os.path.join(ROOT, "oracle", "_ref")
     if ref not in sys.path:
         sys.path.insert(0, ref)
     from crender.cy import Renderer
-    from crender.cy.illumination import GuroIllumination
-    from crender.cy.pixel_buffer_filler import AdvancedPixelBufferFiller as RefFiller
+    from crender.cy.illumination import GuroIllumination, NoIllumination
+    from crender.cy.pixel_buffer_filler import AdvancedPixelBufferFiller
     from crender.cy.triangle_iterator import SimpleIterator
+    return Renderer, GuroIllumination, NoIllumination, AdvancedPixelBufferFiller, SimpleIterator
+
+
+def test_reference_renderer_flow_with_the_drop_in_filler(Filler, trex, capfd):
+    """The run.py flow (run.py:20-26) driving this filler, against the reference flow's buffers (tests/golden/
+    make_golden_seeded.py): with this package's Renderer and GuroIllumination, and -- where oracle/_ref is present -- with
+    the reference's OWN Renderer and GuroIllumination classes (crender/cy/renderer.py:42-49: render_model, in-place
+    illumination on the live views, get_color_buffer), next to the same flow on the reference's own Cython filler."""
+    import cython3dmodelrenderer_b200 as P
     h = w = 256
-    images = []
-    for cls in (RefFiller, Filler):
-        filler = cls(h, w, fov=45, n_threads=1)
-        renderer = Renderer(filler, GuroIllumination(np.array([0, 0, 1], dtype="float32")), SimpleIterator, h, w)
-        image = renderer.render(trex)
-        images.append((np.array(image, copy=True), image[::-1].astype("uint8"),
-                       filler.get_normals_buffer().copy(), filler.get_z_buffer().copy()))
-    capfd.readouterr()
-    (ri, ru8, rn, rz), (gi, gu8, gn, gz) = images
-    assert int((rz < 1e5).sum()) > 5000
-    assert bits_equal(gz, rz) and bits_equal(gn, rn)
-    assert bits_equal(gi, ri), "lit colour buffer differs from the reference flow"
-    assert np.array_equal(gu8, ru8)
+    light = np.array([0, 0, 1], dtype="float32")
+    flows = [(Filler, P.Renderer, P.GuroIllumination, None)]
+    ref = _reference_flow_classes()
+    if ref is not None:
+        RefRenderer, RefGuro, _, RefFiller, SimpleIterator = ref
+        flows += [(RefFiller, RefRenderer, RefGuro, SimpleIterator), (Filler, RefRenderer, RefGuro, SimpleIterator)]
+    for fcls, rcls, ill, it in flows:
+        filler = fcls(h, w, fov=45, n_threads=1)
+        image = rcls(filler, ill(light), it, h, w).render(trex)
+        capfd.readouterr()
+        got = flow_sums(image, filler)
+        assert got["covered"] > 5000
+        assert got == seeded("renderer_flow_trex_256x256_guro"), f"{fcls.__module__}.{rcls.__name__}: differs from the reference flow"
 
 
 def test_drop_in_renderer_and_illumination_match_the_reference_flow(Filler, trex, bunny, capfd):
-    """run.py:20-26 three ways -- the reference's own classes on its own Cython filler; the reference's Renderer driving this
-    package's filler AND GuroIllumination (draw_illumination recognises the filler's live views and lights the device buffers);
-    this package's Renderer + GuroIllumination + filler -- over two render() calls on the same filler (the second composites
-    onto the lit frame and lights the whole buffer again, renderer.py:47-49): bit-identical images, normals and depth."""
-    from oracle import build_ref
-    if not build_ref.built():
-        pytest.skip("oracle/_ref (reference Cython build) not present")
-    import sys
-    from conftest import ROOT
-    ref = os.path.join(ROOT, "oracle", "_ref")
-    if ref not in sys.path:
-        sys.path.insert(0, ref)
+    """run.py:20-26 over two render() calls on the same filler (the second composites onto the lit frame and lights the whole
+    buffer again, renderer.py:47-49), against the reference flow's buffers (tests/golden/make_golden_seeded.py): this package's
+    Renderer + GuroIllumination + filler, and -- where oracle/_ref is present -- the reference's own classes on its own
+    Cython filler and the reference's Renderer driving this package's filler AND GuroIllumination (draw_illumination
+    recognises the filler's live views and lights the device buffers): bit-identical images, normals and depth."""
     import cython3dmodelrenderer_b200 as P
-    from crender.cy import Renderer as RefRenderer
-    from crender.cy.illumination import GuroIllumination as RefGuro, NoIllumination as RefNone
-    from crender.cy.pixel_buffer_filler import AdvancedPixelBufferFiller as RefFiller
-    from crender.cy.triangle_iterator import SimpleIterator
     h, w = 320, 256
     light = [0.3, -0.2, 1.0]
-    for ref_ill, our_ill in ((lambda: RefGuro(light), lambda: P.GuroIllumination(light)), (RefNone, P.NoIllumination)):
-        results = []
-        for fcls, rcls, ill in ((RefFiller, RefRenderer, ref_ill), (Filler, RefRenderer, our_ill), (Filler, P.Renderer, our_ill)):
+    ref = _reference_flow_classes()
+    for kind, our_ill in (("guro", lambda: P.GuroIllumination(light)), ("none", P.NoIllumination)):
+        flows = [(Filler, P.Renderer, our_ill, None)]
+        if ref is not None:
+            RefRenderer, RefGuro, RefNone, RefFiller, SimpleIterator = ref
+            ref_ill = (lambda: RefGuro(light)) if kind == "guro" else RefNone
+            flows += [(RefFiller, RefRenderer, ref_ill, SimpleIterator), (Filler, RefRenderer, our_ill, SimpleIterator)]
+        for fcls, rcls, ill, it in flows:
             filler = fcls(h, w, fov=45, n_threads=1)
-            renderer = rcls(filler, ill(), SimpleIterator, h, w)
-            frames = []
-            for m in (trex, bunny):
+            renderer = rcls(filler, ill(), it, h, w)
+            for k, m in enumerate((trex, bunny)):
                 image = renderer.render(m)
                 if fcls is Filler:
                     assert image is filler.get_color_buffer()      # the live view, the same object every time
-                frames.append((image.copy(), image[::-1].astype("uint8"), filler.get_normals_buffer().copy(), filler.get_z_buffer().copy()))
-            results.append(frames)
-        capfd.readouterr()
-        for other in results[1:]:
-            for (ri, ru8, rn, rz), (gi, gu8, gn, gz) in zip(results[0], other):
-                assert int((rz < 1e5).sum()) > 5000
-                assert bits_equal(gz, rz) and bits_equal(gn, rn)
-                assert bits_equal(gi, ri), "lit colour buffer differs from the reference flow"
-                assert np.array_equal(gu8, ru8)
+                capfd.readouterr()
+                got = flow_sums(image, filler)
+                assert got["covered"] > 5000
+                assert got == seeded("renderer_flow_trex_bunny_320x256")[kind][k], \
+                    f"{kind}, render {k}, {fcls.__module__}.{rcls.__name__}: differs from the reference flow"
     # arrays that are not the live views of a filler of this package: no NumPy path here
     with pytest.raises(TypeError):
         P.GuroIllumination(light).draw_illumination(np.zeros((h, w, 3), np.float32), np.zeros((h, w, 3), np.float32))

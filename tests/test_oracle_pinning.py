@@ -14,10 +14,37 @@ from oracle import build_ref
 from oracle import oracle as O
 
 CHECKS = json.load(open(os.path.join(GOLDEN, "checksums.json")))
+def seeded(key):
+    """What the reference computed on the seeded inputs below (tests/golden/make_golden_seeded.py)."""
+    with open(os.path.join(GOLDEN, "seeded_checksums.json")) as fh:
+        return json.load(fh)[key]
 
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def buffer_sums(f):
+    z = f.get_z_buffer()
+    return {"covered": int((z < 1e5).sum()), "z": sha(z), "color": sha(f.get_color_buffer()),
+            "normals": sha(f.get_normals_buffer())}
+
+
+def random_scene_case(seed):
+    """(h, w, fov, model, passes) of a seeded random scene; passes = 2 composites a second render into the same buffers."""
+    rng = np.random.default_rng(1000 + seed)
+    h, w, fov = int(rng.integers(8, 200)), int(rng.integers(8, 200)), float(rng.uniform(20, 120))
+    return h, w, fov, random_scene(seed), 2 if seed % 3 == 0 else 1
+
+
+def out_of_range_model():
+    """Coordinates far outside int range after projection: exercises the (int)ceil() behaviour of the compiled reference."""
+    v = np.array([[[-3e9, -0.5, 1.0], [3e9, 0.5, 1.0], [0.0, 4e9, 1.0]],
+                  [[-0.5, -0.5, 1.0], [0.5, -0.5, 1.0], [0.0, 3e12, 2.0]],
+                  [[-0.4, -0.4, 1.5], [0.4, -0.4, 1.5], [0.0, 0.4, 1.5]]], dtype=np.float32)
+    n = -np.ones((3, 3, 3), np.float32)
+    c = np.full((3, 3, 3), 100, np.float32)
+    return TriModel(v, c, n)
 
 
 def test_fixture_inputs_match_reference_checksums(trex, bunny, basketball):
@@ -150,10 +177,9 @@ def test_guro_oracle_matches_numpy_formula():
     assert bits_equal(got, want)
 
 
-# ---- against the reference's own compiled code, where it is present (build container / shipped oracle/_ref) ----
+# ---- against the reference's own compiled code: its results on seeded inputs (tests/golden/make_golden_seeded.py), and the
+# build itself wherever oracle/_ref is present (CRB_REFERENCE_SRC at build time, or oracle/build_ref.py) ----
 def _ref_filler_cls():
-    if not build_ref.built():
-        pytest.skip("oracle/_ref (reference Cython build) not present")
     ref = os.path.join(ROOT, "oracle", "_ref")
     if ref not in sys.path:
         sys.path.insert(0, ref)
@@ -163,14 +189,16 @@ def _ref_filler_cls():
 
 @pytest.mark.parametrize("seed", range(24))
 def test_oracle_equals_reference_build_on_random_scenes(seed, capfd):
-    Ref = _ref_filler_cls()
-    rng = np.random.default_rng(1000 + seed)
-    h, w, fov = int(rng.integers(8, 200)), int(rng.integers(8, 200)), float(rng.uniform(20, 120))
-    m = random_scene(seed)
-    r, o = Ref(h, w, fov=fov, n_threads=1), O.OracleFiller(h, w, fov=fov)
-    for _ in range(2 if seed % 3 == 0 else 1):   # second pass composites into the same buffers
-        r.render_model(m)
+    h, w, fov, m, passes = random_scene_case(seed)
+    o = O.OracleFiller(h, w, fov=fov)
+    for _ in range(passes):
         o.render_model(m)
+    assert buffer_sums(o) == seeded("random_scenes")[str(seed)]
+    if not build_ref.built():
+        return
+    r = _ref_filler_cls()(h, w, fov=fov, n_threads=1)
+    for _ in range(passes):
+        r.render_model(m)
     capfd.readouterr()   # the reference printf()s per thread
     assert bits_equal(r.get_z_buffer(), o.get_z_buffer())
     assert bits_equal(r.get_color_buffer(), o.get_color_buffer())
@@ -178,17 +206,15 @@ def test_oracle_equals_reference_build_on_random_scenes(seed, capfd):
 
 
 def test_oracle_equals_reference_build_out_of_range_coordinates(capfd):
-    Ref = _ref_filler_cls()
-    # coordinates far outside int range after projection: exercises the (int)ceil() behaviour of the compiled reference
-    v = np.array([[[-3e9, -0.5, 1.0], [3e9, 0.5, 1.0], [0.0, 4e9, 1.0]],
-                  [[-0.5, -0.5, 1.0], [0.5, -0.5, 1.0], [0.0, 3e12, 2.0]],
-                  [[-0.4, -0.4, 1.5], [0.4, -0.4, 1.5], [0.0, 0.4, 1.5]]], dtype=np.float32)
-    n = -np.ones((3, 3, 3), np.float32)
-    c = np.full((3, 3, 3), 100, np.float32)
-    m = TriModel(v, c, n)
-    r, o = Ref(64, 64, fov=90.0, n_threads=1), O.OracleFiller(64, 64, fov=90.0)
-    r.render_model(m)
+    m = out_of_range_model()
+    o = O.OracleFiller(64, 64, fov=90.0)
     o.render_model(m)
-    capfd.readouterr()
     assert (o.get_z_buffer() < 1e5).sum() > 0
+    want = seeded("out_of_range")
+    assert (sha(o.get_z_buffer()), sha(o.get_color_buffer())) == (want["z"], want["color"])
+    if not build_ref.built():
+        return
+    r = _ref_filler_cls()(64, 64, fov=90.0, n_threads=1)
+    r.render_model(m)
+    capfd.readouterr()
     assert bits_equal(r.get_z_buffer(), o.get_z_buffer()) and bits_equal(r.get_color_buffer(), o.get_color_buffer())
