@@ -315,8 +315,13 @@ __device__ __forceinline__ float background_color(const Frame &)
     return 0.0f;
 }
 
-// run.py:26 .astype('uint8'): C truncation toward zero, then the low 8 bits.
-__device__ __forceinline__ unsigned char to_u8(float c) { return (unsigned char)(int)c; }
+// run.py:26 .astype('uint8'): C truncation toward zero, then the low 8 bits.  NumPy on x86-64 truncates with cvttss2si, which
+// yields INT_MIN (low byte 0) for NaN and for anything outside int range; CUDA's cvt.rzi saturates instead (3e9 and +inf would
+// give 255), so the range test is explicit, as in ceil_to_int_ref.
+__device__ __forceinline__ unsigned char to_u8(float c)
+{
+    return (unsigned char)(c >= -2147483648.0f && c < 2147483648.0f ? (int)c : INT_MIN);
+}
 
 // Address of pixel (x, image row yl of the band's buffers) of view `view` in the flipped uint8 image (run.py:26 image[::-1]):
 // the caller's [views,rows,W,3] array, or -- row exchange -- the receive buffer of the rank that owns the image row.
