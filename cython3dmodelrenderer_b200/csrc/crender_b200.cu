@@ -153,6 +153,10 @@ struct Frame {
     unsigned char *u8x[CRB_MAX_EXCHANGE];
     int u8xN, u8xRows;
     float light[3];
+    // per-pixel texturing (CRB_TEXTURE): packed texels B | G << 8 | R << 16, [texH, texW] (crb_pack_texture / crb_bind_texture);
+    // `c` then holds (u, v, ignored) per corner.  Kept last so that every other member keeps its offset.
+    const uint32_t *tex;
+    int texH, texW;
 };
 
 // ------------------------------------------------------------------------------------------------------------
@@ -274,9 +278,21 @@ __device__ __forceinline__ bool fdiv_ok(float n1, float n2, float n3)
     return fminf(fminf(a1, a2), a3) >= FDIV_LO && fmaxf(fmaxf(a1, a2), a3) <= FDIV_HI;   // NaN: false
 }
 
+// astype('int32') of a float32 on x86-64 (cvttss2si): INT32_MIN for NaN and out-of-range values -- the conversion of
+// model.py:147-150's texel rule (ingest_b200.cu's k_vertex_colors states it the same way).
+__device__ __forceinline__ int f32_to_i32_x86(float x)
+{
+    if (!(x > -2147483904.0f && x < 2147483648.0f)) return INT_MIN;
+    return (int)x;
+}
+
 // pyx:215-242 for the pixel's winning triangle: barycentrics (mu:5-34), depth, colour, normal (left-associated sums).
 // Returns false if the fragment would not have been drawn (some barycentric < 0, NaN depth) -- cannot happen for a key
 // that won, kept as a guard.  All operands come from the triangle's 128-byte shade record.
+// TEX (per-pixel texturing, CRB_TEXTURE; an extension, DESIGN 2): the interpolated colour slots hold (u, v); the texel they
+// name under model.py:147-150's rule replaces the colour before the fused Guro pass.  Compiled in only where asked for, so
+// the per-vertex instantiations are the code they were.
+template <bool TEX = false>
 __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, float px, float py, float &z, float c[3], float n[3])
 {
     const float4 A = R[S_A], B = R[S_B], C = R[S_C];
@@ -295,6 +311,12 @@ __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, 
     c[0] = (X.y * b1 + C1.x * b2) + C1.w * b3;
     c[1] = (X.z * b1 + C1.y * b2) + C2.x * b3;
     c[2] = (X.w * b1 + C1.z * b2) + C2.y * b3;
+    if (TEX) {   // row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1); BGR as cv2.imread gives it
+        const int row = clipi(f32_to_i32_x86((1.0f - c[1]) * (float)F.texH), 0, F.texH - 1);
+        const int col = clipi(f32_to_i32_x86(c[0] * (float)F.texW), 0, F.texW - 1);
+        const uint32_t t = __ldg(F.tex + (row * F.texW + col));     // th * tw < 2^31 (crb_bind_texture)
+        c[0] = (float)(t & 255u); c[1] = (float)((t >> 8) & 255u); c[2] = (float)(t >> 16);
+    }
     if (F.flags & CRB_GURO) {  // guro_illumination.py:23-27 (float32, left-to-right sums)
         // np.sum accumulates from the identity +0.0 (all -0.0 products sum to +0.0, not -0.0)
         const float dot = (__fadd_rn(0.0f, n[0] * F.light[0]) + n[1] * F.light[1]) + n[2] * F.light[2];
@@ -1138,7 +1160,7 @@ constexpr unsigned PK_FAST = 16u;    // FL_SPAN and FL_FDIV: div_rn_by() applies
 constexpr int PK_XA = 8, PK_XB = 14, PK_YT = 20;   // tile-relative rectangle: first x (6 bits), end x (6 bits), first row (5 bits)
 
 // Visibility + deferred shading of one busy tile (n triangles staged at list offset off).
-template <class C>
+template <class C, bool TEX>
 __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, TileSmem<C> &S_, const bool clear, const int view,
                                             const int tx, const int ty, const unsigned n, const unsigned off, const int rowLo, const int rowHi)
 {
@@ -1400,7 +1422,7 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
         if (key != KEY_EMPTY && !DBG(F, FLAG_DBG_NOSHADE)) {
             const unsigned tri = ~(unsigned)(key & 0xFFFFFFFFull);
             float fz, fc[3], fn[3];
-            if (shade_fragment(F, recv + (size_t)(DBG(F, FLAG_DBG_ONEREC) ? 0u : tri) * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn)) {
+            if (shade_fragment<TEX>(F, recv + (size_t)(DBG(F, FLAG_DBG_ONEREC) ? 0u : tri) * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn)) {
                 const float zold = clear ? Z_INIT : F.z[pix];
                 if (!(fz > zold)) {  // pyx:223: drawn unless new_z > z_buffer (equal depth overwrites)
                     z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
@@ -1492,7 +1514,7 @@ __device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C>
 #ifndef CRB_RASTER_MIN_CTAS
 #define CRB_RASTER_MIN_CTAS 8
 #endif
-template <class C>
+template <class C, bool TEX>
 __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, const __grid_constant__ TMaps M)
 {
     constexpr int RT = C::RT, CLEAR_ROWS = C::CLEAR_ROWS;
@@ -1571,7 +1593,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
             __syncthreads();
         }
         if (cta + stride < nb) rec = lst[cta + stride];     // the next tile's record arrives while this one is rasterized
-        raster_tile(F, M, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
+        raster_tile<C, TEX>(F, M, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
                     (int)(cur.w & 255u), (int)(cur.w >> 8));
     }
 #ifdef CRB_PHASE_TIMING
@@ -1654,6 +1676,7 @@ __global__ void __launch_bounds__(NT) k_raster_atomic(const Frame F, unsigned lo
     }
 }
 
+template <bool TEX>
 __global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned long long *keybuf)
 {
     const long long pix = (long long)blockIdx.x * NT + threadIdx.x;
@@ -1667,7 +1690,7 @@ __global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned lon
         const unsigned tri = ~(unsigned)(key & 0xFFFFFFFFull);
         const int y = F.row0 + (int)(pix / F.W), x = (int)(pix % F.W);
         float fz, fc[3], fn[3];
-        if (shade_fragment(F, F.shrec + (size_t)tri * SREC, (float)x, (float)y, fz, fc, fn)) {
+        if (shade_fragment<TEX>(F, F.shrec + (size_t)tri * SREC, (float)x, (float)y, fz, fc, fn)) {
             const float zold = clear ? Z_INIT : F.z[pix];
             if (!(fz > zold)) {
                 z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
@@ -1687,6 +1710,15 @@ __global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned lon
 __global__ void __launch_bounds__(NT) k_fill_u64(unsigned long long *p, long long n, unsigned long long v)
 {
     for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < n; i += (long long)gridDim.x * NT) p[i] = v;
+}
+
+// crb_pack_texture: uint8 [texels,3] (BGR) -> uint32 B | G << 8 | R << 16, so that a textured pixel reads its texel with one
+// aligned 4-byte load instead of three byte loads
+__global__ void __launch_bounds__(NT) k_pack_texture(const uint8_t *__restrict__ bgr, long long texels, uint32_t *__restrict__ out)
+{
+    const long long stride = (long long)gridDim.x * NT;
+    for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < texels; i += stride)
+        out[i] = (uint32_t)bgr[3 * i] | ((uint32_t)bgr[3 * i + 1] << 8) | ((uint32_t)bgr[3 * i + 2] << 16);
 }
 
 // pyx:65-67
@@ -1963,6 +1995,8 @@ struct crb_filler {
     int wide_kernel;       // triangles that span many tiles are scattered by k_fill_wide (CRB_OPT_WIDE_KERNEL = 0: by k_fill itself)
     unsigned char *u8x[CRB_MAX_EXCHANGE];   // crb_set_u8_exchange: receive buffer of every row band (u8x_n == 0: off)
     int u8x_n, u8x_rows;
+    const uint32_t *tex;   // crb_bind_texture: packed texels (caller-owned device memory), NULL = none
+    int tex_h, tex_w;
 };
 
 namespace {
@@ -2070,6 +2104,16 @@ void fill_frame(const crb_filler *f, Frame *F, int set = 0)
     F->hstats = f->hstats_dev;
     F->pairCap = f->pairCap;
     F->slabPixels = (long long)(f->row1 - f->row0) * f->w;
+    F->tex = f->tex;
+    F->texH = f->tex_h;
+    F->texW = f->tex_w;
+}
+
+// CRB_TEXTURE needs a bound texture
+int check_texture(const crb_filler *f, unsigned flags)
+{
+    if ((flags & CRB_TEXTURE) && !f->tex) return fail(CRB_ERR_STATE, "CRB_TEXTURE: no texture bound (crb_bind_texture)");
+    return CRB_OK;
 }
 
 int launch_check(crb_filler *f, const char *name)
@@ -2259,9 +2303,17 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     long long gR = gL + gH;
     if (M.use) gR = (long long)CE * ((gR + CE - 2) / (CE - 1));     // CE - 1 rasterizing CTAs + one clear CTA per group of CE (see k_raster)
     if (prof) CU(cudaEventRecord(f->prof_ev[2 * f->prof_n], st));
-    if (shape == 2) k_raster<RasterSmall><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
-    else if (shape == 3) k_raster<RasterWide><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
-    else k_raster<RasterLarge><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
+    const bool tex = (F.flags & CRB_TEXTURE) != 0;     // per-pixel texturing: the TEX instantiation of the same shape
+    if (shape == 2) {
+        if (tex) k_raster<RasterSmall, true><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
+        else k_raster<RasterSmall, false><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
+    } else if (shape == 3) {
+        if (tex) k_raster<RasterWide, true><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
+        else k_raster<RasterWide, false><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
+    } else {
+        if (tex) k_raster<RasterLarge, true><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
+        else k_raster<RasterLarge, false><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
+    }
     if ((rc = launch_check(f, "k_raster"))) return rc;
     if (prof) {
         CU(cudaEventRecord(f->prof_ev[2 * f->prof_n + 1], st));
@@ -2296,7 +2348,8 @@ int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
         k_raster_atomic<<<(unsigned)((F.T * 32 + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
     }
-    k_shade_atomic<<<(unsigned)((F.slabPixels + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
+    if (F.flags & CRB_TEXTURE) k_shade_atomic<true><<<(unsigned)((F.slabPixels + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
+    else k_shade_atomic<false><<<(unsigned)((F.slabPixels + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
     return launch_check(f, "k_shade_atomic");
 }
 
@@ -2677,15 +2730,38 @@ int crb_render(crb_filler *f, const float *v, const float *c, const float *n, in
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (!f->z || !f->color || !f->normals) return fail(CRB_ERR_STATE, "buffers not bound");
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     CU(cudaSetDevice(f->device));
     { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
     if ((long long)(f->row1 - f->row0) * f->w == 0) return CRB_OK;
     Frame F;
     fill_frame(f, &F);
-    F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC);
+    F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEXTURE);
     F.v = v; F.c = c; F.n = n;
     F.z = f->z; F.color = f->color; F.normals = f->normals;
     return (flags & CRB_PATH_ATOMIC) ? run_atomic(f, F, (cudaStream_t)stream) : run_tiled(f, F, (cudaStream_t)stream);
+}
+
+int crb_pack_texture(const uint8_t *bgr, int th, int tw, uint32_t *out, void *stream)
+{
+    if (!bgr || !out || th < 1 || tw < 1 || (long long)th * tw >= (1ll << 31))
+        return fail(CRB_ERR_INVALID, "crb_pack_texture: bad argument (NULL pointer, or th, tw < 1, or th * tw >= 2^31)");
+    const long long texels = (long long)th * tw;
+    k_pack_texture<<<(unsigned)min((texels + NT - 1) / NT, 4096ll), NT, 0, (cudaStream_t)stream>>>(bgr, texels, out);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(CRB_ERR_CUDA, "launch of k_pack_texture failed: %s", cudaGetErrorString(e));
+    return CRB_OK;
+}
+
+int crb_bind_texture(crb_filler *f, const uint32_t *texels, int th, int tw)
+{
+    if (check_filler(f)) return CRB_ERR_INVALID;
+    if (!texels) { f->tex = nullptr; f->tex_h = f->tex_w = 0; return CRB_OK; }
+    if (th < 1 || tw < 1 || (long long)th * tw >= (1ll << 31))
+        return fail(CRB_ERR_INVALID, "crb_bind_texture: th, tw must be >= 1 with th * tw < 2^31 (got %d x %d)", th, tw);
+    if (reinterpret_cast<uintptr_t>(texels) & 3u) return fail(CRB_ERR_INVALID, "crb_bind_texture: texels must be 4-byte aligned");
+    f->tex = texels; f->tex_h = th; f->tex_w = tw;
+    return CRB_OK;
 }
 
 // H2D of the three [T,3,3] arrays into the filler's staging area.
@@ -2805,6 +2881,7 @@ static int render_host_once(crb_filler *f, const float *v, const float *c, const
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     CU(cudaSetDevice(f->device));
     { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
     cudaStream_t st = (cudaStream_t)stream;
@@ -2935,6 +3012,7 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
     if (n_views > 0 && !views && n_views != 1) return fail(CRB_ERR_INVALID, "views is NULL (allowed for one untransformed view only)");
     if (flags & CRB_PATH_ATOMIC) return fail(CRB_ERR_INVALID, "CRB_PATH_ATOMIC supports single-view renders only");
     if ((flags & CRB_GURO) && !light) return fail(CRB_ERR_INVALID, "CRB_GURO needs a light direction");
+    { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     if ((reinterpret_cast<uintptr_t>(z_out) | reinterpret_cast<uintptr_t>(color_out) | reinterpret_cast<uintptr_t>(normals_out)) & 15u)
         return fail(CRB_ERR_INVALID, "output slabs must be 16-byte aligned");
     if (f->u8x_n && color_u8_out) return fail(CRB_ERR_INVALID, "color_u8_out must be NULL while a row exchange is set (crb_set_u8_exchange)");
@@ -2964,7 +3042,7 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
         Frame F;
         fill_frame(f, &F, set);
         F.T = T; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
-        F.flags = (flags & CRB_GURO) | CRB_CLEAR_FIRST;
+        F.flags = (flags & (CRB_GURO | CRB_TEXTURE)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;
         F.views = views ? views + (size_t)v0 * 16 : nullptr;
         F.z = z_out ? z_out + (size_t)v0 * slab : nullptr;
@@ -3025,6 +3103,7 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
     if (check_filler(f)) return CRB_ERR_INVALID;
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
     if (!image_dev || !image_host) return fail(CRB_ERR_INVALID, "NULL image buffer");
+    { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     CU(cudaSetDevice(f->device));
     cudaStream_t st = (cudaStream_t)stream;
     { int jrc = join_pending(f, st); if (jrc) return jrc; }
@@ -3032,7 +3111,7 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
     if (rc) return rc;
     // one untransformed view, no float32 output: the rasterizer writes the flipped uint8 image itself
     rc = crb_render_views(f, f->stage_v, f->stage_c, f->stage_n, T, nullptr, 1, nullptr, nullptr, nullptr, image_dev,
-                          flags & CRB_GURO, light, stream);
+                          flags & (CRB_GURO | CRB_TEXTURE), light, stream);
     if (rc) return rc;
     const size_t bytes = (size_t)(f->row1 - f->row0) * f->w * 3;
     if (bytes) CU(cudaMemcpyAsync(image_host, image_dev, bytes, cudaMemcpyDeviceToHost, st));

@@ -22,6 +22,19 @@ def _require_cuda():
     return torch
 
 
+def _check_texture(texture):
+    """A texture for per-pixel texturing: uint8 [h,w,3] (what cv2.imread returns, BGR), as NumPy array or torch tensor."""
+    import torch
+    if isinstance(texture, torch.Tensor):
+        ok = texture.dtype == torch.uint8 and texture.dim() == 3 and texture.shape[2] == 3
+    else:
+        texture = np.asarray(texture)
+        ok = texture.dtype == np.uint8 and texture.ndim == 3 and texture.shape[2] == 3
+    if not ok or texture.shape[0] < 1 or texture.shape[1] < 1:
+        raise ValueError("texture must be a uint8 [h,w,3] image (what cv2.imread returns)")
+    return texture
+
+
 def _check_tri_array(a, name):
     """Same acceptance rules as the reference's `float[:, :, :]` memoryviews (pyx:94-96)."""
     if a is None:
@@ -107,6 +120,8 @@ class AdvancedPixelBufferFiller:
     `band=(row0,row1)` -- own only those rows of the h x w image (screen-band sharding), `out_ptrs=(z, color, normals)` --
     raw device addresses of existing [rows,w], [rows,w,3], [rows,w,3] float32 buffers to render into instead of buffers of
     its own (e.g. this band's rows inside another rank's frame, sharding.PeerFrame); their content is taken as it is.
+    `texturing="pixel"` -- render_model samples the model's texture at every pixel (per-pixel texturing, DESIGN 2) instead
+    of blending the colours upstream looks up at the vertices ("vertex", the default and upstream's behaviour).
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -117,7 +132,13 @@ class AdvancedPixelBufferFiller:
     _fetched_by_current = set()
     _view_owner = {}      # address of a host mirror handed out by get_*_buffer() -> weak reference to its filler (owner_of_views)
 
-    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None):
+    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None,
+                 texturing="vertex"):
+        if texturing not in ("vertex", "pixel"):
+            raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
+        self._texturing = texturing
+        self._tex = None              # (source texture, its version, packed uint32 [th,tw] CUDA tensor) bound to the filler
+        self._uv = None               # (texture coordinates, their triangle indices, UV-by-triangle CUDA tensor [T,3,3])
         torch = _require_cuda()
         self._torch = torch
         self._L = _lib.load_library()
@@ -309,12 +330,88 @@ class AdvancedPixelBufferFiller:
         ([T,3,3] float32), never mutates them, composites into the persistent buffers.  (`prefetch=False`, not in the
         reference: do not start downloading the buffers the previous frame's caller fetched -- renderer.Renderer lights the
         colour buffer on the device first.)"""
+        if self._texturing == "pixel":
+            return self._render_model_textured(model, prefetch)
         v = _check_tri_array(getattr(model, "_vertices_by_triangles"), "vertices")
         c = _check_tri_array(getattr(model, "_colors_by_triangles"), "colors")
         n = _check_tri_array(getattr(model, "_normals_by_triangles"), "normals")
         if not (v.shape[0] == c.shape[0] == n.shape[0]):
             raise IndexError("Out of bounds on buffer access (axis 0)")   # what the bounds-checked memoryviews raise
         self.render_arrays(v, c, n, prefetch=prefetch)
+
+    def _render_model_textured(self, model, prefetch):
+        """render_model with texturing="pixel": vertices and normals by triangle as upstream, and -- in place of the colours --
+        the texture coordinates by triangle, gathered on the device, with the model's texture bound.  Both are made once per
+        model (cached on the identity of `_texture_coords`, `_triangles_texture_coords` and `_texture`, which Model never
+        changes), so a render loop over one model uploads neither again."""
+        torch = self._torch
+        v = _check_tri_array(getattr(model, "_vertices_by_triangles"), "vertices")
+        n = _check_tri_array(getattr(model, "_normals_by_triangles"), "normals")
+        tex = getattr(model, "_texture", None)
+        vt = getattr(model, "_texture_coords", None)
+        tri = getattr(model, "_triangles_texture_coords", None)
+        if tex is None or vt is None or tri is None:
+            raise ValueError('texturing="pixel" needs a textured model (_texture, _texture_coords and _triangles_texture_coords); '
+                             'this one has none')
+        u = self._uv
+        if u is None or u[0] is not vt or u[1] is not tri:
+            from .model import _wrap_indices
+            a = np.asarray(vt, dtype=np.float32)
+            if a.ndim != 2 or a.shape[1] < 2:
+                raise ValueError(f"texture coordinates must be [n,2] or [n,3], got {tuple(a.shape)}")
+            idx = _wrap_indices(tri, a.shape[0])
+            if idx.size == 0:
+                idx = idx.reshape(0, 3)
+            if idx.ndim != 2 or idx.shape[1] != 3:
+                raise ValueError(f"texture coordinate indices must be [T,3], got {tuple(idx.shape)}")
+            with torch.cuda.device(self._dev):
+                d_vt = torch.from_numpy(np.ascontiguousarray(a[:, :2])).to(self._dev)
+                d_vt = torch.nn.functional.pad(d_vt, (0, 1)).contiguous()       # [n,2] -> [n,3]: (u, v, 0)
+                d_idx = torch.from_numpy(idx).to(self._dev)
+                uv = torch.empty((idx.shape[0], 3, 3), dtype=torch.float32, device=self._dev)
+                check(self._L.crb_model_gather(d_vt.data_ptr(), d_idx.data_ptr(), idx.shape[0], uv.data_ptr(), self._stream()))
+            self._uv = u = (vt, tri, uv)
+        if not (v.shape[0] == u[2].shape[0] == n.shape[0]):
+            raise IndexError("Out of bounds on buffer access (axis 0)")
+        self.render_arrays(v, u[2], n, prefetch=prefetch, texture=tex)
+
+    def _bind_texture(self, texture):
+        """Packs (crb_pack_texture) and binds (crb_bind_texture) `texture`, unless it is what is bound already: the same NumPy
+        array object, or the same torch tensor unchanged since (its version counter)."""
+        torch = self._torch
+        texture = _check_texture(texture)
+        version = texture._version if isinstance(texture, torch.Tensor) else None
+        t = self._tex
+        if t is not None and t[0] is texture and t[1] == version:
+            return
+        self._validate()       # the previous frame may have to be drawn again, with the texture it was drawn with
+        check(self._L.crb_join(self._handle, self._stream()))      # work in flight on the filler's streams reads the old one
+        th, tw = int(texture.shape[0]), int(texture.shape[1])
+        with torch.cuda.device(self._dev):
+            if isinstance(texture, torch.Tensor):
+                d_bgr = texture.to(self._dev).contiguous()
+            else:
+                d_bgr = torch.from_numpy(np.ascontiguousarray(texture)).to(self._dev)
+            packed = torch.empty((th, tw), dtype=torch.int32, device=self._dev)
+            check(self._L.crb_pack_texture(d_bgr.data_ptr(), th, tw, packed.data_ptr(), self._stream()))
+        check(self._L.crb_bind_texture(self._handle, packed.data_ptr(), th, tw))
+        self._tex = (texture, version, packed)
+
+    def _uv_array(self, c, on_device):
+        """Texture coordinates by triangle, [T,3,3] (third component ignored) or [T,3,2] float32 -> [T,3,3]."""
+        torch = self._torch
+        if isinstance(c, torch.Tensor):
+            if c.dtype != torch.float32 or c.dim() != 3 or tuple(c.shape[1:]) not in ((3, 3), (3, 2)):
+                raise ValueError("texture coordinates must be float32 [T,3,3] or [T,3,2]")
+            if c.shape[2] == 2:
+                c = torch.nn.functional.pad(c, (0, 1))
+            return c.to(self._dev).contiguous() if on_device else c.cpu().numpy()
+        c = np.asarray(c)
+        if c.dtype != np.float32 or c.ndim != 3 or c.shape[1:] not in ((3, 3), (3, 2)):
+            raise ValueError("texture coordinates must be float32 [T,3,3] or [T,3,2]")
+        if c.shape[2] == 2:
+            c = np.concatenate([c, np.zeros(c.shape[:2] + (1,), np.float32)], axis=2)
+        return torch.from_numpy(np.ascontiguousarray(c)).to(self._dev) if on_device else c
 
     def get_normals_buffer(self):
         """pyx:246-247 -- live float32 [h,w,3] view (same array object on every call)."""
@@ -339,11 +436,21 @@ class AdvancedPixelBufferFiller:
             self._stale[name] = True
         self._exposed.clear()   # arrays handed out earlier are detached until fetched again
 
-    def render_arrays(self, v, c, n, path="tiled", check_status=True, prefetch=True):
+    def render_arrays(self, v, c, n, path="tiled", check_status=True, prefetch=True, texture=None):
         """Render [T,3,3] float32 arrays.  numpy inputs are staged through pinned memory and copied H2D;
-        torch CUDA tensors are used in place (device-resident inputs)."""
+        torch CUDA tensors are used in place (device-resident inputs).  `texture` (uint8 [h,w,3], BGR; NumPy or torch):
+        per-pixel texturing -- `c` then holds texture coordinates by triangle, [T,3,3] (third component ignored) or
+        [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE)."""
         torch = self._torch
         flags = _lib.CRB_PATH_ATOMIC if path == "atomic" else 0
+        if texture is not None:
+            texture = _check_texture(texture)
+            # one residence for all three: on the device if any of them is a CUDA tensor
+            on_device = any(isinstance(a, torch.Tensor) and a.is_cuda for a in (v, c, n))
+            c = self._uv_array(c, on_device)
+            if on_device:
+                v, n = (a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a)).to(self._dev) for a in (v, n))
+            flags |= _lib.CRB_TEXTURE
         on_device = all(isinstance(a, torch.Tensor) for a in (v, c, n))
         if on_device:
             for a in (v, c, n):
@@ -358,6 +465,8 @@ class AdvancedPixelBufferFiller:
             v, c, n = (np.asarray(a) for a in (v, c, n))
             T = v.shape[0]
         self._validate()                 # an earlier frame this one composites onto must have been drawn
+        if texture is not None:
+            self._bind_texture(texture)
         if self._pending_clear:
             flags |= _lib.CRB_CLEAR_FIRST
         else:
@@ -459,7 +568,7 @@ class AdvancedPixelBufferFiller:
 
     def render_views(self, v, c, n, views, z_out=None, color_out=None, normals_out=None, color_u8_out=None,
                      want=("z", "color", "normals"), guro_light=None, chunk=32, check_status=True, defer_join=False,
-                     u8_exchange=None):
+                     u8_exchange=None, texture=None):
         """Batched multi-view render (config C5): every view gets fresh-filler buffers in its own slab.
 
         v, c, n: torch CUDA float32 [T,3,3] (device-resident base mesh);  views: [V,16] float32 (numpy or CUDA tensor,
@@ -471,8 +580,13 @@ class AdvancedPixelBufferFiller:
         `u8_exchange=(rows_per_band, [address, ...])` (sharding.RowExchange.plan): the flipped uint8 images leave the
         rasterizer row band by row band straight into the listed receive buffers (other GPUs' memory) instead of a
         local array -- the view-sharded render and its delivery in one kernel (crb_set_u8_exchange).
+        `texture` (uint8 [h,w,3], BGR): per-pixel texturing -- `c` holds texture coordinates by triangle, [T,3,3] or
+        [T,3,2], host or CUDA (see render_arrays).
         Returns a dict of the produced tensors."""
         torch = self._torch
+        if texture is not None:
+            texture = _check_texture(texture)
+            c = self._uv_array(c, True)
         for a in (v, c, n):
             if not isinstance(a, torch.Tensor) or not a.is_cuda or a.dtype != torch.float32 or tuple(a.shape[1:]) != (3, 3):
                 raise ValueError("render_views needs CUDA float32 tensors of shape [T,3,3]")
@@ -501,6 +615,9 @@ class AdvancedPixelBufferFiller:
         if color_u8_out is not None:
             out["color_u8"] = color_u8_out
         flags, light = 0, None
+        if texture is not None:
+            self._bind_texture(texture)
+            flags |= _lib.CRB_TEXTURE
         if guro_light is not None:
             # GuroIllumination.__init__ (guro_illumination.py:17-18): negate, then normalise, in float32
             l = -np.asarray(guro_light, dtype="float32")

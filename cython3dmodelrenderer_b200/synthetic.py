@@ -38,3 +38,17 @@ def uv_sphere(n_lon=3200, n_lat=1564, center=(0.0, 0.0, 1.5), radius=0.5):
     v = (n * np.float32(radius) + np.asarray(center, dtype=np.float32)).astype(np.float32)
     col = (np.float32(127.5) * (n + np.float32(1.0))).astype(np.float32)
     return ArrayModel(v, col, n)
+
+
+def spherical_uvs(v, center=None):
+    """Texture coordinates by triangle, float32 [T,3,2], from a spherical projection of the corners `v` ([T,3,3]) about
+    `center` (default: the mean corner): u = 0.5 + atan2(z, x) / 2pi (longitude), v = 0.5 + asin(y / r) / pi (latitude).
+    For uv_sphere these are its latitude-longitude coordinates.  For per-pixel texturing (`texture=` of the filler's
+    render_arrays / render_views) of meshes that come without texture coordinates."""
+    v = np.asarray(v, dtype=np.float64)
+    c = v.reshape(-1, 3).mean(axis=0) if center is None else np.asarray(center, dtype=np.float64)
+    d = v - c
+    r = np.linalg.norm(d, axis=-1)
+    u = 0.5 + np.arctan2(d[..., 2], d[..., 0]) / (2.0 * np.pi)
+    w = 0.5 + np.arcsin(np.clip(d[..., 1] / np.where(r > 0, r, 1.0), -1.0, 1.0)) / np.pi
+    return np.ascontiguousarray(np.stack([u, w], axis=-1), dtype=np.float32)

@@ -69,6 +69,12 @@ extern "C" {
                                   then copied (at the granularity of 32-pixel tile rows), by a kernel writing into the pinned + mapped host arrays; the arrays end up
                                   bit-identical to a full download.  The arrays must come from cudaHostAlloc /
                                   cudaHostRegister (e.g. torch pin_memory). */
+#define CRB_TEXTURE 1024u      /* per-pixel texturing (every render entry point; an extension, the reference textures vertices only):
+                                  `c` holds texture coordinates (u, v, ignored) per corner instead of colours.  They are interpolated
+                                  like colours, and the winning fragment's colour is the texel of the texture bound with
+                                  crb_bind_texture at row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1)
+                                  (float32, int32 as x86-64 converts: NaN and out-of-range give INT32_MIN) -- model.py:147-150's
+                                  rule -- as float BGR, lit afterwards by CRB_GURO.  Without a bound texture: CRB_ERR_STATE. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u
@@ -142,6 +148,17 @@ int crb_device_buffers(const crb_filler *f, float **z, float **color, float **no
 
 /* z = 1e6, colour = 0, normals = 0 (pyx:65-67), asynchronous on `stream`. */
 int crb_init_buffers(crb_filler *f, void *stream);
+
+/* ---- per-pixel texturing (CRB_TEXTURE) ----------------------------------------------------------------------- */
+
+/* bgr: DEVICE uint8 [th,tw,3] (cv2.imread's layout) -> out: DEVICE uint32 [th,tw], texel = B | G << 8 | R << 16, on the current
+ * device, asynchronous on `stream`.  CRB_ERR_INVALID for NULL pointers, th or tw < 1, or th * tw >= 2^31. */
+int crb_pack_texture(const uint8_t *bgr, int th, int tw, uint32_t *out, void *stream);
+
+/* Binds packed texels (crb_pack_texture; caller-owned DEVICE memory that must outlive the renders using it, like
+ * crb_bind_buffers) as the texture of CRB_TEXTURE renders.  texels = NULL unbinds.  CRB_ERR_INVALID for th or tw < 1,
+ * th * tw >= 2^31, or a pointer that is not 4-byte aligned. */
+int crb_bind_texture(crb_filler *f, const uint32_t *texels, int th, int tw);
 
 /* ---- render_model: pyx:92-104 -> project (pyx:106-130) + cull/bbox/raster/z-test/writes (pyx:177-244) ------- */
 

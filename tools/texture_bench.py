@@ -1,0 +1,161 @@
+"""Per-pixel texturing (CRB_TEXTURE) against per-vertex colours: frames/s and k_raster time of both modes on two workloads,
+alternated, in one process.  Prints one JSON line (GPU name and power limit read in the same run).
+
+  trex_1024_orbit  the headline workload of bench.py: T-Rex (tests/golden/trex_fit.npz) at 1024^2, batches of 128 orbit views
+                   rendered by render_views into float32 z / colour / normals slabs.  The fixture has no texture coordinates:
+                   seeded spherical-projection ones (synthetic.spherical_uvs) and a seeded 709 x 709 texture.
+  sphere_8192      the 10 M-triangle synthetic.uv_sphere, one frame at 8192^2 (render_arrays, device-resident inputs, fused
+                   clear): its latitude-longitude coordinates and a seeded 4096 x 2048 texture.
+
+Each round times both modes back to back (order alternating between rounds); the report gives the median and the spread
+(min, max) over the rounds.  `k_raster_ms` is the tile rasterizer's device time per step (crb_profile: CUDA events around
+each launch), `step_ms` the whole step (CUDA events).
+
+    python tools/texture_bench.py [--rounds 7] [--steps 20] [--out FILE]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def gpu_info(torch):
+    info = {"gpu": torch.cuda.get_device_name(0)}
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+        info["power_limit"], info["clocks_max_sm"] = [s.strip() for s in q.split(",")][:2]
+    except Exception as e:      # (reported, not fatal: the numbers still stand with the card's name)
+        info["power_limit"] = f"unavailable: {e}"
+    return info
+
+
+def timed(torch, f, step, steps):
+    torch.cuda.synchronize()
+    f.profile(True)
+    f.profile_read()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(steps):
+        step()
+    e1.record()
+    torch.cuda.synchronize()
+    launches, k_ms = f.profile_read()
+    f.profile(False)
+    return e0.elapsed_time(e1) / steps, k_ms / steps, launches
+
+
+def summary(xs):
+    xs = sorted(xs)
+    return {"median": float(np.median(xs)), "min": float(xs[0]), "max": float(xs[-1]), "n": len(xs)}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--rounds", type=int, default=7)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps per mode and round (headline); the sphere runs steps/4 + 1")
+    ap.add_argument("--views", type=int, default=128)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("texture_bench needs a CUDA device")
+    from cython3dmodelrenderer_b200 import AdvancedPixelBufferFiller, synthetic, views as VW
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from conftest import load_indexed
+    dev = torch.device("cuda", 0)
+    result = {"tool": "tools/texture_bench.py", **gpu_info(torch), "rounds": args.rounds, "workloads": {}}
+
+    # ---- headline: T-Rex 1024^2, 128 orbit views per step
+    m = load_indexed("trex")
+    T = int(m._vertices_by_triangles.shape[0])
+    uv = synthetic.spherical_uvs(m._vertices_by_triangles)
+    tex = np.random.default_rng(709).integers(0, 256, (709, 709, 3), dtype=np.uint8)
+    V, RES = args.views, 1024
+    dv, dc, dn = (torch.from_numpy(a).to(dev) for a in (m._vertices_by_triangles, m._colors_by_triangles, m._normals_by_triangles))
+    duv = torch.nn.functional.pad(torch.from_numpy(uv).to(dev), (0, 1)).contiguous()
+    dviews = torch.from_numpy(VW.orbit_views(V, count=V)).to(dev)
+    z = torch.empty((V, RES, RES), dtype=torch.float32, device=dev)
+    col = torch.empty((V, RES, RES, 3), dtype=torch.float32, device=dev)
+    nrm = torch.empty((V, RES, RES, 3), dtype=torch.float32, device=dev)
+    fill = {mode: AdvancedPixelBufferFiller(RES, RES, fov=45.0, device=0) for mode in ("vertex", "pixel")}
+
+    def trex_step(mode):
+        f = fill[mode]
+        kw = {"texture": tex} if mode == "pixel" else {}
+        c = duv if mode == "pixel" else dc
+        return lambda: f.render_views(dv, c, dn, dviews, z_out=z, color_out=col, normals_out=nrm, chunk=V, check_status=False,
+                                      **kw)
+    for mode in fill:     # workspace, status check, texture upload, warm-up
+        fill[mode].render_views(dv, duv if mode == "pixel" else dc, dn, dviews, z_out=z, color_out=col, normals_out=nrm, chunk=V,
+                                **({"texture": tex} if mode == "pixel" else {}))
+        for _ in range(3):
+            trex_step(mode)()
+    rows = {mode: {"fps": [], "step_ms": [], "k_raster_ms": []} for mode in fill}
+    for r in range(args.rounds):
+        for mode in (("vertex", "pixel") if r % 2 == 0 else ("pixel", "vertex")):
+            step_ms, k_ms, _ = timed(torch, fill[mode], trex_step(mode), args.steps)
+            rows[mode]["fps"].append(V / (step_ms / 1e3))
+            rows[mode]["step_ms"].append(step_ms)
+            rows[mode]["k_raster_ms"].append(k_ms)
+    result["workloads"]["trex_1024_orbit"] = {
+        "triangles": T, "views_per_step": V, "resolution": RES, "texture": [709, 709], "steps": args.steps,
+        **{mode: {k: summary(v) for k, v in rows[mode].items()} for mode in rows},
+        "pixel_over_vertex_k_raster": float(np.median(rows["pixel"]["k_raster_ms"]) / np.median(rows["vertex"]["k_raster_ms"])),
+        "pixel_over_vertex_fps": float(np.median(rows["pixel"]["fps"]) / np.median(rows["vertex"]["fps"]))}
+    del z, col, nrm, fill
+    torch.cuda.empty_cache()
+
+    # ---- 10 M-triangle sphere at 8192^2, one frame per step
+    s = synthetic.uv_sphere(3200, 1564)
+    T = int(s._vertices_by_triangles.shape[0])
+    suv = synthetic.spherical_uvs(s._vertices_by_triangles, center=(0.0, 0.0, 1.5))
+    stex = np.random.default_rng(4096).integers(0, 256, (2048, 4096, 3), dtype=np.uint8)
+    sv, sc, sn = (torch.from_numpy(a).to(dev) for a in (s._vertices_by_triangles, s._colors_by_triangles, s._normals_by_triangles))
+    suvd = torch.nn.functional.pad(torch.from_numpy(suv).to(dev), (0, 1)).contiguous()
+    del s, suv
+    RES = 8192
+    fs = AdvancedPixelBufferFiller(RES, RES, fov=45.0, device=0)
+
+    def sphere_step(mode):
+        def step():
+            fs.clear()
+            if mode == "pixel":
+                fs.render_arrays(sv, suvd, sn, check_status=False, texture=stex)
+            else:
+                fs.render_arrays(sv, sc, sn, check_status=False)
+        return step
+    for mode in ("vertex", "pixel"):
+        fs.clear()
+        fs.render_arrays(sv, suvd if mode == "pixel" else sc, sn, **({"texture": stex} if mode == "pixel" else {}))
+        fs.get_z_buffer()         # status checked (the pair list fits)
+        for _ in range(2):
+            sphere_step(mode)()
+    srows = {mode: {"fps": [], "step_ms": [], "k_raster_ms": []} for mode in ("vertex", "pixel")}
+    ssteps = args.steps // 4 + 1
+    for r in range(args.rounds):
+        for mode in (("vertex", "pixel") if r % 2 == 0 else ("pixel", "vertex")):
+            step_ms, k_ms, _ = timed(torch, fs, sphere_step(mode), ssteps)
+            srows[mode]["fps"].append(1e3 / step_ms)
+            srows[mode]["step_ms"].append(step_ms)
+            srows[mode]["k_raster_ms"].append(k_ms)
+    result["workloads"]["sphere_8192"] = {
+        "triangles": T, "resolution": RES, "texture": [2048, 4096], "steps": ssteps,
+        **{mode: {k: summary(v) for k, v in srows[mode].items()} for mode in srows},
+        "pixel_over_vertex_k_raster": float(np.median(srows["pixel"]["k_raster_ms"]) / np.median(srows["vertex"]["k_raster_ms"])),
+        "pixel_over_vertex_fps": float(np.median(srows["pixel"]["fps"]) / np.median(srows["vertex"]["fps"]))}
+    line = json.dumps(result)
+    print(line)
+    if args.out:
+        with open(args.out, "w") as fh:
+            fh.write(line + "\n")
+
+
+if __name__ == "__main__":
+    main()
