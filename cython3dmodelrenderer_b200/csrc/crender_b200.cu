@@ -57,6 +57,7 @@ constexpr unsigned FLAG_DBG_ONEREC = 0x100000u;   // ablation: every pixel shade
 constexpr unsigned FLAG_DBG_NOCLEAR = 0x10000u, FLAG_DBG_NOSHADE = 0x20000u, FLAG_DBG_NOROWS = 0x40000u, FLAG_DBG_NOOUT = 0x80000u;  // ablation switches (CRB_DEBUG_SKIP)
 constexpr unsigned FLAG_OUT_DIRECT = 0x200u;   // experiment: shaded pixels stored straight from registers (12-byte strided stores)
 constexpr unsigned FLAG_OUT_TMA = 0x100u;   // internal Frame.flags bit: shaded colour / normal rows leave through TMA boxes
+constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR;   // per-pixel texturing and its modes
 #ifndef CRB_CH
 #define CRB_CH 96               // triangles staged in shared memory per pass of the tile rasterizer
 #endif
@@ -98,6 +99,7 @@ static_assert(TW == 32, "a tile row is one warp wide");
 //   prefetched into L1 when a tile stages the triangle):
 //     S_A (x0 y0 x1 y1)  S_B (x2 y2 z0 z1)  S_C (z2 l03 l13 l23)      screen-space vertices + denominators of mu:14,17,20
 //     S_N0 (n0.xyz n1.x)  S_N1 (n1.yz n2.xy)  S_X (n2.z c0.xyz)  S_C1 (c1.xyz c2.x)  S_C2 (c2.yz flags -)
+//                                    (c_k: the colour, or with CRB_TEXTURE (u, v, -), with CRB_TEX_PERSPECTIVE (u*w, v*w, w), w = 1/z)
 //   recE (bbox x, bbox y, local, flags)  packed half-open pixel rectangle of a DRAWN triangle; the entries of a 256-triangle chunk are
 //                                    dense: chunk c of view v has alive[v,c] entries at [v*T + c*256, ...), entry j = triangle
 //                                    c*256 + local (k_fill and the atomic path walk drawn triangles only, with full warps)
@@ -154,7 +156,8 @@ struct Frame {
     int u8xN, u8xRows;
     float light[3];
     // per-pixel texturing (CRB_TEXTURE): packed texels B | G << 8 | R << 16, [texH, texW] (crb_pack_texture / crb_bind_texture);
-    // `c` then holds (u, v, ignored) per corner.  Kept last so that every other member keeps its offset.
+    // `c` then holds (u, v, ignored) per corner (the record's colour slots: the same, or (u/z, v/z, 1/z) with CRB_TEX_PERSPECTIVE).
+    // Kept last so that every other member keeps its offset.
     const uint32_t *tex;
     int texH, texW;
 };
@@ -286,13 +289,50 @@ __device__ __forceinline__ int f32_to_i32_x86(float x)
     return (int)x;
 }
 
+// Shading mode of shade_fragment / k_raster / k_shade_atomic: per-vertex colours (TEX_NONE), or per-pixel texturing
+// (CRB_TEXTURE) with nearest (model.py:147-150's rule) or bilinear (CRB_TEX_BILINEAR) sampling, either of them with
+// TEX_PERSP (CRB_TEX_PERSPECTIVE) added.  All five are compile-time: a uniform branch on the divide costs the nearest
+// instantiation of the large rasterizer shape a register.
+enum TexMode { TEX_NONE = 0, TEX_NEAREST = 1, TEX_BILINEAR = 2, TEX_PERSP = 4 };
+
+// Texel (r, c) of the packed texture as float B, G, R
+__device__ __forceinline__ void texel_bgr(const Frame &F, int r, int c, float t[3])
+{
+    const uint32_t p = __ldg(F.tex + (r * F.texW + c));     // th * tw < 2^31 (crb_bind_texture)
+    t[0] = (float)(p & 255u); t[1] = (float)((p >> 8) & 255u); t[2] = (float)(p >> 16);
+}
+
+// CRB_TEX_BILINEAR (DESIGN 2): texel centres at (col + 0.5) / tw, (row + 0.5) / th -- those of the nearest rule -- clamped to
+// the border texels.  float32, one rounding per operation, no FMA (the file is built with -fmad=false).
+__device__ __forceinline__ void sample_bilinear(const Frame &F, float u, float v, float c[3])
+{
+    const float tw = (float)F.texW, th = (float)F.texH;
+    float sx = u * tw - 0.5f, sy = (1.0f - v) * th - 0.5f;
+    sx = fminf(fmaxf(sx, -1.0f), tw);       // fmaxf(NaN, -1) = -1
+    sy = fminf(fmaxf(sy, -1.0f), th);
+    const float x0 = floorf(sx), y0 = floorf(sy);
+    const float fx = sx - x0, fy = sy - y0, gx = 1.0f - fx, gy = 1.0f - fy;     // (sx - x0 is exact unless -1 < sx < 0)
+    const long long ix = (long long)x0, iy = (long long)y0;                      // in [-1, 2^31]
+    const int c0 = (int)min(max(ix, 0ll), (long long)F.texW - 1), c1 = (int)min(max(ix + 1, 0ll), (long long)F.texW - 1);
+    const int r0 = (int)min(max(iy, 0ll), (long long)F.texH - 1), r1 = (int)min(max(iy + 1, 0ll), (long long)F.texH - 1);
+    float t00[3], t01[3], t10[3], t11[3];
+    texel_bgr(F, r0, c0, t00); texel_bgr(F, r0, c1, t01);
+    texel_bgr(F, r1, c0, t10); texel_bgr(F, r1, c1, t11);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float top = t00[k] * gx + t01[k] * fx, bot = t10[k] * gx + t11[k] * fx;
+        c[k] = top * gy + bot * fy;
+    }
+}
+
 // pyx:215-242 for the pixel's winning triangle: barycentrics (mu:5-34), depth, colour, normal (left-associated sums).
 // Returns false if the fragment would not have been drawn (some barycentric < 0, NaN depth) -- cannot happen for a key
 // that won, kept as a guard.  All operands come from the triangle's 128-byte shade record.
-// TEX (per-pixel texturing, CRB_TEXTURE; an extension, DESIGN 2): the interpolated colour slots hold (u, v); the texel they
-// name under model.py:147-150's rule replaces the colour before the fused Guro pass.  Compiled in only where asked for, so
-// the per-vertex instantiations are the code they were.
-template <bool TEX = false>
+// TEX != TEX_NONE (per-pixel texturing, CRB_TEXTURE; an extension, DESIGN 2): the interpolated colour slots hold (u, v, -), or
+// with CRB_TEX_PERSPECTIVE (U, V, W) = (u/z, v/z, 1/z), divided back to u = U/W, v = V/W; the texel they name (nearest) or
+// the bilinear blend of the four around them replaces the colour before the fused Guro pass.  Compiled in only where asked
+// for, so the per-vertex instantiations are the code they were.
+template <int TEX = TEX_NONE>
 __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, float px, float py, float &z, float c[3], float n[3])
 {
     const float4 A = R[S_A], B = R[S_B], C = R[S_C];
@@ -311,11 +351,16 @@ __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, 
     c[0] = (X.y * b1 + C1.x * b2) + C1.w * b3;
     c[1] = (X.z * b1 + C1.y * b2) + C2.x * b3;
     c[2] = (X.w * b1 + C1.z * b2) + C2.y * b3;
-    if (TEX) {   // row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1); BGR as cv2.imread gives it
-        const int row = clipi(f32_to_i32_x86((1.0f - c[1]) * (float)F.texH), 0, F.texH - 1);
-        const int col = clipi(f32_to_i32_x86(c[0] * (float)F.texW), 0, F.texW - 1);
-        const uint32_t t = __ldg(F.tex + (row * F.texW + col));     // th * tw < 2^31 (crb_bind_texture)
-        c[0] = (float)(t & 255u); c[1] = (float)((t >> 8) & 255u); c[2] = (float)(t >> 16);
+    if (TEX != TEX_NONE) {
+        float u = c[0], v = c[1];
+        if (TEX & TEX_PERSP) { u = c[0] / c[2]; v = c[1] / c[2]; }    // correctly rounded (-prec-div=true)
+        if (TEX & TEX_BILINEAR) {
+            sample_bilinear(F, u, v, c);
+        } else {   // row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1); BGR as cv2.imread gives it
+            const int row = clipi(f32_to_i32_x86((1.0f - v) * (float)F.texH), 0, F.texH - 1);
+            const int col = clipi(f32_to_i32_x86(u * (float)F.texW), 0, F.texW - 1);
+            texel_bgr(F, row, col, c);
+        }
     }
     if (F.flags & CRB_GURO) {  // guro_illumination.py:23-27 (float32, left-to-right sums)
         // np.sum accumulates from the identity +0.0 (all -0.0 products sum to +0.0, not -0.0)
@@ -445,7 +490,9 @@ __device__ __forceinline__ unsigned block_compact(const bool flag, unsigned *wsu
 }
 
 // One chunk of NT consecutive triangles of one view.  Every early exit below is taken by the whole CTA or lies behind
-// the last barrier, so the function can be called in a loop (chunk-list mode).
+// the last barrier, so the function can be called in a loop (chunk-list mode).  PERSP: the colour slots of the record get
+// the perspective-correct texture coordinates of CRB_TEX_PERSPECTIVE.
+template <bool PERSP>
 __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, const long long chunk, const long long chunksPerView,
                                             float *sv, float *sn, float *sc, float *sM, unsigned char *slist, unsigned *wsum,
                                             const bool staged)
@@ -610,9 +657,25 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
     }
     R[S_N0] = make_float4(nx[0], ny[0], nz[0], nx[1]);
     R[S_N1] = make_float4(ny[1], nz[1], nx[2], ny[2]);
-    R[S_X] = make_float4(nz[2], q[0], q[1], q[2]);
-    R[S_C1] = make_float4(q[3], q[4], q[5], q[6]);
-    R[S_C2] = make_float4(q[7], q[8], __uint_as_float(fl), 0.0f);
+    if (PERSP) {
+        // CRB_TEX_PERSPECTIVE (DESIGN 2): per corner (u*w, v*w, w), w = 1 / z with z the camera-space depth project_vertex
+        // divides by -- still in sv; for batched views view_point's z row gives the same bits again
+        float t[9];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const float *p = sv + mi * 9 + k * 3;
+            const float zc = F.views ? ((sM[6] * (p[0] - sM[9]) + sM[7] * (p[1] - sM[10])) + sM[8] * (p[2] - sM[11])) + sM[14] : p[2];
+            const float w = 1.0f / zc;
+            t[3 * k] = q[3 * k] * w; t[3 * k + 1] = q[3 * k + 1] * w; t[3 * k + 2] = w;
+        }
+        R[S_X] = make_float4(nz[2], t[0], t[1], t[2]);
+        R[S_C1] = make_float4(t[3], t[4], t[5], t[6]);
+        R[S_C2] = make_float4(t[7], t[8], __uint_as_float(fl), 0.0f);
+    } else {
+        R[S_X] = make_float4(nz[2], q[0], q[1], q[2]);
+        R[S_C1] = make_float4(q[3], q[4], q[5], q[6]);
+        R[S_C2] = make_float4(q[7], q[8], __uint_as_float(fl), 0.0f);
+    }
     }
     if (F.flags & CRB_PATH_ATOMIC) return;
 
@@ -648,6 +711,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
 constexpr int SETUP_STAGES = 2;
 constexpr size_t SETUP_STAGE_FLOATS = 3 * (size_t)NT * 9;
 constexpr size_t SETUP_DYN_SMEM = SETUP_STAGES * SETUP_STAGE_FLOATS * sizeof(float);
+template <bool PERSP>
 __global__ void __launch_bounds__(NT, CRB_SETUP_MIN_CTAS) k_setup(const Frame F)
 {
     extern __shared__ __align__(128) float stg[];          // [SETUP_STAGES][3][NT * 9]
@@ -698,7 +762,7 @@ __global__ void __launch_bounds__(NT, CRB_SETUP_MIN_CTAS) k_setup(const Frame F)
             uses ^= 1u << s;
         }
         float *d = stg + (size_t)s * SETUP_STAGE_FLOATS;
-        setup_chunk(F, view, chunk, chunksPerView, d, d + NT * 9, d + 2 * NT * 9, sM, slist, wsum, staged);
+        setup_chunk<PERSP>(F, view, chunk, chunksPerView, d, d + NT * 9, d + 2 * NT * 9, sM, slist, wsum, staged);
         __syncthreads();                                // everybody is done with the stage (and with sM / slist / wsum)
         const long long w2 = w + (long long)SETUP_STAGES * gridDim.x;
         if (threadIdx.x == 0 && w2 < nItems) issue(w2, s);
@@ -1160,7 +1224,7 @@ constexpr unsigned PK_FAST = 16u;    // FL_SPAN and FL_FDIV: div_rn_by() applies
 constexpr int PK_XA = 8, PK_XB = 14, PK_YT = 20;   // tile-relative rectangle: first x (6 bits), end x (6 bits), first row (5 bits)
 
 // Visibility + deferred shading of one busy tile (n triangles staged at list offset off).
-template <class C, bool TEX>
+template <class C, int TEX>
 __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, TileSmem<C> &S_, const bool clear, const int view,
                                             const int tx, const int ty, const unsigned n, const unsigned off, const int rowLo, const int rowHi)
 {
@@ -1514,7 +1578,7 @@ __device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C>
 #ifndef CRB_RASTER_MIN_CTAS
 #define CRB_RASTER_MIN_CTAS 8
 #endif
-template <class C, bool TEX>
+template <class C, int TEX>
 __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, const __grid_constant__ TMaps M)
 {
     constexpr int RT = C::RT, CLEAR_ROWS = C::CLEAR_ROWS;
@@ -1676,7 +1740,7 @@ __global__ void __launch_bounds__(NT) k_raster_atomic(const Frame F, unsigned lo
     }
 }
 
-template <bool TEX>
+template <int TEX>
 __global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned long long *keybuf)
 {
     const long long pix = (long long)blockIdx.x * NT + threadIdx.x;
@@ -2109,9 +2173,11 @@ void fill_frame(const crb_filler *f, Frame *F, int set = 0)
     F->texW = f->tex_w;
 }
 
-// CRB_TEXTURE needs a bound texture
+// CRB_TEX_PERSPECTIVE and CRB_TEX_BILINEAR are modes of CRB_TEXTURE, which needs a bound texture
 int check_texture(const crb_filler *f, unsigned flags)
 {
+    if ((flags & (CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR)) && !(flags & CRB_TEXTURE))
+        return fail(CRB_ERR_INVALID, "CRB_TEX_PERSPECTIVE / CRB_TEX_BILINEAR need CRB_TEXTURE");
     if ((flags & CRB_TEXTURE) && !f->tex) return fail(CRB_ERR_STATE, "CRB_TEXTURE: no texture bound (crb_bind_texture)");
     return CRB_OK;
 }
@@ -2174,9 +2240,17 @@ int setup_smem_attr(int device)
 {
     static bool done[64] = {};
     if (device >= 0 && device < 64 && done[device]) return CRB_OK;
-    CU(cudaFuncSetAttribute(k_setup, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
+    CU(cudaFuncSetAttribute(k_setup<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
+    CU(cudaFuncSetAttribute(k_setup<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
     if (device >= 0 && device < 64) done[device] = true;
     return CRB_OK;
+}
+
+// k_setup with `grid` CTAs; CRB_TEX_PERSPECTIVE frames write the perspective-correct texture coordinates into the records
+void launch_setup(const Frame &F, unsigned grid, cudaStream_t st)
+{
+    if (F.flags & CRB_TEX_PERSPECTIVE) k_setup<true><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
+    else k_setup<false><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
 }
 
 #ifndef CRB_PREPASS_EIGHTHS
@@ -2218,7 +2292,7 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
         const long long items = F.chunks ? (long long)gT : (long long)gT * F.nViews;
-        k_setup<<<(unsigned)min(items, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), NT, SETUP_DYN_SMEM, st>>>(F);
+        launch_setup(F, (unsigned)min(items, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
     } else {
         CU(cudaMemsetAsync(F.total, 0, 8, st));
@@ -2242,6 +2316,25 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
 }
 
 // raster + shade (+ fused clear) of the frame run_prep binned
+// shading instantiation of a frame: per-vertex colours, or per-pixel texturing with its filter and interpolation
+int tex_mode(const Frame &F)
+{
+    if (!(F.flags & CRB_TEXTURE)) return TEX_NONE;
+    return ((F.flags & CRB_TEX_BILINEAR) ? TEX_BILINEAR : TEX_NEAREST) | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
+}
+
+template <class C>
+void launch_raster(const Frame &F, const TMaps &M, unsigned grid, cudaStream_t st)
+{
+    switch (tex_mode(F)) {
+    case TEX_NEAREST: k_raster<C, TEX_NEAREST><<<grid, C::RT, 0, st>>>(F, M); break;
+    case TEX_NEAREST | TEX_PERSP: k_raster<C, TEX_NEAREST | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
+    case TEX_BILINEAR: k_raster<C, TEX_BILINEAR><<<grid, C::RT, 0, st>>>(F, M); break;
+    case TEX_BILINEAR | TEX_PERSP: k_raster<C, TEX_BILINEAR | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
+    default: k_raster<C, TEX_NONE><<<grid, C::RT, 0, st>>>(F, M);
+    }
+}
+
 int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
 {
     int rc;
@@ -2303,17 +2396,10 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     long long gR = gL + gH;
     if (M.use) gR = (long long)CE * ((gR + CE - 2) / (CE - 1));     // CE - 1 rasterizing CTAs + one clear CTA per group of CE (see k_raster)
     if (prof) CU(cudaEventRecord(f->prof_ev[2 * f->prof_n], st));
-    const bool tex = (F.flags & CRB_TEXTURE) != 0;     // per-pixel texturing: the TEX instantiation of the same shape
-    if (shape == 2) {
-        if (tex) k_raster<RasterSmall, true><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
-        else k_raster<RasterSmall, false><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
-    } else if (shape == 3) {
-        if (tex) k_raster<RasterWide, true><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
-        else k_raster<RasterWide, false><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
-    } else {
-        if (tex) k_raster<RasterLarge, true><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
-        else k_raster<RasterLarge, false><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
-    }
+    // per-pixel texturing: the instantiation of the same shape with the frame's texture filter
+    if (shape == 2) launch_raster<RasterSmall>(F, M, (unsigned)gR, st);
+    else if (shape == 3) launch_raster<RasterWide>(F, M, (unsigned)gR, st);
+    else launch_raster<RasterLarge>(F, M, (unsigned)gR, st);
     if ((rc = launch_check(f, "k_raster"))) return rc;
     if (prof) {
         CU(cudaEventRecord(f->prof_ev[2 * f->prof_n + 1], st));
@@ -2343,13 +2429,19 @@ int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
     }
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
-        k_setup<<<(unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), NT, SETUP_DYN_SMEM, st>>>(F);
+        launch_setup(F, (unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
         k_raster_atomic<<<(unsigned)((F.T * 32 + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
     }
-    if (F.flags & CRB_TEXTURE) k_shade_atomic<true><<<(unsigned)((F.slabPixels + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
-    else k_shade_atomic<false><<<(unsigned)((F.slabPixels + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
+    const unsigned gS = (unsigned)((F.slabPixels + NT - 1) / NT);
+    switch (tex_mode(F)) {
+    case TEX_NEAREST: k_shade_atomic<TEX_NEAREST><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    case TEX_NEAREST | TEX_PERSP: k_shade_atomic<TEX_NEAREST | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    case TEX_BILINEAR: k_shade_atomic<TEX_BILINEAR><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    case TEX_BILINEAR | TEX_PERSP: k_shade_atomic<TEX_BILINEAR | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    default: k_shade_atomic<TEX_NONE><<<gS, NT, 0, st>>>(F, f->keybuf);
+    }
     return launch_check(f, "k_shade_atomic");
 }
 
@@ -2736,7 +2828,7 @@ int crb_render(crb_filler *f, const float *v, const float *c, const float *n, in
     if ((long long)(f->row1 - f->row0) * f->w == 0) return CRB_OK;
     Frame F;
     fill_frame(f, &F);
-    F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEXTURE);
+    F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEX_FLAGS);
     F.v = v; F.c = c; F.n = n;
     F.z = f->z; F.color = f->color; F.normals = f->normals;
     return (flags & CRB_PATH_ATOMIC) ? run_atomic(f, F, (cudaStream_t)stream) : run_tiled(f, F, (cudaStream_t)stream);
@@ -3042,7 +3134,7 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
         Frame F;
         fill_frame(f, &F, set);
         F.T = T; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
-        F.flags = (flags & (CRB_GURO | CRB_TEXTURE)) | CRB_CLEAR_FIRST;
+        F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;
         F.views = views ? views + (size_t)v0 * 16 : nullptr;
         F.z = z_out ? z_out + (size_t)v0 * slab : nullptr;
@@ -3111,7 +3203,7 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
     if (rc) return rc;
     // one untransformed view, no float32 output: the rasterizer writes the flipped uint8 image itself
     rc = crb_render_views(f, f->stage_v, f->stage_c, f->stage_n, T, nullptr, 1, nullptr, nullptr, nullptr, image_dev,
-                          flags & (CRB_GURO | CRB_TEXTURE), light, stream);
+                          flags & (CRB_GURO | CRB_TEX_FLAGS), light, stream);
     if (rc) return rc;
     const size_t bytes = (size_t)(f->row1 - f->row0) * f->w * 3;
     if (bytes) CU(cudaMemcpyAsync(image_host, image_dev, bytes, cudaMemcpyDeviceToHost, st));

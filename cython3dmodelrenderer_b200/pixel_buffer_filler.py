@@ -122,6 +122,10 @@ class AdvancedPixelBufferFiller:
     its own (e.g. this band's rows inside another rank's frame, sharding.PeerFrame); their content is taken as it is.
     `texturing="pixel"` -- render_model samples the model's texture at every pixel (per-pixel texturing, DESIGN 2) instead
     of blending the colours upstream looks up at the vertices ("vertex", the default and upstream's behaviour).
+    `texture_filter="nearest" | "bilinear"` and `perspective_correct=False | True` -- how every textured render of this filler
+    (render_model with texturing="pixel", render_arrays / render_views with texture=) samples: the nearest texel or a bilinear
+    blend of four (CRB_TEX_BILINEAR), from texture coordinates interpolated affinely in screen space or perspective-correctly
+    (CRB_TEX_PERSPECTIVE).
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -133,10 +137,17 @@ class AdvancedPixelBufferFiller:
     _view_owner = {}      # address of a host mirror handed out by get_*_buffer() -> weak reference to its filler (owner_of_views)
 
     def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None,
-                 texturing="vertex"):
+                 texturing="vertex", texture_filter="nearest", perspective_correct=False):
         if texturing not in ("vertex", "pixel"):
             raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
+        if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear"):
+            raise ValueError(f"texture_filter must be 'nearest' or 'bilinear', got {texture_filter!r}")
+        if not isinstance(perspective_correct, (bool, np.bool_)):
+            raise ValueError(f"perspective_correct must be True or False, got {perspective_correct!r}")
         self._texturing = texturing
+        # render flags of every textured frame (kept in the arguments of a frame, so a redraw of it samples the same way)
+        self._tex_flags = (_lib.CRB_TEXTURE | (_lib.CRB_TEX_BILINEAR if texture_filter == "bilinear" else 0)
+                           | (_lib.CRB_TEX_PERSPECTIVE if perspective_correct else 0))
         self._tex = None              # (source texture, its version, packed uint32 [th,tw] CUDA tensor) bound to the filler
         self._uv = None               # (texture coordinates, their triangle indices, UV-by-triangle CUDA tensor [T,3,3])
         torch = _require_cuda()
@@ -440,7 +451,8 @@ class AdvancedPixelBufferFiller:
         """Render [T,3,3] float32 arrays.  numpy inputs are staged through pinned memory and copied H2D;
         torch CUDA tensors are used in place (device-resident inputs).  `texture` (uint8 [h,w,3], BGR; NumPy or torch):
         per-pixel texturing -- `c` then holds texture coordinates by triangle, [T,3,3] (third component ignored) or
-        [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE)."""
+        [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE), sampled as the constructor's `texture_filter` and
+        `perspective_correct` say."""
         torch = self._torch
         flags = _lib.CRB_PATH_ATOMIC if path == "atomic" else 0
         if texture is not None:
@@ -450,7 +462,7 @@ class AdvancedPixelBufferFiller:
             c = self._uv_array(c, on_device)
             if on_device:
                 v, n = (a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a)).to(self._dev) for a in (v, n))
-            flags |= _lib.CRB_TEXTURE
+            flags |= self._tex_flags
         on_device = all(isinstance(a, torch.Tensor) for a in (v, c, n))
         if on_device:
             for a in (v, c, n):
@@ -617,7 +629,7 @@ class AdvancedPixelBufferFiller:
         flags, light = 0, None
         if texture is not None:
             self._bind_texture(texture)
-            flags |= _lib.CRB_TEXTURE
+            flags |= self._tex_flags
         if guro_light is not None:
             # GuroIllumination.__init__ (guro_illumination.py:17-18): negate, then normalise, in float32
             l = -np.asarray(guro_light, dtype="float32")

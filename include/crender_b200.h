@@ -75,6 +75,17 @@ extern "C" {
                                   crb_bind_texture at row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1)
                                   (float32, int32 as x86-64 converts: NaN and out-of-range give INT32_MIN) -- model.py:147-150's
                                   rule -- as float BGR, lit afterwards by CRB_GURO.  Without a bound texture: CRB_ERR_STATE. */
+#define CRB_TEX_PERSPECTIVE 2048u  /* with CRB_TEXTURE: perspective-correct coordinates.  Per corner w = 1 / z, z the camera-space depth
+                                      the projection divides by (after the view transform for crb_render_views); (u*w, v*w, w) are
+                                      interpolated like colours to (U, V, W), then u = U / W, v = V / W (float32, correctly rounded; no
+                                      clipping: z == 0 or corners on both sides of the camera plane give whatever IEEE gives, and the
+                                      texel rule then maps NaN to row / column 0). */
+#define CRB_TEX_BILINEAR 4096u     /* with CRB_TEXTURE: bilinear filtering instead of the nearest texel (DESIGN 2).  sx = u*tw - 0.5,
+                                      sy = (1 - v)*th - 0.5, each clamped with fmin(fmax(s, -1), tw or th) (NaN -> -1); the four
+                                      texels around (sx, sy), indices clamped to the texture, blended in float32 as
+                                      (t00*gx + t01*fx)*gy + (t10*gx + t11*fx)*fy with fx = sx - floor(sx), gx = 1 - fx (same for y).
+                                      At texel centres this is the nearest texel.  Either mode bit without CRB_TEXTURE: CRB_ERR_INVALID
+                                      on every render entry point. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u

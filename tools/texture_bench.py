@@ -1,5 +1,8 @@
-"""Per-pixel texturing (CRB_TEXTURE) against per-vertex colours: frames/s and k_raster time of both modes on two workloads,
-alternated, in one process.  Prints one JSON line (GPU name and power limit read in the same run).
+"""Per-pixel texturing (CRB_TEXTURE) against per-vertex colours: frames/s and k_raster time of each shading mode on two
+workloads, alternated, in one process.  Prints one JSON line (GPU name and power limit read in the same run).
+
+Modes: "vertex" (per-vertex colours), and per-pixel texturing sampled "nearest" / "bilinear" (CRB_TEX_BILINEAR) from affine
+or, with the suffix "_persp", perspective-correct (CRB_TEX_PERSPECTIVE) coordinates -- five in all.
 
   trex_1024_orbit  the headline workload of bench.py: T-Rex (tests/golden/trex_fit.npz) at 1024^2, batches of 128 orbit views
                    rendered by render_views into float32 z / colour / normals slabs.  The fixture has no texture coordinates:
@@ -7,9 +10,9 @@ alternated, in one process.  Prints one JSON line (GPU name and power limit read
   sphere_8192      the 10 M-triangle synthetic.uv_sphere, one frame at 8192^2 (render_arrays, device-resident inputs, fused
                    clear): its latitude-longitude coordinates and a seeded 4096 x 2048 texture.
 
-Each round times both modes back to back (order alternating between rounds); the report gives the median and the spread
-(min, max) over the rounds.  `k_raster_ms` is the tile rasterizer's device time per step (crb_profile: CUDA events around
-each launch), `step_ms` the whole step (CUDA events).
+Each round times every mode back to back (the order rotates between rounds); the report gives the median and the spread
+(min, max) over the rounds, and each mode's medians over those of "vertex" and of "nearest".  `k_raster_ms` is the tile
+rasterizer's device time per step (crb_profile: CUDA events around each launch), `step_ms` the whole step (CUDA events).
 
     python tools/texture_bench.py [--rounds 7] [--steps 20] [--out FILE]
 """
@@ -56,6 +59,40 @@ def summary(xs):
     return {"median": float(np.median(xs)), "min": float(xs[0]), "max": float(xs[-1]), "n": len(xs)}
 
 
+MODES = {"vertex": None, "nearest": ("nearest", False), "nearest_persp": ("nearest", True), "bilinear": ("bilinear", False),
+         "bilinear_persp": ("bilinear", True)}
+
+
+def make_filler(AdvancedPixelBufferFiller, mode, res):
+    if MODES[mode] is None:
+        return AdvancedPixelBufferFiller(res, res, fov=45.0, device=0)
+    filt, persp = MODES[mode]
+    return AdvancedPixelBufferFiller(res, res, fov=45.0, device=0, texture_filter=filt, perspective_correct=persp)
+
+
+def rounds_of(modes, rounds, run):
+    """`rounds` rounds of every mode, the order rotated by one each round; returns mode -> {fps, step_ms, k_raster_ms} lists."""
+    rows = {mode: {"fps": [], "step_ms": [], "k_raster_ms": []} for mode in modes}
+    for r in range(rounds):
+        k = r % len(modes)
+        for mode in modes[k:] + modes[:k]:
+            fps, step_ms, k_ms = run(mode)
+            rows[mode]["fps"].append(fps)
+            rows[mode]["step_ms"].append(step_ms)
+            rows[mode]["k_raster_ms"].append(k_ms)
+    return rows
+
+
+def report(rows):
+    out = {mode: {k: summary(v) for k, v in rows[mode].items()} for mode in rows}
+    for base in ("vertex", "nearest"):
+        for mode in rows:
+            if mode != base:
+                out[mode][f"over_{base}_k_raster"] = float(np.median(rows[mode]["k_raster_ms"]) / np.median(rows[base]["k_raster_ms"]))
+                out[mode][f"over_{base}_fps"] = float(np.median(rows[mode]["fps"]) / np.median(rows[base]["fps"]))
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=7)
@@ -63,6 +100,7 @@ def main():
     ap.add_argument("--views", type=int, default=128)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
+    modes = list(MODES)
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("texture_bench needs a CUDA device")
@@ -70,7 +108,7 @@ def main():
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from conftest import load_indexed
     dev = torch.device("cuda", 0)
-    result = {"tool": "tools/texture_bench.py", **gpu_info(torch), "rounds": args.rounds, "workloads": {}}
+    result = {"tool": "tools/texture_bench.py", **gpu_info(torch), "rounds": args.rounds, "modes": modes, "workloads": {}}
 
     # ---- headline: T-Rex 1024^2, 128 orbit views per step
     m = load_indexed("trex")
@@ -84,31 +122,26 @@ def main():
     z = torch.empty((V, RES, RES), dtype=torch.float32, device=dev)
     col = torch.empty((V, RES, RES, 3), dtype=torch.float32, device=dev)
     nrm = torch.empty((V, RES, RES, 3), dtype=torch.float32, device=dev)
-    fill = {mode: AdvancedPixelBufferFiller(RES, RES, fov=45.0, device=0) for mode in ("vertex", "pixel")}
+    fill = {mode: make_filler(AdvancedPixelBufferFiller, mode, RES) for mode in modes}
 
     def trex_step(mode):
         f = fill[mode]
-        kw = {"texture": tex} if mode == "pixel" else {}
-        c = duv if mode == "pixel" else dc
+        kw = {"texture": tex} if MODES[mode] else {}
+        c = duv if MODES[mode] else dc
         return lambda: f.render_views(dv, c, dn, dviews, z_out=z, color_out=col, normals_out=nrm, chunk=V, check_status=False,
                                       **kw)
     for mode in fill:     # workspace, status check, texture upload, warm-up
-        fill[mode].render_views(dv, duv if mode == "pixel" else dc, dn, dviews, z_out=z, color_out=col, normals_out=nrm, chunk=V,
-                                **({"texture": tex} if mode == "pixel" else {}))
+        fill[mode].render_views(dv, duv if MODES[mode] else dc, dn, dviews, z_out=z, color_out=col, normals_out=nrm, chunk=V,
+                                **({"texture": tex} if MODES[mode] else {}))
         for _ in range(3):
             trex_step(mode)()
-    rows = {mode: {"fps": [], "step_ms": [], "k_raster_ms": []} for mode in fill}
-    for r in range(args.rounds):
-        for mode in (("vertex", "pixel") if r % 2 == 0 else ("pixel", "vertex")):
-            step_ms, k_ms, _ = timed(torch, fill[mode], trex_step(mode), args.steps)
-            rows[mode]["fps"].append(V / (step_ms / 1e3))
-            rows[mode]["step_ms"].append(step_ms)
-            rows[mode]["k_raster_ms"].append(k_ms)
+
+    def trex_run(mode):
+        step_ms, k_ms, _ = timed(torch, fill[mode], trex_step(mode), args.steps)
+        return V / (step_ms / 1e3), step_ms, k_ms
+    rows = rounds_of(modes, args.rounds, trex_run)
     result["workloads"]["trex_1024_orbit"] = {
-        "triangles": T, "views_per_step": V, "resolution": RES, "texture": [709, 709], "steps": args.steps,
-        **{mode: {k: summary(v) for k, v in rows[mode].items()} for mode in rows},
-        "pixel_over_vertex_k_raster": float(np.median(rows["pixel"]["k_raster_ms"]) / np.median(rows["vertex"]["k_raster_ms"])),
-        "pixel_over_vertex_fps": float(np.median(rows["pixel"]["fps"]) / np.median(rows["vertex"]["fps"]))}
+        "triangles": T, "views_per_step": V, "resolution": RES, "texture": [709, 709], "steps": args.steps, **report(rows)}
     del z, col, nrm, fill
     torch.cuda.empty_cache()
 
@@ -121,35 +154,33 @@ def main():
     suvd = torch.nn.functional.pad(torch.from_numpy(suv).to(dev), (0, 1)).contiguous()
     del s, suv
     RES = 8192
-    fs = AdvancedPixelBufferFiller(RES, RES, fov=45.0, device=0)
+    fills = {mode: make_filler(AdvancedPixelBufferFiller, mode, RES) for mode in modes}
 
     def sphere_step(mode):
+        fs = fills[mode]
+
         def step():
             fs.clear()
-            if mode == "pixel":
+            if MODES[mode]:
                 fs.render_arrays(sv, suvd, sn, check_status=False, texture=stex)
             else:
                 fs.render_arrays(sv, sc, sn, check_status=False)
         return step
-    for mode in ("vertex", "pixel"):
+    for mode in modes:
+        fs = fills[mode]
         fs.clear()
-        fs.render_arrays(sv, suvd if mode == "pixel" else sc, sn, **({"texture": stex} if mode == "pixel" else {}))
+        fs.render_arrays(sv, suvd if MODES[mode] else sc, sn, **({"texture": stex} if MODES[mode] else {}))
         fs.get_z_buffer()         # status checked (the pair list fits)
         for _ in range(2):
             sphere_step(mode)()
-    srows = {mode: {"fps": [], "step_ms": [], "k_raster_ms": []} for mode in ("vertex", "pixel")}
     ssteps = args.steps // 4 + 1
-    for r in range(args.rounds):
-        for mode in (("vertex", "pixel") if r % 2 == 0 else ("pixel", "vertex")):
-            step_ms, k_ms, _ = timed(torch, fs, sphere_step(mode), ssteps)
-            srows[mode]["fps"].append(1e3 / step_ms)
-            srows[mode]["step_ms"].append(step_ms)
-            srows[mode]["k_raster_ms"].append(k_ms)
+
+    def sphere_run(mode):
+        step_ms, k_ms, _ = timed(torch, fills[mode], sphere_step(mode), ssteps)
+        return 1e3 / step_ms, step_ms, k_ms
+    srows = rounds_of(modes, args.rounds, sphere_run)
     result["workloads"]["sphere_8192"] = {
-        "triangles": T, "resolution": RES, "texture": [2048, 4096], "steps": ssteps,
-        **{mode: {k: summary(v) for k, v in srows[mode].items()} for mode in srows},
-        "pixel_over_vertex_k_raster": float(np.median(srows["pixel"]["k_raster_ms"]) / np.median(srows["vertex"]["k_raster_ms"])),
-        "pixel_over_vertex_fps": float(np.median(srows["pixel"]["fps"]) / np.median(srows["vertex"]["fps"]))}
+        "triangles": T, "resolution": RES, "texture": [2048, 4096], "steps": ssteps, **report(srows)}
     line = json.dumps(result)
     print(line)
     if args.out:
