@@ -19,7 +19,7 @@ CRB_OK = 0
 CRB_ERR_INVALID, CRB_ERR_CUDA, CRB_ERR_ZERODIV, CRB_ERR_STATE, CRB_ERR_OVERFLOW = -1, -2, -3, -4, -5
 CRB_ERR_SYNTAX, CRB_ERR_RANGE = -6, -7
 CRB_CLEAR_FIRST, CRB_PATH_ATOMIC, CRB_GURO, CRB_NO_SYNC, CRB_DL_SPARSE, CRB_DEFER_JOIN, CRB_HOST_PAGEABLE, CRB_SYNC_UPLOAD = 1, 2, 4, 8, 16, 32, 64, 128
-CRB_TEXTURE, CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR = 1024, 2048, 4096
+CRB_TEXTURE, CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR, CRB_TEX_TRILINEAR = 1024, 2048, 4096, 8192
 CRB_OPT_CHUNK_PIPELINE, CRB_OPT_TMA, CRB_OPT_TMA_ROWS, CRB_OPT_BAND_PREPASS, CRB_OPT_RASTER_CTAS, CRB_OPT_SPLIT_HEAVY, CRB_OPT_WIDE_KERNEL = 1, 2, 3, 4, 5, 6, 7
 CRB_OPT_RASTER_SHAPE = 8
 CRB_BUF_Z, CRB_BUF_COLOR, CRB_BUF_NORMALS, CRB_BUF_ALL = 1, 2, 4, 7
@@ -79,6 +79,9 @@ SIGNATURES = {
     "crb_profile_read": (_i, [_vp, _ip, ctypes.POINTER(ctypes.c_double)]),
     "crb_pack_texture": (_i, [_vp, _i, _i, _vp, _vp]),
     "crb_bind_texture": (_i, [_vp, _vp, _i, _i]),
+    "crb_mip_layout": (_i, [_i, _i, _ip, _i64p]),
+    "crb_pack_texture_mips": (_i, [_vp, _i, _i, _vp, _vp]),
+    "crb_bind_texture_mips": (_i, [_vp, _vp, _i, _i]),
     # include/crender_ingest_b200.h (model ingest, SURVEY 8f N4)
     "crb_obj_parse": (_i, [ctypes.c_char_p, _sz, _vpp]),
     "crb_obj_free": (None, [_vp]),

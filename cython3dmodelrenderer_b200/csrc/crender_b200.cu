@@ -57,7 +57,7 @@ constexpr unsigned FLAG_DBG_ONEREC = 0x100000u;   // ablation: every pixel shade
 constexpr unsigned FLAG_DBG_NOCLEAR = 0x10000u, FLAG_DBG_NOSHADE = 0x20000u, FLAG_DBG_NOROWS = 0x40000u, FLAG_DBG_NOOUT = 0x80000u;  // ablation switches (CRB_DEBUG_SKIP)
 constexpr unsigned FLAG_OUT_DIRECT = 0x200u;   // experiment: shaded pixels stored straight from registers (12-byte strided stores)
 constexpr unsigned FLAG_OUT_TMA = 0x100u;   // internal Frame.flags bit: shaded colour / normal rows leave through TMA boxes
-constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR;   // per-pixel texturing and its modes
+constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR;   // per-pixel texturing and its modes
 #ifndef CRB_CH
 #define CRB_CH 96               // triangles staged in shared memory per pass of the tile rasterizer
 #endif
@@ -159,6 +159,8 @@ struct Frame {
     // `c` then holds (u, v, ignored) per corner (the record's colour slots: the same, or (u/z, v/z, 1/z) with CRB_TEX_PERSPECTIVE).
     // Kept last so that every other member keeps its offset.
     const uint32_t *tex;
+    // With CRB_TEX_TRILINEAR `tex` is a whole mip chain (crb_bind_texture_mips) of the [texH, texW] texture: its layout follows
+    // from the size alone (mip_step), so the Frame -- every kernel's parameter block -- does not grow.
     int texH, texW;
 };
 
@@ -291,37 +293,78 @@ __device__ __forceinline__ int f32_to_i32_x86(float x)
 
 // Shading mode of shade_fragment / k_raster / k_shade_atomic: per-vertex colours (TEX_NONE), or per-pixel texturing
 // (CRB_TEXTURE) with nearest (model.py:147-150's rule) or bilinear (CRB_TEX_BILINEAR) sampling, either of them with
-// TEX_PERSP (CRB_TEX_PERSPECTIVE) added.  All five are compile-time: a uniform branch on the divide costs the nearest
-// instantiation of the large rasterizer shape a register.
-enum TexMode { TEX_NONE = 0, TEX_NEAREST = 1, TEX_BILINEAR = 2, TEX_PERSP = 4 };
+// TEX_PERSP (CRB_TEX_PERSPECTIVE) added, and trilinear mip filtering (CRB_TEX_TRILINEAR) with or without it.  All are
+// compile-time: a uniform branch on the divide costs the nearest instantiation of the large rasterizer shape a register.
+enum TexMode { TEX_NONE = 0, TEX_NEAREST = 1, TEX_BILINEAR = 2, TEX_PERSP = 4, TEX_TRILINEAR = 8 };
 
-// Texel (r, c) of the packed texture as float B, G, R
-__device__ __forceinline__ void texel_bgr(const Frame &F, int r, int c, float t[3])
+// Texel (r, c) of a packed [th, tw] level as float B, G, R
+__device__ __forceinline__ void texel_bgr(const uint32_t *tex, int tw, int r, int c, float t[3])
 {
-    const uint32_t p = __ldg(F.tex + (r * F.texW + c));     // th * tw < 2^31 (crb_bind_texture)
+    const uint32_t p = __ldg(tex + (r * tw + c));     // th * tw < 2^31 (crb_bind_texture)
     t[0] = (float)(p & 255u); t[1] = (float)((p >> 8) & 255u); t[2] = (float)(p >> 16);
 }
 
 // CRB_TEX_BILINEAR (DESIGN 2): texel centres at (col + 0.5) / tw, (row + 0.5) / th -- those of the nearest rule -- clamped to
 // the border texels.  float32, one rounding per operation, no FMA (the file is built with -fmad=false).
-__device__ __forceinline__ void sample_bilinear(const Frame &F, float u, float v, float c[3])
+__device__ __forceinline__ void sample_bilinear(const uint32_t *tex, int H, int W, float u, float v, float c[3])
 {
-    const float tw = (float)F.texW, th = (float)F.texH;
+    const float tw = (float)W, th = (float)H;
     float sx = u * tw - 0.5f, sy = (1.0f - v) * th - 0.5f;
     sx = fminf(fmaxf(sx, -1.0f), tw);       // fmaxf(NaN, -1) = -1
     sy = fminf(fmaxf(sy, -1.0f), th);
     const float x0 = floorf(sx), y0 = floorf(sy);
     const float fx = sx - x0, fy = sy - y0, gx = 1.0f - fx, gy = 1.0f - fy;     // (sx - x0 is exact unless -1 < sx < 0)
     const long long ix = (long long)x0, iy = (long long)y0;                      // in [-1, 2^31]
-    const int c0 = (int)min(max(ix, 0ll), (long long)F.texW - 1), c1 = (int)min(max(ix + 1, 0ll), (long long)F.texW - 1);
-    const int r0 = (int)min(max(iy, 0ll), (long long)F.texH - 1), r1 = (int)min(max(iy + 1, 0ll), (long long)F.texH - 1);
+    const int c0 = (int)min(max(ix, 0ll), (long long)W - 1), c1 = (int)min(max(ix + 1, 0ll), (long long)W - 1);
+    const int r0 = (int)min(max(iy, 0ll), (long long)H - 1), r1 = (int)min(max(iy + 1, 0ll), (long long)H - 1);
     float t00[3], t01[3], t10[3], t11[3];
-    texel_bgr(F, r0, c0, t00); texel_bgr(F, r0, c1, t01);
-    texel_bgr(F, r1, c0, t10); texel_bgr(F, r1, c1, t11);
+    texel_bgr(tex, W, r0, c0, t00); texel_bgr(tex, W, r0, c1, t01);
+    texel_bgr(tex, W, r1, c0, t10); texel_bgr(tex, W, r1, c1, t11);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
         const float top = t00[k] * gx + t01[k] * fx, bot = t10[k] * gx + t11[k] * fx;
         c[k] = top * gy + bot * fy;
+    }
+}
+
+// CRB_TEX_TRILINEAR (DESIGN 2): level of detail of a pixel from the screen-space derivatives of (u, v) -- ux = du/dx etc. --
+// clamped to the chain: lc = fmin(fmax(0.5 * L2(r2), 0), L-1), r2 = fmax(|(ux*tw, vx*th)|^2, |(uy*tw, vy*th)|^2), with the
+// piecewise-linear log2 L2(f * 2^k) = (k - 1) + (2f - 1), f in [0.5, 1) (frexp; exact at powers of two).  r2 = 0, +inf and NaN
+// give L2 = -2, +inf and NaN here, which clamp to the same lc as the definition's -inf, +inf and NaN.
+__device__ __forceinline__ float mip_lod(const Frame &F, float ux, float vx, float uy, float vy)
+{
+    const float p = ux * (float)F.texW, q = vx * (float)F.texH, r = uy * (float)F.texW, s = vy * (float)F.texH;
+    const float r2 = fmaxf(p * p + q * q, r * r + s * s);
+    int k;
+    const float f = frexpf(r2, &k);
+    const float l2 = (float)(k - 1) + (2.0f * f - 1.0f);
+    return fminf(fmaxf(0.5f * l2, 0.0f), (float)(31 - __clz(max(F.texH, F.texW))));    // L - 1; fmaxf(NaN, 0) = 0
+}
+
+// The next level of a chain from level (p, h, w): levels are stored back to back, each max(1, h >> 1) x max(1, w >> 1)
+__device__ __forceinline__ const uint32_t *mip_step(const uint32_t *p, int &h, int &w)
+{
+    p += h * w;
+    h = max(1, h >> 1); w = max(1, w >> 1);
+    return p;
+}
+
+// CRB_TEX_TRILINEAR: bilinear samples of levels l0 = floor(lc) and l1 = min(l0 + 1, L-1), blended c0*(1 - fr) + c1*fr,
+// fr = lc - l0.  With fr == 0 that is c0 bit for bit (texels are finite and >= 0), so the second level is not read.
+__device__ __forceinline__ void sample_trilinear(const Frame &F, float lc, float u, float v, float c[3])
+{
+    const int l0 = (int)floorf(lc);
+    const float fr = lc - (float)l0;
+    int h = F.texH, w = F.texW;
+    const uint32_t *p = F.tex;
+    for (int l = 0; l < l0; ++l) p = mip_step(p, h, w);
+    sample_bilinear(p, h, w, u, v, c);
+    if (fr != 0.0f) {   // then lc < L-1, so l1 = l0 + 1
+        p = mip_step(p, h, w);
+        float c1[3];
+        sample_bilinear(p, h, w, u, v, c1);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) c[k] = c[k] * (1.0f - fr) + c1[k] * fr;
     }
 }
 
@@ -354,12 +397,24 @@ __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, 
     if (TEX != TEX_NONE) {
         float u = c[0], v = c[1];
         if (TEX & TEX_PERSP) { u = c[0] / c[2]; v = c[1] / c[2]; }    // correctly rounded (-prec-div=true)
-        if (TEX & TEX_BILINEAR) {
-            sample_bilinear(F, u, v, c);
+        if (TEX & TEX_TRILINEAR) {
+            // barycentric gradients: d(b1, b2, b3)/dx = ((y2-y1)/l03, (y0-y2)/l13, (y1-y0)/l23), d/dy = ((x1-x2)/l03, ...)
+            const float gx0 = (B.y - A.w) / C.y, gx1 = (A.y - B.y) / C.z, gx2 = (A.w - A.y) / C.w;
+            const float gy0 = (A.z - B.x) / C.y, gy1 = (B.x - A.x) / C.z, gy2 = (A.x - A.z) / C.w;
+            float ux = (X.y * gx0 + C1.x * gx1) + C1.w * gx2, vx = (X.z * gx0 + C1.y * gx1) + C2.x * gx2;
+            float uy = (X.y * gy0 + C1.x * gy1) + C1.w * gy2, vy = (X.z * gy0 + C1.y * gy1) + C2.x * gy2;
+            if (TEX & TEX_PERSP) {   // d(U/W) = (dU - u dW) / W
+                const float wx = (X.w * gx0 + C1.z * gx1) + C2.y * gx2, wy = (X.w * gy0 + C1.z * gy1) + C2.y * gy2;
+                ux = (ux - u * wx) / c[2]; vx = (vx - v * wx) / c[2];
+                uy = (uy - u * wy) / c[2]; vy = (vy - v * wy) / c[2];
+            }
+            sample_trilinear(F, mip_lod(F, ux, vx, uy, vy), u, v, c);
+        } else if (TEX & TEX_BILINEAR) {
+            sample_bilinear(F.tex, F.texH, F.texW, u, v, c);
         } else {   // row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1); BGR as cv2.imread gives it
             const int row = clipi(f32_to_i32_x86((1.0f - v) * (float)F.texH), 0, F.texH - 1);
             const int col = clipi(f32_to_i32_x86(u * (float)F.texW), 0, F.texW - 1);
-            texel_bgr(F, row, col, c);
+            texel_bgr(F.tex, F.texW, row, col, c);
         }
     }
     if (F.flags & CRB_GURO) {  // guro_illumination.py:23-27 (float32, left-to-right sums)
@@ -1785,6 +1840,27 @@ __global__ void __launch_bounds__(NT) k_pack_texture(const uint8_t *__restrict__
         out[i] = (uint32_t)bgr[3 * i] | ((uint32_t)bgr[3 * i + 1] << 8) | ((uint32_t)bgr[3 * i + 2] << 16);
 }
 
+// crb_pack_texture_mips: level k+1 of a mip chain from level k (DESIGN 2), one thread per destination texel, per channel
+// (t[r0][c0] + t[r0][c1] + t[r1][c0] + t[r1][c1] + 2) >> 2 with r0 = min(2r, sh-1), r1 = min(2r+1, sh-1), columns alike
+__global__ void __launch_bounds__(NT) k_mip_level(const uint32_t *__restrict__ src, int sh, int sw, uint32_t *__restrict__ dst, int dh, int dw)
+{
+    const long long n = (long long)dh * dw, stride = (long long)gridDim.x * NT;
+    for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < n; i += stride) {
+        const int r = (int)(i / dw), c = (int)(i - (long long)r * dw);
+        const int r0 = min(2 * r, sh - 1), r1 = min(2 * r + 1, sh - 1), c0 = min(2 * c, sw - 1), c1 = min(2 * c + 1, sw - 1);
+        const uint32_t a = __ldg(src + r0 * sw + c0), b = __ldg(src + r0 * sw + c1);
+        const uint32_t d = __ldg(src + r1 * sw + c0), e = __ldg(src + r1 * sw + c1);
+        uint32_t out = 0;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const int sh8 = 8 * k;
+            const uint32_t s = ((a >> sh8) & 255u) + ((b >> sh8) & 255u) + ((d >> sh8) & 255u) + ((e >> sh8) & 255u) + 2u;
+            out |= (s >> 2) << sh8;
+        }
+        dst[i] = out;
+    }
+}
+
 // pyx:65-67
 __global__ void __launch_bounds__(NT) k_init_buffers(float *z, float *color, float *normals, long long pixels)
 {
@@ -2061,6 +2137,7 @@ struct crb_filler {
     int u8x_n, u8x_rows;
     const uint32_t *tex;   // crb_bind_texture: packed texels (caller-owned device memory), NULL = none
     int tex_h, tex_w;
+    int tex_levels;        // crb_bind_texture_mips: levels of the bound chain; 0 = a single level (crb_bind_texture)
 };
 
 namespace {
@@ -2173,12 +2250,17 @@ void fill_frame(const crb_filler *f, Frame *F, int set = 0)
     F->texW = f->tex_w;
 }
 
-// CRB_TEX_PERSPECTIVE and CRB_TEX_BILINEAR are modes of CRB_TEXTURE, which needs a bound texture
+// CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR and CRB_TEX_TRILINEAR are modes of CRB_TEXTURE, which needs a bound texture;
+// CRB_TEX_TRILINEAR needs a bound mip chain and excludes CRB_TEX_BILINEAR
 int check_texture(const crb_filler *f, unsigned flags)
 {
-    if ((flags & (CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR)) && !(flags & CRB_TEXTURE))
-        return fail(CRB_ERR_INVALID, "CRB_TEX_PERSPECTIVE / CRB_TEX_BILINEAR need CRB_TEXTURE");
+    if ((flags & (CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR)) && !(flags & CRB_TEXTURE))
+        return fail(CRB_ERR_INVALID, "CRB_TEX_PERSPECTIVE / CRB_TEX_BILINEAR / CRB_TEX_TRILINEAR need CRB_TEXTURE");
+    if ((flags & CRB_TEX_BILINEAR) && (flags & CRB_TEX_TRILINEAR))
+        return fail(CRB_ERR_INVALID, "CRB_TEX_BILINEAR and CRB_TEX_TRILINEAR exclude each other");
     if ((flags & CRB_TEXTURE) && !f->tex) return fail(CRB_ERR_STATE, "CRB_TEXTURE: no texture bound (crb_bind_texture)");
+    if ((flags & CRB_TEX_TRILINEAR) && !f->tex_levels)
+        return fail(CRB_ERR_STATE, "CRB_TEX_TRILINEAR: no mip chain bound (crb_bind_texture_mips)");
     return CRB_OK;
 }
 
@@ -2320,7 +2402,8 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
 int tex_mode(const Frame &F)
 {
     if (!(F.flags & CRB_TEXTURE)) return TEX_NONE;
-    return ((F.flags & CRB_TEX_BILINEAR) ? TEX_BILINEAR : TEX_NEAREST) | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
+    const int filter = (F.flags & CRB_TEX_TRILINEAR) ? TEX_TRILINEAR : (F.flags & CRB_TEX_BILINEAR) ? TEX_BILINEAR : TEX_NEAREST;
+    return filter | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
 }
 
 template <class C>
@@ -2331,6 +2414,8 @@ void launch_raster(const Frame &F, const TMaps &M, unsigned grid, cudaStream_t s
     case TEX_NEAREST | TEX_PERSP: k_raster<C, TEX_NEAREST | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
     case TEX_BILINEAR: k_raster<C, TEX_BILINEAR><<<grid, C::RT, 0, st>>>(F, M); break;
     case TEX_BILINEAR | TEX_PERSP: k_raster<C, TEX_BILINEAR | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
+    case TEX_TRILINEAR: k_raster<C, TEX_TRILINEAR><<<grid, C::RT, 0, st>>>(F, M); break;
+    case TEX_TRILINEAR | TEX_PERSP: k_raster<C, TEX_TRILINEAR | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
     default: k_raster<C, TEX_NONE><<<grid, C::RT, 0, st>>>(F, M);
     }
 }
@@ -2440,6 +2525,8 @@ int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
     case TEX_NEAREST | TEX_PERSP: k_shade_atomic<TEX_NEAREST | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
     case TEX_BILINEAR: k_shade_atomic<TEX_BILINEAR><<<gS, NT, 0, st>>>(F, f->keybuf); break;
     case TEX_BILINEAR | TEX_PERSP: k_shade_atomic<TEX_BILINEAR | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    case TEX_TRILINEAR: k_shade_atomic<TEX_TRILINEAR><<<gS, NT, 0, st>>>(F, f->keybuf); break;
+    case TEX_TRILINEAR | TEX_PERSP: k_shade_atomic<TEX_TRILINEAR | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
     default: k_shade_atomic<TEX_NONE><<<gS, NT, 0, st>>>(F, f->keybuf);
     }
     return launch_check(f, "k_shade_atomic");
@@ -2848,11 +2935,56 @@ int crb_pack_texture(const uint8_t *bgr, int th, int tw, uint32_t *out, void *st
 int crb_bind_texture(crb_filler *f, const uint32_t *texels, int th, int tw)
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
-    if (!texels) { f->tex = nullptr; f->tex_h = f->tex_w = 0; return CRB_OK; }
+    if (!texels) { f->tex = nullptr; f->tex_h = f->tex_w = f->tex_levels = 0; return CRB_OK; }
     if (th < 1 || tw < 1 || (long long)th * tw >= (1ll << 31))
         return fail(CRB_ERR_INVALID, "crb_bind_texture: th, tw must be >= 1 with th * tw < 2^31 (got %d x %d)", th, tw);
     if (reinterpret_cast<uintptr_t>(texels) & 3u) return fail(CRB_ERR_INVALID, "crb_bind_texture: texels must be 4-byte aligned");
-    f->tex = texels; f->tex_h = th; f->tex_w = tw;
+    f->tex = texels; f->tex_h = th; f->tex_w = tw; f->tex_levels = 0;
+    return CRB_OK;
+}
+
+int crb_mip_layout(int th, int tw, int *levels, long long *texels)
+{
+    if (th < 1 || tw < 1 || (long long)th * tw >= (1ll << 31))
+        return fail(CRB_ERR_INVALID, "crb_mip_layout: th, tw must be >= 1 with th * tw < 2^31 (got %d x %d)", th, tw);
+    int L = 1;
+    long long n = (long long)th * tw;
+    for (int h = th, w = tw; h > 1 || w > 1; ++L) {
+        h = max(1, h >> 1); w = max(1, w >> 1);
+        n += (long long)h * w;
+    }
+    if (n >= (1ll << 31)) return fail(CRB_ERR_INVALID, "crb_mip_layout: a %d x %d chain has %lld >= 2^31 texels", th, tw, n);
+    if (levels) *levels = L;
+    if (texels) *texels = n;
+    return CRB_OK;
+}
+
+int crb_pack_texture_mips(const uint8_t *bgr, int th, int tw, uint32_t *out, void *stream)
+{
+    int L;
+    { int rc = crb_mip_layout(th, tw, &L, nullptr); if (rc) return rc; }
+    { int rc = crb_pack_texture(bgr, th, tw, out, stream); if (rc) return rc; }
+    uint32_t *src = out;
+    for (int l = 1, h = th, w = tw; l < L; ++l) {
+        const int dh = max(1, h >> 1), dw = max(1, w >> 1);
+        uint32_t *dst = src + (long long)h * w;
+        const long long n = (long long)dh * dw;
+        k_mip_level<<<(unsigned)min((n + NT - 1) / NT, 4096ll), NT, 0, (cudaStream_t)stream>>>(src, h, w, dst, dh, dw);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return fail(CRB_ERR_CUDA, "launch of k_mip_level failed: %s", cudaGetErrorString(e));
+        src = dst; h = dh; w = dw;
+    }
+    return CRB_OK;
+}
+
+int crb_bind_texture_mips(crb_filler *f, const uint32_t *chain, int th, int tw)
+{
+    if (check_filler(f)) return CRB_ERR_INVALID;
+    if (!chain) return crb_bind_texture(f, nullptr, 0, 0);
+    int L;
+    { int rc = crb_mip_layout(th, tw, &L, nullptr); if (rc) return rc; }
+    { int rc = crb_bind_texture(f, chain, th, tw); if (rc) return rc; }
+    f->tex_levels = L;
     return CRB_OK;
 }
 

@@ -122,10 +122,11 @@ class AdvancedPixelBufferFiller:
     its own (e.g. this band's rows inside another rank's frame, sharding.PeerFrame); their content is taken as it is.
     `texturing="pixel"` -- render_model samples the model's texture at every pixel (per-pixel texturing, DESIGN 2) instead
     of blending the colours upstream looks up at the vertices ("vertex", the default and upstream's behaviour).
-    `texture_filter="nearest" | "bilinear"` and `perspective_correct=False | True` -- how every textured render of this filler
-    (render_model with texturing="pixel", render_arrays / render_views with texture=) samples: the nearest texel or a bilinear
-    blend of four (CRB_TEX_BILINEAR), from texture coordinates interpolated affinely in screen space or perspective-correctly
-    (CRB_TEX_PERSPECTIVE).
+    `texture_filter="nearest" | "bilinear" | "trilinear"` and `perspective_correct=False | True` -- how every textured render of
+    this filler (render_model with texturing="pixel", render_arrays / render_views with texture=) samples: the nearest texel, a
+    bilinear blend of four (CRB_TEX_BILINEAR), or a blend of bilinear samples of the two levels of the texture's mip chain that
+    the pixel's footprint in the texture selects (CRB_TEX_TRILINEAR; the chain is built on the device when the texture is bound),
+    from texture coordinates interpolated affinely in screen space or perspective-correctly (CRB_TEX_PERSPECTIVE).
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -140,15 +141,17 @@ class AdvancedPixelBufferFiller:
                  texturing="vertex", texture_filter="nearest", perspective_correct=False):
         if texturing not in ("vertex", "pixel"):
             raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
-        if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear"):
-            raise ValueError(f"texture_filter must be 'nearest' or 'bilinear', got {texture_filter!r}")
+        if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear", "trilinear"):
+            raise ValueError(f"texture_filter must be 'nearest', 'bilinear' or 'trilinear', got {texture_filter!r}")
         if not isinstance(perspective_correct, (bool, np.bool_)):
             raise ValueError(f"perspective_correct must be True or False, got {perspective_correct!r}")
         self._texturing = texturing
         # render flags of every textured frame (kept in the arguments of a frame, so a redraw of it samples the same way)
         self._tex_flags = (_lib.CRB_TEXTURE | (_lib.CRB_TEX_BILINEAR if texture_filter == "bilinear" else 0)
+                           | (_lib.CRB_TEX_TRILINEAR if texture_filter == "trilinear" else 0)
                            | (_lib.CRB_TEX_PERSPECTIVE if perspective_correct else 0))
-        self._tex = None              # (source texture, its version, packed uint32 [th,tw] CUDA tensor) bound to the filler
+        # (source texture, its version, packed uint32 CUDA tensor: [th,tw], or with "trilinear" the whole mip chain) bound to the filler
+        self._tex = None
         self._uv = None               # (texture coordinates, their triangle indices, UV-by-triangle CUDA tensor [T,3,3])
         torch = _require_cuda()
         self._torch = torch
@@ -387,8 +390,9 @@ class AdvancedPixelBufferFiller:
         self.render_arrays(v, u[2], n, prefetch=prefetch, texture=tex)
 
     def _bind_texture(self, texture):
-        """Packs (crb_pack_texture) and binds (crb_bind_texture) `texture`, unless it is what is bound already: the same NumPy
-        array object, or the same torch tensor unchanged since (its version counter)."""
+        """Packs (crb_pack_texture) and binds (crb_bind_texture) `texture` -- with texture_filter="trilinear" its mip chain
+        (crb_pack_texture_mips, crb_bind_texture_mips) -- unless it is what is bound already: the same NumPy array object, or the
+        same torch tensor unchanged since (its version counter)."""
         torch = self._torch
         texture = _check_texture(texture)
         version = texture._version if isinstance(texture, torch.Tensor) else None
@@ -403,9 +407,16 @@ class AdvancedPixelBufferFiller:
                 d_bgr = texture.to(self._dev).contiguous()
             else:
                 d_bgr = torch.from_numpy(np.ascontiguousarray(texture)).to(self._dev)
-            packed = torch.empty((th, tw), dtype=torch.int32, device=self._dev)
-            check(self._L.crb_pack_texture(d_bgr.data_ptr(), th, tw, packed.data_ptr(), self._stream()))
-        check(self._L.crb_bind_texture(self._handle, packed.data_ptr(), th, tw))
+            if self._tex_flags & _lib.CRB_TEX_TRILINEAR:
+                texels = ctypes.c_int64()
+                check(self._L.crb_mip_layout(th, tw, None, ctypes.byref(texels)))
+                packed = torch.empty((texels.value,), dtype=torch.int32, device=self._dev)
+                check(self._L.crb_pack_texture_mips(d_bgr.data_ptr(), th, tw, packed.data_ptr(), self._stream()))
+            else:
+                packed = torch.empty((th, tw), dtype=torch.int32, device=self._dev)
+                check(self._L.crb_pack_texture(d_bgr.data_ptr(), th, tw, packed.data_ptr(), self._stream()))
+        bind = self._L.crb_bind_texture_mips if self._tex_flags & _lib.CRB_TEX_TRILINEAR else self._L.crb_bind_texture
+        check(bind(self._handle, packed.data_ptr(), th, tw))
         self._tex = (texture, version, packed)
 
     def _uv_array(self, c, on_device):

@@ -86,6 +86,17 @@ extern "C" {
                                       (t00*gx + t01*fx)*gy + (t10*gx + t11*fx)*fy with fx = sx - floor(sx), gx = 1 - fx (same for y).
                                       At texel centres this is the nearest texel.  Either mode bit without CRB_TEXTURE: CRB_ERR_INVALID
                                       on every render entry point. */
+#define CRB_TEX_TRILINEAR 8192u    /* with CRB_TEXTURE: trilinear mip filtering (DESIGN 2) of the chain bound with crb_bind_texture_mips
+                                      (L levels, level 0 the texture).  Per pixel, from the record's corners and denominators:
+                                      gx = ((y2-y1)/l03, (y0-y2)/l13, (y1-y0)/l23), gy = ((x1-x2)/l03, (x2-x0)/l13, (x0-x1)/l23), and for
+                                      corner values a_k, a_x = (a0*gx0 + a1*gx1) + a2*gx2 (a_y alike).  Affine: ux = u_x, vx = v_x, ...;
+                                      with CRB_TEX_PERSPECTIVE ux = (U_x - u*W_x) / W, vx = (V_x - v*W_x) / W (y alike).  p = ux*tw,
+                                      q = vx*th, r = uy*tw, s = vy*th (level 0's size); r2 = fmax(p*p + q*q, r*r + s*s);
+                                      L2 = (k - 1) + (2f - 1) with r2 = f * 2^k, f in [0.5, 1) (frexp; r2 = 0: -inf, +inf: +inf, NaN: NaN);
+                                      lc = fmin(fmax(0.5*L2, 0), L-1) (NaN -> 0); l0 = floor(lc), fr = lc - l0, l1 = min(l0 + 1, L-1);
+                                      colour = c0*(1 - fr) + c1*fr with c0, c1 CRB_TEX_BILINEAR's blend on levels l0, l1.  float32, one
+                                      rounding per operation.  Where lc == 0 this is CRB_TEX_BILINEAR bit for bit.  Without CRB_TEXTURE,
+                                      or with CRB_TEX_BILINEAR: CRB_ERR_INVALID; no chain bound: CRB_ERR_STATE. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u
@@ -170,6 +181,23 @@ int crb_pack_texture(const uint8_t *bgr, int th, int tw, uint32_t *out, void *st
  * crb_bind_buffers) as the texture of CRB_TEXTURE renders.  texels = NULL unbinds.  CRB_ERR_INVALID for th or tw < 1,
  * th * tw >= 2^31, or a pointer that is not 4-byte aligned. */
 int crb_bind_texture(crb_filler *f, const uint32_t *texels, int th, int tw);
+
+/* Mip chain of a [th,tw] texture for CRB_TEX_TRILINEAR: L = 1 + floor(log2(max(th, tw))) levels, level k+1 of size
+ * max(1, th_k >> 1) x max(1, tw_k >> 1), row-major and back to back from level 0 (the packed texture).  Writes L to *levels and
+ * the chain's total texels to *texels (either may be NULL).  CRB_ERR_INVALID for th or tw < 1, th * tw >= 2^31, or a chain of
+ * 2^31 texels or more. */
+int crb_mip_layout(int th, int tw, int *levels, long long *texels);
+
+/* bgr: DEVICE uint8 [th,tw,3] -> out: DEVICE uint32, the whole chain (crb_mip_layout's texels): level 0 as crb_pack_texture
+ * packs it, then each level from the one before, per channel (t[r0][c0] + t[r0][c1] + t[r1][c0] + t[r1][c1] + 2) >> 2 in integers,
+ * r0 = min(2r, th_k - 1), r1 = min(2r + 1, th_k - 1), columns alike.  Current device, asynchronous on `stream`.
+ * CRB_ERR_INVALID as crb_mip_layout, or for NULL pointers. */
+int crb_pack_texture_mips(const uint8_t *bgr, int th, int tw, uint32_t *out, void *stream);
+
+/* Binds a chain (crb_pack_texture_mips; caller-owned DEVICE memory, 4-byte aligned) of a [th,tw] texture.  It serves
+ * CRB_TEX_TRILINEAR, and nearest and bilinear renders from level 0, exactly as crb_bind_texture of level 0 would.  chain = NULL
+ * unbinds; crb_bind_texture replaces it.  CRB_ERR_INVALID as crb_mip_layout. */
+int crb_bind_texture_mips(crb_filler *f, const uint32_t *chain, int th, int tw);
 
 /* ---- render_model: pyx:92-104 -> project (pyx:106-130) + cull/bbox/raster/z-test/writes (pyx:177-244) ------- */
 
