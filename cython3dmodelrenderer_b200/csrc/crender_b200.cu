@@ -31,6 +31,7 @@
 #include <atomic>
 #include <mutex>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "crender_b200.h"
@@ -42,52 +43,22 @@ namespace {
 
 constexpr int TW = 32;          // tile width in pixels  (one 128-byte line of z, three of colour / normals)
 constexpr int TH = 32;          // tile height in pixels
-constexpr int NT = 256;         // threads per CTA in every kernel but the tile rasterizer
-// The tile rasterizer is instantiated in two CTA shapes (RasterShape / RasterLarge / RasterSmall, further down); the macros below
-// are the large shape's parameters, the CRB_SMALL_* ones the small shape's.
-#ifndef CRB_RT
-#define CRB_RT 128              // threads per CTA of k_raster (a multiple of 32)
-#endif
-#ifdef CRB_ABLATION
-#define DBG(F, bit) (((F).flags & (bit)) != 0u)
-#else
-#define DBG(F, bit) ((void)(bit), false)
-#endif
-constexpr unsigned FLAG_DBG_ONEREC = 0x100000u;   // ablation: every pixel shades from record 0 (measures the cost of the gathers; wrong image)
-constexpr unsigned FLAG_DBG_NOCLEAR = 0x10000u, FLAG_DBG_NOSHADE = 0x20000u, FLAG_DBG_NOROWS = 0x40000u, FLAG_DBG_NOOUT = 0x80000u;  // ablation switches (CRB_DEBUG_SKIP)
-constexpr unsigned FLAG_OUT_DIRECT = 0x200u;   // experiment: shaded pixels stored straight from registers (12-byte strided stores)
-constexpr unsigned FLAG_OUT_TMA = 0x100u;   // internal Frame.flags bit: shaded colour / normal rows leave through TMA boxes
+constexpr int NT = 256;         // threads per CTA in every kernel but the tile rasterizer (its CTA shapes: RasterShape, further down)
 constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR;   // per-pixel texturing and its modes
-#ifndef CRB_CH
-#define CRB_CH 96               // triangles staged in shared memory per pass of the tile rasterizer
-#endif
 constexpr unsigned SPLIT_N = 48;  // single-view launches: tiles with more triangles than this are rasterized by SPLIT_BANDS CTAs, 8 rows each
 constexpr int SPLIT_BANDS = 4;
-#ifndef CRB_CLEAR_EVERY
-#define CRB_CLEAR_EVERY 4
-#endif
-constexpr unsigned CE = CRB_CLEAR_EVERY;  // every CE-th CTA of k_raster is a clear CTA (power of two)
+constexpr unsigned CE = 4;        // every CE-th CTA of k_raster is a clear CTA (power of two)
 constexpr int WIDE_TILES = 12;    // a triangle whose pixel rectangle touches more tiles than this is binned by its whole warp
 constexpr unsigned HEAVY_N = 64;  // tiles with more triangles than this are rasterized first (longest first: shorter kernel tail)
-#ifndef CRB_FQ
-#define CRB_FQ 256              // fragments a warp compacts per round (8 per row)
-#endif
-#ifndef CRB_KEY_STRIDE
-#define CRB_KEY_STRIDE 35
-#endif
 // 64-bit keys, row stride 35 = 3 (mod 16 bank pairs): the fragments a warp evaluates together are a few consecutive pixels of
 // consecutive rows (a small triangle), and with a shift of three bank pairs per row they spread over all the banks
 // (stride 33 shifted one pair per row: 60 % of the key accesses were bank-conflict replays)
-constexpr int KEY_STRIDE = CRB_KEY_STRIDE;
+constexpr int KEY_STRIDE = 35;
 constexpr unsigned long long KEY_EMPTY = 0xFFFFFFFFFFFFFFFFull;
 constexpr float Z_INIT = 1e6f;  // pyx:67
 constexpr float REJ_EPS = 1e-6f;      // fast-reject guard band on barycentric numerators (see tri_fast_setup)
 constexpr float L3_MIN = 1e-30f, L3_MAX = 1e30f;
 constexpr int MAX_DIM = 65535;  // bbox corners are packed in 16 bits
-#ifndef CRB_CLEAR_ROWS
-#define CRB_CLEAR_ROWS 16       // rows per TMA box of the fused clear (the constant pattern must fit the staging area it shares)
-#endif
-constexpr int BOX_ROWS = 8;       // rows per TMA box (clear pattern and shaded rows go out 8 tile rows at a time)
 constexpr int HSTAT_WORDS = 4;    // 64-bit words of busy-tile statistics k_raster posts per position in a batch of launches (8 positions)
 constexpr size_t HSTAT_BYTES = 8 * HSTAT_WORDS * 8;
 constexpr int PROF_MAX = 8192;  // k_raster launches that can be timed between two crb_profile_read calls
@@ -276,11 +247,6 @@ __device__ __forceinline__ float div_rn_by(float a, float d, float r)
 __device__ __forceinline__ bool fdiv_ok_lo(float n1, float n2, float n3)
 {
     return fminf(fminf(fabsf(n1), fabsf(n2)), fabsf(n3)) >= FDIV_LO;   // NaN: false
-}
-__device__ __forceinline__ bool fdiv_ok(float n1, float n2, float n3)
-{
-    const float a1 = fabsf(n1), a2 = fabsf(n2), a3 = fabsf(n3);
-    return fminf(fminf(a1, a2), a3) >= FDIV_LO && fmaxf(fmaxf(a1, a2), a3) <= FDIV_HI;   // NaN: false
 }
 
 // astype('int32') of a float32 on x86-64 (cvttss2si): INT32_MIN for NaN and out-of-range values -- the conversion of
@@ -755,9 +721,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
     }
 }
 
-#ifndef CRB_SETUP_MIN_CTAS
-#define CRB_SETUP_MIN_CTAS 3
-#endif
+constexpr int SETUP_MIN_CTAS = 3;
 // Persistent: a few CTAs per SM walk the (view, chunk) work items -- all chunks of all views, or the chunks k_band_chunks listed
 // for a band-sharded filler -- through a ring of SETUP_STAGES shared-memory stages.  One thread issues the three 9 216-byte bulk
 // copies (cp.async.bulk, completion counted on the stage's mbarrier) of the item two turns ahead as soon as the CTA is done
@@ -767,7 +731,7 @@ constexpr int SETUP_STAGES = 2;
 constexpr size_t SETUP_STAGE_FLOATS = 3 * (size_t)NT * 9;
 constexpr size_t SETUP_DYN_SMEM = SETUP_STAGES * SETUP_STAGE_FLOATS * sizeof(float);
 template <bool PERSP>
-__global__ void __launch_bounds__(NT, CRB_SETUP_MIN_CTAS) k_setup(const Frame F)
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
 {
     extern __shared__ __align__(128) float stg[];          // [SETUP_STAGES][3][NT * 9]
     __shared__ __align__(8) unsigned long long bar[SETUP_STAGES];
@@ -1039,10 +1003,8 @@ __device__ __forceinline__ void fill_chunk(const Frame &F, const int view, const
     }
 }
 
-#ifndef CRB_FILL_MIN_CTAS
-#define CRB_FILL_MIN_CTAS 16
-#endif
-__global__ void __launch_bounds__(FT, CRB_FILL_MIN_CTAS) k_fill(const Frame F)
+constexpr int FILL_MIN_CTAS = 16;
+__global__ void __launch_bounds__(FT, FILL_MIN_CTAS) k_fill(const Frame F)
 {
     const long long chunksPerView = (F.T + NT - 1) / NT;
     const unsigned tix = (blockIdx.x & (NT / FT - 1)) * FT + threadIdx.x;
@@ -1117,11 +1079,11 @@ __device__ __forceinline__ void smem_key_min(unsigned long long *p, unsigned lon
 }
 
 // Tensor maps (TMA) of the three output arrays of one launch, as 3-D tensors [view][row][x] (x in floats: W for z,
-// 3W for colour / normals) with boxes of BOX_ROWS rows x one tile width.  Built on the host per launch (the output
-// pointers are per call).  `use` bit k = map k is valid (CRB_BUF_* order); 0 = the launch uses plain stores only.
+// 3W for colour / normals) with boxes of the shape's CLEAR_ROWS rows x one tile width: the fused clear.  Built on the
+// host per launch (the output pointers are per call).  `use` bit k = map k is valid (CRB_BUF_* order); 0 = the launch
+// uses plain stores only.
 struct __align__(64) TMaps {
-    CUtensorMap z, c, n;        // boxes of BOX_ROWS rows: the shaded rows of a busy tile
-    CUtensorMap zt, ct, nt;     // boxes of a whole tile (TH rows): the fused clear
+    CUtensorMap zt, ct, nt;
     unsigned use;
 };
 
@@ -1154,13 +1116,13 @@ __device__ unsigned long long g_phase[16];
 #define PH(k) do { } while (0)
 #endif
 
-// Shape of the tile rasterizer: threads per CTA, triangles staged per pass, fragment queue per warp, rows per clear box, resident CTAs
-// per SM the launch bounds ask for, and whether shaded colour / normal rows are staged in shared memory (TMA boxes / vector stores)
-// or stored straight from registers.  Three shapes are instantiated, see RasterLarge / RasterSmall / RasterWide below.
-template <int RT_, int CH_, int FQ_, int CLEAR_ROWS_, int MIN_CTAS_, bool OUT_STAGE_>
+// Shape of the tile rasterizer: threads per CTA (a multiple of 32), triangles staged in shared memory per pass, fragments a warp
+// compacts per round, rows per TMA box of the fused clear (the constant pattern must fit the staging area it
+// shares), and resident CTAs per SM the launch bounds ask for.  Shaded pixels are stored straight from registers.  Three shapes
+// are instantiated, see RasterLarge / RasterSmall / RasterWide below.
+template <int RT_, int CH_, int FQ_, int CLEAR_ROWS_, int MIN_CTAS_>
 struct RasterShape {
     static constexpr int RT = RT_, CH = CH_, FQ = FQ_, CLEAR_ROWS = CLEAR_ROWS_, MIN_CTAS = MIN_CTAS_;
-    static constexpr bool OUT_STAGE = OUT_STAGE_;
     static_assert(CH_ <= RT_ && CH_ <= 256 && RT_ % 32 == 0 && RT_ <= NT, "one staged triangle per thread, 8-bit owner index");
     static_assert(FQ_ % 32 == 0 && FQ_ >= 64 && TH % CLEAR_ROWS_ == 0, "queue rounds of FQ/32 - 1 pixels per row; whole clear boxes per tile");
 };
@@ -1168,7 +1130,7 @@ struct RasterShape {
 template <class C>
 struct __align__(128) TileSmem {
     static constexpr int RT = C::RT, CH = C::CH, FQ = C::FQ, CLEAR_ROWS = C::CLEAR_ROWS;
-    // TMA source first (128-byte aligned): shaded colour / normal rows of the tile
+    // TMA source first (128-byte aligned): the clear pattern
     union {
         struct {
             // per staged triangle (written by its staging thread, see raster_tile): the three edges in the sign-normalised form
@@ -1183,10 +1145,7 @@ struct __align__(128) TileSmem {
             float4 slot[RT / 32][2][32];   // per warp, per trip parity: the trip's 32 rows (A1 A2 A3 | staged triangle, tile row)
             unsigned short fq[RT / 32][FQ];  // per warp: queue of fragments (row lane | x << 5 | trip parity << 10)
         } st;
-        struct {                              // (without row staging: only the 3 KB the staged uint8 image of a tile needs)
-            float col[C::OUT_STAGE ? TH * TW * 3 : TH * TW * 3 / 4];
-            float nrm[C::OUT_STAGE ? TH * TW * 3 : 4];
-        } out;
+        unsigned char u8[TH * TW * 3];        // the staged uint8 image of a tile (raster_tile's u8stage)
         struct {                              // clear CTAs only: the constant pattern their TMA boxes are stored from
             float z[CLEAR_ROWS * TW];         //   Z_INIT
             float c[CLEAR_ROWS * TW * 3];     //   background colour = 0 (background_color) = the cleared normals: one pattern serves both
@@ -1280,13 +1239,11 @@ constexpr int PK_XA = 8, PK_XB = 14, PK_YT = 20;   // tile-relative rectangle: f
 
 // Visibility + deferred shading of one busy tile (n triangles staged at list offset off).
 template <class C, int TEX>
-__device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, TileSmem<C> &S_, const bool clear, const int view,
+__device__ __forceinline__ void raster_tile(const Frame &F, TileSmem<C> &S_, const bool clear, const int view,
                                             const int tx, const int ty, const unsigned n, const unsigned off, const int rowLo, const int rowHi)
 {
-    constexpr int RT = C::RT, CH = C::CH, FQ = C::FQ;      // (shadow the defaults of the same names)
-    constexpr bool OUT_STAGE = C::OUT_STAGE;
+    constexpr int RT = C::RT, CH = C::CH, FQ = C::FQ;
     typedef TileSmem<C> TS;
-#ifndef CRB_NO_OPAQUE_SMEM
     // The address of the CTA's shared memory goes through an empty asm: under the 40-register cap the compiler otherwise re-derives
     // the shared-window base (S2R SR_CgaCtaId + LEA) inside the exact and the shading loops instead of keeping it; an opaque
     // value cannot be rematerialised, and __isShared keeps the accesses LDS / STS / ATOMS.
@@ -1294,9 +1251,6 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
     asm volatile("" : "+l"(Sp));
     __builtin_assume(__isShared(Sp));
     TS &S = *Sp;
-#else
-    TS &S = S_;
-#endif
     const int x0 = tx * TW, yl0 = ty * TH;       // yl0: row inside the band's buffers
     const int y0 = F.row0 + yl0;                  // absolute image row
     const int tw = min(TW, F.W - x0), th = min(min(TH, F.row1 - y0), rowHi);   // this CTA's rows of the tile: [rowLo, th)
@@ -1323,7 +1277,6 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
             // correctly rounded reciprocals of the (sign-normalised) denominators, for div_rn_by: RN(1/-x) = -RN(1/x), so these are
             // the bits k_setup's rcp.rn of the signed denominators would give after the same sign flip
             tr3 = make_float4(__frcp_rn(c.y), __frcp_rn(c.z), __frcp_rn(c.w), 0.0f);
-#ifndef CRB_NO_REC_PREFETCH
             if (CH < 64) {   // the shading pass will want this triangle's 128-byte record: start pulling it into L1 now (T-Rex x128
                              // -2.6 %; tiles of ~150 triangles evict them again before they are shaded: the large shape goes without)
                 const char *sr = reinterpret_cast<const char *>(F.shrec + ((long long)view * F.T + d.z) * SREC);
@@ -1332,7 +1285,6 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
                 asm volatile("prefetch.global.L1 [%0];" :: "l"(sr + 64));
                 asm volatile("prefetch.global.L1 [%0];" :: "l"(sr + 96));
             }
-#endif
             // edge vectors, sign-normalised (exact negation: flip the sign bit)
             const unsigned s1 = (d.w & 1u) << 31, s2 = (d.w & 2u) << 30, s3 = (d.w & 4u) << 29;
             S.u.st.e0[tid] = make_float4(__uint_as_float(__float_as_uint(a.z - b.x) ^ s1), b.y,
@@ -1368,15 +1320,12 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
         // Row work items, 32 per warp per trip.  Trip counts are warp-uniform and the body is predicated, so the warp
         // stays converged (a per-thread `for (r = tid; ...)` with early `continue`s lets lanes drift apart under
         // independent thread scheduling: measured 7.5 active lanes per instruction).
-        if (DBG(F, FLAG_DBG_NOROWS)) totalRows = 0;
         // Tiles of a few large triangles (on average 16+ rows of the tile each: long spans, a full queue round per row)
         // have too few rows to occupy eight warps 32 at a time: there a trip of fewer than NT rows is dealt out in equal
         // shares (bunny 4096^2: k_raster 343 -> 304 us).  Tiles of many small triangles keep whole warps: the span pass
         // costs a warp the same with 8 active lanes as with 32, and those tiles are bound by issue slots, not latency.
-#ifndef CRB_DEAL_ROWS
-#define CRB_DEAL_ROWS 16
-#endif
-        const bool deal = totalRows >= (unsigned)CRB_DEAL_ROWS * m;
+        constexpr unsigned DEAL_ROWS = 16;
+        const bool deal = totalRows >= DEAL_ROWS * m;
         // Exact pass.  The surviving pixels of a trip's 32 rows are intervals (first x, count).  In rounds of at most FQ/32 - 1
         // pixels per row, the rows append one entry per fragment (row lane | x << 5 | trip parity << 10) to the warp's queue at
         // the positions an exclusive scan of the counts assigns, and the queue is evaluated 32 entries at a time -- whole
@@ -1516,17 +1465,13 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
     __syncthreads();
     PH(6);
 
-    // ---- deferred shading of the winners, staged so that colour / normals leave as whole rows ---------------
+    // ---- deferred shading of the winners ---------------------------------------------------------------------
     const long long slab = (long long)view * F.slabPixels;
-    const bool tma = OUT_STAGE && clear && M.use != 0u && (F.flags & FLAG_OUT_TMA);     // colour / normal rows leave through TMA boxes
-    const bool vec = OUT_STAGE && clear && !tma && (tw == TW) && ((F.W & 3) == 0) && !(F.flags & FLAG_OUT_DIRECT) &&
-                     (F.color || F.normals);                                                            // ... or as 16-byte vector stores
-    const bool stage = tma || vec;
-    // The uint8 image of a fresh frame whose float32 rows need no staging (image-only frames: HostImagePipeline, the row exchange,
-    // PeerImage) is staged instead: the shading loop writes its three bytes per pixel into shared memory and the tile's rows leave
-    // as 16-byte vector stores, six per 96-byte row = three whole sectors -- what a row exchange sends over NVLink is sectors, and
-    // three byte stores per pixel touch each of them partially (N = 8: 0.77 of the rendering rate delivered).
-    const bool u8stage = !stage && clear && F.color_u8 && tw == TW && !(F.W & 15) && (!F.u8xN || F.u8xRows % TH == 0);
+    // The uint8 image of a fresh frame (image-only frames: HostImagePipeline, the row exchange, PeerImage) is staged: the shading
+    // loop writes its three bytes per pixel into shared memory and the tile's rows leave as 16-byte vector stores, six per 96-byte
+    // row = three whole sectors -- what a row exchange sends over NVLink is sectors, and three byte stores per pixel touch each of
+    // them partially (N = 8: 0.77 of the rendering rate delivered).
+    const bool u8stage = clear && F.color_u8 && tw == TW && !(F.W & 15) && (!F.u8xN || F.u8xRows % TH == 0);
     const float bg = background_color(F);
     const long long tilebase = slab + (long long)yl0 * F.W + x0;          // first pixel of the tile in its slab
     const unsigned rowStep = (unsigned)(RT / TW) * (unsigned)F.W;
@@ -1538,10 +1483,10 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
         const unsigned long long key = S.keys[yy * KEY_STRIDE + xx];
         float z = Z_INIT, c[3] = {bg, bg, bg}, nn[3] = {0.f, 0.f, 0.f};
         bool write = clear;
-        if (key != KEY_EMPTY && !DBG(F, FLAG_DBG_NOSHADE)) {
+        if (key != KEY_EMPTY) {
             const unsigned tri = ~(unsigned)(key & 0xFFFFFFFFull);
             float fz, fc[3], fn[3];
-            if (shade_fragment<TEX>(F, recv + (size_t)(DBG(F, FLAG_DBG_ONEREC) ? 0u : tri) * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn)) {
+            if (shade_fragment<TEX>(F, recv + (size_t)tri * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn)) {
                 const float zold = clear ? Z_INIT : F.z[pix];
                 if (!(fz > zold)) {  // pyx:223: drawn unless new_z > z_buffer (equal depth overwrites)
                     z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
@@ -1549,59 +1494,22 @@ __device__ __forceinline__ void raster_tile(const Frame &F, const TMaps &M, Tile
                 }
             }
         }
-        if (OUT_STAGE && stage) {
-            S.u.out.col[p * 3] = c[0]; S.u.out.col[p * 3 + 1] = c[1]; S.u.out.col[p * 3 + 2] = c[2];
-            S.u.out.nrm[p * 3] = nn[0]; S.u.out.nrm[p * 3 + 1] = nn[1]; S.u.out.nrm[p * 3 + 2] = nn[2];
-            if (F.z && !DBG(F, FLAG_DBG_NOOUT)) F.z[pix] = z;
-        } else if (write) {
+        if (write) {
             if (F.z) F.z[pix] = z;
             if (F.color) { F.color[pix * 3] = c[0]; F.color[pix * 3 + 1] = c[1]; F.color[pix * 3 + 2] = c[2]; }
             if (F.normals) { F.normals[pix * 3] = nn[0]; F.normals[pix * 3 + 1] = nn[1]; F.normals[pix * 3 + 2] = nn[2]; }
         }
-        if (F.color_u8 && write) {       // (one test on the float32-only path, as before the staging)
-            unsigned char *o = u8stage ? reinterpret_cast<unsigned char *>(S.u.out.col) + p * 3 : u8_pixel(F, view, yl0 + yy, x0 + xx);
+        if (F.color_u8 && write) {
+            unsigned char *o = u8stage ? S.u.u8 + p * 3 : u8_pixel(F, view, yl0 + yy, x0 + xx);
             o[0] = to_u8(c[0]); o[1] = to_u8(c[1]); o[2] = to_u8(c[2]);
         }
     }
     PH(7);
     if (u8stage) {
         __syncthreads();
-        const unsigned char *sb = reinterpret_cast<const unsigned char *>(S.u.out.col);
         for (int i = tid; i < (th - rowLo) * 6; i += RT) {
             const int r = rowLo + i / 6, q = i - (i / 6) * 6;
-            reinterpret_cast<uint4 *>(u8_pixel(F, view, yl0 + r, x0))[q] = reinterpret_cast<const uint4 *>(sb + r * (TW * 3))[q];
-        }
-    }
-    if (DBG(F, FLAG_DBG_NOOUT)) return;
-    if (OUT_STAGE && tma) {
-        fence_async_smem();
-        __syncthreads();
-        PH(8);
-        if (lane == 0) {   // box job j: array j/4 (colour, normals), row block j%4; one job per warp with eight warps
-            for (unsigned job = wid; job < 8u; job += RT / 32) {
-                const int r = (int)(job & 3u) * BOX_ROWS;
-                if (r >= rowLo && r < th) {       // row bands are multiples of BOX_ROWS
-                    if (job < 4u) { if (M.use & CRB_BUF_COLOR) tma_store_box(&M.c, S.u.out.col + r * TW * 3, x0 * 3, yl0 + r, view); }
-                    else if (M.use & CRB_BUF_NORMALS) tma_store_box(&M.n, S.u.out.nrm + r * TW * 3, x0 * 3, yl0 + r, view);
-                }
-            }
-            tma_commit();
-        }
-    } else if (OUT_STAGE && vec) {
-        __syncthreads();
-        const int q = tid & 7;
-        for (int r = rowLo + (tid >> 3); r < th; r += RT / 8) {
-            const long long o = (slab + (long long)(yl0 + r) * F.W + x0) * 3;
-            if (F.color) {
-                float4 *g = reinterpret_cast<float4 *>(F.color + o);
-                const float4 *sc = reinterpret_cast<const float4 *>(S.u.out.col + r * TW * 3);
-                g[q] = sc[q]; g[q + 8] = sc[q + 8]; g[q + 16] = sc[q + 16];
-            }
-            if (F.normals) {
-                float4 *g = reinterpret_cast<float4 *>(F.normals + o);
-                const float4 *sn = reinterpret_cast<const float4 *>(S.u.out.nrm + r * TW * 3);
-                g[q] = sn[q]; g[q + 8] = sn[q + 8]; g[q + 16] = sn[q + 16];
-            }
+            reinterpret_cast<uint4 *>(u8_pixel(F, view, yl0 + r, x0))[q] = reinterpret_cast<const uint4 *>(S.u.u8 + r * (TW * 3))[q];
         }
     }
     PH(9);
@@ -1628,11 +1536,8 @@ __device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C>
 // frame) -- a few thousand cycles of queueing, no arithmetic -- so those stores drain beside the rasterizing CTAs that
 // share its SM for the whole length of the kernel.  Launches without tensor maps clear with plain stores up front,
 // every CTA adopting its share of the empty tiles.
-// Resident CTAs per SM follow the shape (RasterSmall 12 at 40 registers, RasterLarge 8 at 62, RasterWide 6 at 40); the
+// Resident CTAs per SM follow the shape (RasterSmall 12 at 40 registers, RasterLarge 8 at up to 64, RasterWide 6 at 40); the
 // static_assert in k_raster ties each shape's shared memory to the residency its launch bounds ask for.
-#ifndef CRB_RASTER_MIN_CTAS
-#define CRB_RASTER_MIN_CTAS 8
-#endif
 template <class C, int TEX>
 __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, const __grid_constant__ TMaps M)
 {
@@ -1654,7 +1559,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
             unsigned t = e < nAll ? F.empty[e] : 0u;              // speculative: flies with the totals
             const unsigned long long pairs = F.total[0];
             const unsigned ne = (unsigned)F.total[3];
-            if (pairs > (unsigned long long)F.pairCap || DBG(F, FLAG_DBG_NOCLEAR)) return;     // frame skipped: buffers stay untouched
+            if (pairs > (unsigned long long)F.pairCap) return;     // frame skipped: buffers stay untouched
             const float bg = background_color(F);
             for (int i = threadIdx.x; i < CLEAR_ROWS * TW * 3 / 4; i += RT) {
                 reinterpret_cast<float4 *>(S.u.pat.c)[i] = make_float4(bg, bg, bg, bg);       // (bg is 0.0f: also the normals' pattern)
@@ -1696,7 +1601,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
         hs[1] = (unsigned long long)nHeavy | ((F.total[5] > 0xFFFFFFFFull ? 0xFFFFFFFFull : F.total[5]) << 32);     // + triangles that span many tiles
         hs[2] = pairs;                                                                                                  // (triangle, tile) pairs: the next launch's shape
     }
-    if (clear && !split && !DBG(F, FLAG_DBG_NOCLEAR)) {
+    if (clear && !split) {
         const unsigned ne = (unsigned)F.total[3];
         for (unsigned e = bidx; e < ne; e += Gb) {
             const unsigned t = F.empty[e];
@@ -1707,19 +1612,11 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
     PH(0);
     for (unsigned cta = first; cta < nb; cta += stride) {
         const uint4 cur = rec;
-        if (cta != first) {
-            if ((threadIdx.x & 31) == 0) tma_wait_read();   // the previous tile's rows have left shared memory
-            __syncthreads();
-        }
+        if (cta != first) __syncthreads();                  // the previous tile is done with shared memory
         if (cta + stride < nb) rec = lst[cta + stride];     // the next tile's record arrives while this one is rasterized
-        raster_tile<C, TEX>(F, M, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
+        raster_tile<C, TEX>(F, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
                     (int)(cur.w & 255u), (int)(cur.w >> 8));
     }
-#ifdef CRB_PHASE_TIMING
-    ph_t = clock64();
-#endif
-    if ((threadIdx.x & 31) == 0) tma_wait_read();           // shared memory must outlive the bulk reads
-    PH(10);
 }
 
 // The two throughput shapes of the tile rasterizer, both CTAs of 128 threads that store shaded pixels straight from registers
@@ -1738,34 +1635,12 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
 //     128 threads, CH 128, FQ 256,      7 CTAs/SM, 66 registers       965 / 270 / 1133
 // Tiles of ~150 triangles (the sphere) want many triangles per staging pass and registers instead of warps; ordinary frames want
 // many small CTAs.  run_raster picks the shape per launch from the triangles per busy tile the previous launch posted.
-#ifdef CRB_LARGE_OUT_STAGE       // (shaded rows staged for TMA boxes: 24 KB more shared memory per CTA, needs CRB_RASTER_MIN_CTAS <= 6)
-constexpr bool LARGE_OUT_STAGE = true;
-#else
-constexpr bool LARGE_OUT_STAGE = false;
-#endif
-typedef RasterShape<CRB_RT, CRB_CH, CRB_FQ, CRB_CLEAR_ROWS, CRB_RASTER_MIN_CTAS, LARGE_OUT_STAGE> RasterLarge;
-#ifndef CRB_SMALL_RT
-#define CRB_SMALL_RT 128
-#endif
-#ifndef CRB_SMALL_CH
-#define CRB_SMALL_CH 24
-#endif
-#ifndef CRB_SMALL_FQ
-#define CRB_SMALL_FQ 256
-#endif
-#ifndef CRB_SMALL_CLEAR_ROWS
-#define CRB_SMALL_CLEAR_ROWS 8
-#endif
-#ifndef CRB_SMALL_MIN_CTAS
-#define CRB_SMALL_MIN_CTAS 12
-#endif
-typedef RasterShape<CRB_SMALL_RT, CRB_SMALL_CH, CRB_SMALL_FQ, CRB_SMALL_CLEAR_ROWS, CRB_SMALL_MIN_CTAS, false> RasterSmall;
+typedef RasterShape<128, 96, 256, 16, 8> RasterLarge;
+typedef RasterShape<128, 24, 256, 8, 12> RasterSmall;
 // ... and a third for frames of so few busy tiles that they do not fill the machine once (a single 1024^2 frame): eight warps per
 // tile, 128 triangles per pass -- such a frame takes as long as its slowest CTA, and idle warps cost nothing there
-typedef RasterShape<256, 128, 256, 16, 6, false> RasterWide;
-#ifndef CRB_SHAPE_LARGE_FROM
-#define CRB_SHAPE_LARGE_FROM 64      // triangles per busy tile from which the large shape is launched
-#endif
+typedef RasterShape<256, 128, 256, 16, 6> RasterWide;
+constexpr int SHAPE_LARGE_FROM = 64;      // triangles per busy tile from which the large shape is launched
 
 // ------------------------------------------------------------------------------------------------------------
 // Differential path (CRB_PATH_ATOMIC): one warp per triangle, global 64-bit atomicMin, then a per-pixel shade.
@@ -2109,7 +1984,7 @@ struct crb_filler {
     int raster_ctas;       // experiments: fixed k_raster grid (0 = automatic)
     int raster_shape;      // CRB_OPT_RASTER_SHAPE: 0 = per launch from the posted statistics, 1 = RasterLarge, 2 = RasterSmall, 3 = RasterWide
     int sm_count;
-    int use_tma;           // tensor maps are built where the layout allows (CRB_NO_TMA=1 disables): k_clear stores TMA boxes
+    int use_tma;           // tensor maps are built where the layout allows (CRB_OPT_TMA = 0 disables): the fused clear stores TMA boxes
     unsigned *shown_busy;        // sparse read-back: per tile, mask of the 32 rows that hold something in the frame the caller's host arrays show
     long long shown_tiles;
     unsigned long long *tiles_copied;   // device counter behind crb_readback_stats
@@ -2124,9 +1999,6 @@ struct crb_filler {
     int pending_join;      // 1 + set of the last pipelined launch the caller's stream has not been made to wait for (CRB_DEFER_JOIN)
     int split_heavy;       // single-view launches cut heavy tiles into row bands (CRB_SPLIT_HEAVY=0 disables)
     int band_prepass;      // band-sharded fillers list the chunks that reach the band first (CRB_OPT_BAND_PREPASS)
-    int tiles_per_cta;     // k_raster grid = estimated busy tiles / this (CRB_TILES_PER_CTA)
-    unsigned dbg_flags;    // ablation switches (CRB_DEBUG_SKIP), never set in production
-    int out_tma;           // ... and so does k_raster for the shaded colour / normal rows (CRB_OUT_TMA=0 disables)
     unsigned long long *hstats;      // pinned + mapped: busy-tile statistics of the most recent k_raster launch
     unsigned long long *hstats_dev;
     bool prof_on;
@@ -2292,7 +2164,7 @@ EncodeTiledFn encode_tiled_fn()
     return fn;
 }
 
-// [views][rows][W*comps] float32, boxes of BOX_ROWS x (TW*comps).  Returns false if the layout cannot be described.
+// [views][rows][W*comps] float32, boxes of box_rows x (TW*comps).  Returns false if the layout cannot be described.
 bool encode_map(CUtensorMap *m, float *base, int comps, const Frame &F, int box_rows)
 {
     EncodeTiledFn fn = encode_tiled_fn();
@@ -2310,9 +2182,9 @@ bool encode_map(CUtensorMap *m, float *base, int comps, const Frame &F, int box_
 unsigned encode_maps(TMaps *M, const Frame &F, int clear_rows)
 {
     unsigned use = 0;
-    if (F.z) { if (!encode_map(&M->z, F.z, 1, F, BOX_ROWS) || !encode_map(&M->zt, F.z, 1, F, clear_rows)) return 0u; use |= CRB_BUF_Z; }
-    if (F.color) { if (!encode_map(&M->c, F.color, 3, F, BOX_ROWS) || !encode_map(&M->ct, F.color, 3, F, clear_rows)) return 0u; use |= CRB_BUF_COLOR; }
-    if (F.normals) { if (!encode_map(&M->n, F.normals, 3, F, BOX_ROWS) || !encode_map(&M->nt, F.normals, 3, F, clear_rows)) return 0u; use |= CRB_BUF_NORMALS; }
+    if (F.z) { if (!encode_map(&M->zt, F.z, 1, F, clear_rows)) return 0u; use |= CRB_BUF_Z; }
+    if (F.color) { if (!encode_map(&M->ct, F.color, 3, F, clear_rows)) return 0u; use |= CRB_BUF_COLOR; }
+    if (F.normals) { if (!encode_map(&M->nt, F.normals, 3, F, clear_rows)) return 0u; use |= CRB_BUF_NORMALS; }
     return use;
 }
 
@@ -2335,10 +2207,8 @@ void launch_setup(const Frame &F, unsigned grid, cudaStream_t st)
     else k_setup<false><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
 }
 
-#ifndef CRB_PREPASS_EIGHTHS
-#define CRB_PREPASS_EIGHTHS 5  // the band pre-pass runs for bands of at most this many eighths of the frame (half-frame bands gain
-                               // 7 %; a cut balanced by measurement lands a few strips off the middle, which must not switch it off)
-#endif
+constexpr int PREPASS_EIGHTHS = 5;  // the band pre-pass runs for bands of at most this many eighths of the frame (half-frame bands gain
+                                    // 7 %; a cut balanced by measurement lands a few strips off the middle, which must not switch it off)
 // project/setup/count -> alloc -> fill for up to maxViews views
 int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
 {
@@ -2360,7 +2230,7 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     // (it reads the vertex array once more than k_setup alone would: it pays when many chunks miss the band -- measured on the
     // 10 M-triangle sphere with the persistent k_setup that walks the listed chunks through its bulk-copy ring: half-frame bands
     // 1.14 -> 1.06 ms; round 1, with one-chunk CTAs: half 1.16 -> 1.22 ms, quarter 0.84 -> 0.82, eighth 0.59 -> 0.51)
-    if (banded && f->band_prepass && 8ll * (F.row1 - F.row0) <= (long long)CRB_PREPASS_EIGHTHS * F.H && F.nViews == 1 && !F.views && F.T >= 8 * NT && !(F.flags & CRB_PATH_ATOMIC) &&
+    if (banded && f->band_prepass && 8ll * (F.row1 - F.row0) <= (long long)PREPASS_EIGHTHS * F.H && F.nViews == 1 && !F.views && F.T >= 8 * NT && !(F.flags & CRB_PATH_ATOMIC) &&
         !(reinterpret_cast<uintptr_t>(F.v) & 15u)) {
         const size_t so = (size_t)(reinterpret_cast<const char *>(F.alive) - reinterpret_cast<const char *>(f->alive));   // workspace set in use
         F.chunks = reinterpret_cast<unsigned *>(reinterpret_cast<char *>(f->chunks) + so);
@@ -2374,7 +2244,7 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
         const long long items = F.chunks ? (long long)gT : (long long)gT * F.nViews;
-        launch_setup(F, (unsigned)min(items, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), st);
+        launch_setup(F, (unsigned)min(items, (long long)f->sm_count * SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
     } else {
         CU(cudaMemsetAsync(F.total, 0, 8, st));
@@ -2397,7 +2267,6 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     return CRB_OK;
 }
 
-// raster + shade (+ fused clear) of the frame run_prep binned
 // shading instantiation of a frame: per-vertex colours, or per-pixel texturing with its filter and interpolation
 int tex_mode(const Frame &F)
 {
@@ -2406,20 +2275,23 @@ int tex_mode(const Frame &F)
     return filter | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
 }
 
-template <class C>
-void launch_raster(const Frame &F, const TMaps &M, unsigned grid, cudaStream_t st)
+// Calls fn(std::integral_constant<int, MODE>()) with the frame's tex_mode as a compile-time constant: the one list of the shading
+// instantiations of k_raster and k_shade_atomic
+template <class Fn>
+void with_tex_mode(const Frame &F, Fn &&fn)
 {
     switch (tex_mode(F)) {
-    case TEX_NEAREST: k_raster<C, TEX_NEAREST><<<grid, C::RT, 0, st>>>(F, M); break;
-    case TEX_NEAREST | TEX_PERSP: k_raster<C, TEX_NEAREST | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
-    case TEX_BILINEAR: k_raster<C, TEX_BILINEAR><<<grid, C::RT, 0, st>>>(F, M); break;
-    case TEX_BILINEAR | TEX_PERSP: k_raster<C, TEX_BILINEAR | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
-    case TEX_TRILINEAR: k_raster<C, TEX_TRILINEAR><<<grid, C::RT, 0, st>>>(F, M); break;
-    case TEX_TRILINEAR | TEX_PERSP: k_raster<C, TEX_TRILINEAR | TEX_PERSP><<<grid, C::RT, 0, st>>>(F, M); break;
-    default: k_raster<C, TEX_NONE><<<grid, C::RT, 0, st>>>(F, M);
+    case TEX_NEAREST: fn(std::integral_constant<int, TEX_NEAREST>()); break;
+    case TEX_NEAREST | TEX_PERSP: fn(std::integral_constant<int, TEX_NEAREST | TEX_PERSP>()); break;
+    case TEX_BILINEAR: fn(std::integral_constant<int, TEX_BILINEAR>()); break;
+    case TEX_BILINEAR | TEX_PERSP: fn(std::integral_constant<int, TEX_BILINEAR | TEX_PERSP>()); break;
+    case TEX_TRILINEAR: fn(std::integral_constant<int, TEX_TRILINEAR>()); break;
+    case TEX_TRILINEAR | TEX_PERSP: fn(std::integral_constant<int, TEX_TRILINEAR | TEX_PERSP>()); break;
+    default: fn(std::integral_constant<int, TEX_NONE>());
     }
 }
 
+// raster + shade (+ fused clear) of the frame run_prep binned
 int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
 {
     int rc;
@@ -2446,7 +2318,7 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
                 per_tile = (double)hp / records;
             }
         }
-        shape = busy <= (double)wave ? 3 : (busy <= 4.0 * (double)wave || per_tile >= (double)CRB_SHAPE_LARGE_FROM) ? 1 : 2;
+        shape = busy <= (double)wave ? 3 : (busy <= 4.0 * (double)wave || per_tile >= (double)SHAPE_LARGE_FROM) ? 1 : 2;
     }
     const int clear_rows = shape == 2 ? RasterSmall::CLEAR_ROWS : shape == 3 ? RasterWide::CLEAR_ROWS : RasterLarge::CLEAR_ROWS;
     const int min_ctas = shape == 2 ? RasterSmall::MIN_CTAS : shape == 3 ? RasterWide::MIN_CTAS : RasterLarge::MIN_CTAS;
@@ -2454,9 +2326,6 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     memset(&M, 0, sizeof(M));
     const bool clear = (F.flags & CRB_CLEAR_FIRST) != 0;
     if (f->use_tma && clear && !(F.W & 3) && !F.color_u8) M.use = encode_maps(&M, F, clear_rows);
-    if (M.use && f->out_tma == 1) F.flags |= FLAG_OUT_TMA;
-    if (f->out_tma == 2) F.flags |= FLAG_OUT_DIRECT;
-    F.flags |= f->dbg_flags;
     // Grid: one CTA per busy tile.  The busy count is only known on the device, so the grid is sized from the busy
     // FRACTION the previous launch posted (+12 % and a floor of one wave); k_raster walks with stride gridDim when the
     // estimate was low, and an all-tiles grid is used until a first launch has reported.
@@ -2467,7 +2336,7 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
         const unsigned long long hh = *reinterpret_cast<volatile unsigned long long *>(f->hstats + HSTAT_WORDS * slot + 1) & 0xFFFFFFFFull;
         const double tiles = (double)(hs >> 32), light = (double)(hs & 0xFFFFFFFFull), heavy = (double)hh;
         if (tiles > 0) {
-            gL = (long long)(light / tiles * 1.125 * (double)nAllTiles / (double)f->tiles_per_cta) + 56;
+            gL = (long long)(light / tiles * 1.125 * (double)nAllTiles) + 56;
             gH = (long long)(heavy / tiles * 1.125 * (double)nAllTiles) + 8;
             const long long wave = (long long)f->sm_count * min_ctas;
             if (gL + gH < wave) gL = wave - gH;
@@ -2481,10 +2350,12 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     long long gR = gL + gH;
     if (M.use) gR = (long long)CE * ((gR + CE - 2) / (CE - 1));     // CE - 1 rasterizing CTAs + one clear CTA per group of CE (see k_raster)
     if (prof) CU(cudaEventRecord(f->prof_ev[2 * f->prof_n], st));
-    // per-pixel texturing: the instantiation of the same shape with the frame's texture filter
-    if (shape == 2) launch_raster<RasterSmall>(F, M, (unsigned)gR, st);
-    else if (shape == 3) launch_raster<RasterWide>(F, M, (unsigned)gR, st);
-    else launch_raster<RasterLarge>(F, M, (unsigned)gR, st);
+    with_tex_mode(F, [&](auto mode) {
+        constexpr int TEX = decltype(mode)::value;
+        if (shape == 2) k_raster<RasterSmall, TEX><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
+        else if (shape == 3) k_raster<RasterWide, TEX><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
+        else k_raster<RasterLarge, TEX><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
+    });
     if ((rc = launch_check(f, "k_raster"))) return rc;
     if (prof) {
         CU(cudaEventRecord(f->prof_ev[2 * f->prof_n + 1], st));
@@ -2514,21 +2385,13 @@ int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
     }
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
-        launch_setup(F, (unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * CRB_SETUP_MIN_CTAS), st);
+        launch_setup(F, (unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
         k_raster_atomic<<<(unsigned)((F.T * 32 + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
     }
     const unsigned gS = (unsigned)((F.slabPixels + NT - 1) / NT);
-    switch (tex_mode(F)) {
-    case TEX_NEAREST: k_shade_atomic<TEX_NEAREST><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    case TEX_NEAREST | TEX_PERSP: k_shade_atomic<TEX_NEAREST | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    case TEX_BILINEAR: k_shade_atomic<TEX_BILINEAR><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    case TEX_BILINEAR | TEX_PERSP: k_shade_atomic<TEX_BILINEAR | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    case TEX_TRILINEAR: k_shade_atomic<TEX_TRILINEAR><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    case TEX_TRILINEAR | TEX_PERSP: k_shade_atomic<TEX_TRILINEAR | TEX_PERSP><<<gS, NT, 0, st>>>(F, f->keybuf); break;
-    default: k_shade_atomic<TEX_NONE><<<gS, NT, 0, st>>>(F, f->keybuf);
-    }
+    with_tex_mode(F, [&](auto mode) { k_shade_atomic<decltype(mode)::value><<<gS, NT, 0, st>>>(F, f->keybuf); });
     return launch_check(f, "k_shade_atomic");
 }
 
@@ -2765,15 +2628,6 @@ int crb_create(int h, int w, float fov, float z_near, float z_far, int device, c
             for (int k = 0; k < 2; ++k) { f->ev_fill[k] = sh.ev_fill[k]; f->ev_raster[k] = sh.ev_raster[k]; }
             f->hstats = sh.hstats; f->hstats_dev = sh.hstats_dev;
         }
-        f->tiles_per_cta = 1;
-        f->out_tma = 1;
-#ifdef CRB_ABLATION     // development builds only (make variants): switches read from the environment
-        if (const char *e = getenv("CRB_RASTER_CTAS")) f->raster_ctas = atoi(e);
-        if (const char *e = getenv("CRB_TILES_PER_CTA")) { int k = atoi(e); if (k >= 1 && k <= 64) f->tiles_per_cta = k; }
-        if (const char *e = getenv("CRB_NO_TMA")) f->use_tma = atoi(e) ? 0 : 1;
-        if (const char *e = getenv("CRB_OUT_TMA")) f->out_tma = atoi(e);
-        if (const char *e = getenv("CRB_DEBUG_SKIP")) f->dbg_flags = ((unsigned)atoi(e) & 31u) << 16;
-#endif
     }
     *out = f;
     return CRB_OK;
@@ -3457,7 +3311,6 @@ int crb_set_option(crb_filler *f, int option, int value)
     switch (option) {
     case CRB_OPT_CHUNK_PIPELINE: f->chunk_pipeline = value ? 1 : 0; return CRB_OK;
     case CRB_OPT_TMA: f->use_tma = value ? 1 : 0; return CRB_OK;
-    case CRB_OPT_TMA_ROWS: f->out_tma = (value == 2) ? 2 : (value ? 1 : 0); return CRB_OK;
     case CRB_OPT_RASTER_CTAS: f->raster_ctas = value > 0 ? value : 0; return CRB_OK;
     case CRB_OPT_SPLIT_HEAVY: f->split_heavy = value ? 1 : 0; return CRB_OK;
     case CRB_OPT_WIDE_KERNEL: f->wide_kernel = value ? 1 : 0; return CRB_OK;

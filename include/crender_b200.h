@@ -218,13 +218,10 @@ int crb_render_host(crb_filler *f, const float *v, const float *c, const float *
 
 /* Tuning switches (defaults: all on).  CRB_OPT_CHUNK_PIPELINE: crb_render_views runs the setup / binning kernels of launch
  * i+1 on an internal stream beside the rasterizer of launch i (two workspace sets).  CRB_OPT_TMA: tensor-map (TMA box) stores
- * for the fused clear and the shaded rows where the layout allows.  Results do not depend on any of them. */
+ * for the fused clear where the layout allows.  Results do not depend on any of them.  (Option 3 is retired: it is refused
+ * as unknown.) */
 #define CRB_OPT_CHUNK_PIPELINE 1
 #define CRB_OPT_TMA 2
-#define CRB_OPT_TMA_ROWS 3   /* shaded colour / normal rows of busy tiles as TMA boxes (1), staged 16-byte vector stores (0) or
-                                12-byte stores straight from registers (2).  Only builds with -DCRB_LARGE_OUT_STAGE have a rasterizer
-                                shape that stages rows (24 KB of shared memory per CTA); the shipped shapes store from registers
-                                whatever this says -- smaller CTAs without the staging measured 12-15 % faster (DESIGN 6c) */
 #define CRB_OPT_BAND_PREPASS 4   /* band-sharded fillers (crb_set_band): a streaming pre-pass lists the 256-triangle chunks that
                                     can reach the band, and the setup / binning kernels visit only those (1, default) */
 #define CRB_OPT_RASTER_CTAS 5    /* > 0: fixed k_raster grid (a grid smaller than the busy tiles makes every CTA walk several tiles);

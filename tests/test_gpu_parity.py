@@ -541,7 +541,7 @@ def test_orbit_views_at_1024_equal_reference_goldens(Filler, trex):
             (info["z"], info["color"], info["normals"]), k
 
 
-@pytest.mark.parametrize("mode", ["tma", "tma_vec_rows", "tma_direct_rows", "plain", "tiny_grid", "tma_tiny_grid"])
+@pytest.mark.parametrize("mode", ["tma", "plain", "tiny_grid", "tma_tiny_grid"])
 @pytest.mark.parametrize("size", [(96, 128), (100, 76), (50, 36), (257, 388), (64, 30)])
 def test_fused_clear_store_paths(mode, size, Filler, O):
     """clear()+render takes the store path the layout allows: TMA boxes (rows that are 16-byte multiples), clipped by
@@ -553,7 +553,6 @@ def test_fused_clear_store_paths(mode, size, Filler, O):
         m = random_scene(seed, T=300)
         g, o = Filler(h, w, fov=60.0), O.OracleFiller(h, w, fov=60.0)
         g.set_option(_lib.CRB_OPT_TMA, 0 if mode in ("plain", "tiny_grid") else 1)
-        g.set_option(_lib.CRB_OPT_TMA_ROWS, {"tma_vec_rows": 0, "tma_direct_rows": 2}.get(mode, 1))
         if "tiny_grid" in mode:
             g.set_option(_lib.CRB_OPT_RASTER_CTAS, 3)
         g.render_model(random_scene(seed + 50, T=40))      # stale contents the fused clear must wipe
@@ -713,6 +712,14 @@ def test_chunk_pipeline_and_tma_switches_do_not_change_results(Filler, trex):
         else:
             for k in ref:
                 assert np.array_equal(ref[k], got[k]), (pipe, tma, k)
+
+
+def test_retired_option_number_is_refused(Filler):
+    """Option 3 (the retired shaded-row store switch) is unknown to crb_set_option: it is refused, never silently accepted."""
+    from cython3dmodelrenderer_b200 import _lib
+    f = Filler(64, 64, fov=45.0)
+    assert f._L.crb_set_option(f._handle, 3, 1) == _lib.CRB_ERR_INVALID
+    _lib.check(f._L.crb_set_option(f._handle, _lib.CRB_OPT_TMA, 1))      # the numbers around it still work
 
 
 def test_integration_stub_flow_without_torch(O, trex):

@@ -26,7 +26,7 @@ def phase_ranges():
     ev = find(r"const bool flush =", pub)
     left = find(r"if \(b\) \{\s+// what is left", ev)
     shade = find(r"---- deferred shading", left)
-    out = find(r"if \(DBG\(F, FLAG_DBG_NOOUT\)\) return;", shade)
+    out = find(r"^\s+PH\(7\);", shade)
     end = find(r"^// The fused clear through TMA", out)
     kr = find(r"^__global__ void __launch_bounds__\(C::RT, C::MIN_CTAS\) k_raster")
     kend = find(r"^// The two shapes of the tile rasterizer", kr)
@@ -44,7 +44,7 @@ def phase_ranges():
             ("exact pass", [(ev, left - 1), (dv, dve - 1), (km, kme - 1), (dk, dke - 1)]),
             ("queue leftovers", [(left, shade - 1)]),
             ("shading", [(shade, out - 1), (sf, sfe - 1)]),
-            ("row output (TMA / vector stores)", [(out, end - 1)])]
+            ("row output (staged uint8 image)", [(out, end - 1)])]
 
 
 def run(cmd):

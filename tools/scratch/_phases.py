@@ -25,7 +25,7 @@ for _ in range(N):
 torch.cuda.synchronize()
 _lib.check(f._L.crb_phase_cycles(ph, 1))
 names = {0: "head+clears", 2: "keys init / chunk barrier", 3: "staging+scan+owner", 4: "barrier after staging", 5: "row loop (visibility)",
-         6: "barrier before shading", 7: "shading loop", 8: "fence+barrier", 9: "row output", 10: "final tma wait"}
+         6: "barrier before shading", 7: "shading loop", 9: "uint8 row output"}
 tot = sum(ph)
 print(f"{name} {res}^2 x {V} views: warp-cycles per view {tot / N / V:.0f}")
 for k, nm in names.items():
