@@ -44,7 +44,8 @@ namespace {
 constexpr int TW = 32;          // tile width in pixels  (one 128-byte line of z, three of colour / normals)
 constexpr int TH = 32;          // tile height in pixels
 constexpr int NT = 256;         // threads per CTA in every kernel but the tile rasterizer (its CTA shapes: RasterShape, further down)
-constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR;   // per-pixel texturing and its modes
+constexpr unsigned CRB_TEX_FLAGS = CRB_TEXTURE | CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR |
+                                   CRB_TEX_REPEAT | CRB_TEX_MIRROR;   // per-pixel texturing and its modes
 constexpr unsigned SPLIT_N = 48;  // single-view launches: tiles with more triangles than this are rasterized by SPLIT_BANDS CTAs, 8 rows each
 constexpr int SPLIT_BANDS = 4;
 constexpr unsigned CE = 4;        // every CE-th CTA of k_raster is a clear CTA (power of two)
@@ -259,9 +260,11 @@ __device__ __forceinline__ int f32_to_i32_x86(float x)
 
 // Shading mode of shade_fragment / k_raster / k_shade_atomic: per-vertex colours (TEX_NONE), or per-pixel texturing
 // (CRB_TEXTURE) with nearest (model.py:147-150's rule) or bilinear (CRB_TEX_BILINEAR) sampling, either of them with
-// TEX_PERSP (CRB_TEX_PERSPECTIVE) added, and trilinear mip filtering (CRB_TEX_TRILINEAR) with or without it.  All are
-// compile-time: a uniform branch on the divide costs the nearest instantiation of the large rasterizer shape a register.
-enum TexMode { TEX_NONE = 0, TEX_NEAREST = 1, TEX_BILINEAR = 2, TEX_PERSP = 4, TEX_TRILINEAR = 8 };
+// TEX_PERSP (CRB_TEX_PERSPECTIVE) added, and trilinear mip filtering (CRB_TEX_TRILINEAR) with or without it; each of them
+// addresses the texture clamped to its border texels, or with TEX_REPEAT / TEX_MIRROR (CRB_TEX_REPEAT / CRB_TEX_MIRROR) wrapped.
+// All are compile-time: a uniform branch on the divide costs the nearest instantiation of the large rasterizer shape a register.
+enum TexMode { TEX_NONE = 0, TEX_NEAREST = 1, TEX_BILINEAR = 2, TEX_PERSP = 4, TEX_TRILINEAR = 8, TEX_REPEAT = 16, TEX_MIRROR = 32 };
+constexpr int TEX_WRAP = TEX_REPEAT | TEX_MIRROR;
 
 // Texel (r, c) of a packed [th, tw] level as float B, G, R
 __device__ __forceinline__ void texel_bgr(const uint32_t *tex, int tw, int r, int c, float t[3])
@@ -270,19 +273,55 @@ __device__ __forceinline__ void texel_bgr(const uint32_t *tex, int tw, int r, in
     t[0] = (float)(p & 255u); t[1] = (float)((p >> 8) & 255u); t[2] = (float)(p >> 16);
 }
 
+// CRB_TEX_REPEAT / CRB_TEX_MIRROR (DESIGN 2): the float a texel index is floored from, with NaN and |x| >= 2^31 taken as 0,
+// so that floor(x) and floor(x) + 1 fit int32
+__device__ __forceinline__ float wrap_arg(float x)
+{
+    return fabsf(x) < 2147483648.0f ? x : 0.0f;
+}
+
+// Index k wrapped into [0, n), n >= 1 (floor modulo): repeat k mod n; mirror m = k mod 2n, then m < n ? m : 2n-1 - m.
+// For k < 0, k mod N = N-1 - (~k mod N) with ~k = -1 - k >= 0, so one unsigned 32-bit remainder serves (2n < 2^32).  Mirror
+// is symmetric about -1/2 (index(k) = index(-1 - k)), so it needs no sign fix-up.
+template <int TEX>
+__device__ __forceinline__ int wrap_texel(int k, int n)
+{
+    const unsigned a = k < 0 ? ~(unsigned)k : (unsigned)k;
+    if (TEX & TEX_REPEAT) {
+        const unsigned r = a % (unsigned)n;
+        return (int)(k < 0 ? (unsigned)n - 1u - r : r);
+    }
+    const unsigned n2 = 2u * (unsigned)n, m = a % n2;
+    return (int)(m < (unsigned)n ? m : n2 - 1u - m);
+}
+
 // CRB_TEX_BILINEAR (DESIGN 2): texel centres at (col + 0.5) / tw, (row + 0.5) / th -- those of the nearest rule -- clamped to
-// the border texels.  float32, one rounding per operation, no FMA (the file is built with -fmad=false).
+// the border texels, or with TEX_REPEAT / TEX_MIRROR in TEX wrapped by wrap_texel.  float32, one rounding per operation, no
+// FMA (the file is built with -fmad=false).
+template <int TEX>
 __device__ __forceinline__ void sample_bilinear(const uint32_t *tex, int H, int W, float u, float v, float c[3])
 {
     const float tw = (float)W, th = (float)H;
     float sx = u * tw - 0.5f, sy = (1.0f - v) * th - 0.5f;
-    sx = fminf(fmaxf(sx, -1.0f), tw);       // fmaxf(NaN, -1) = -1
-    sy = fminf(fmaxf(sy, -1.0f), th);
+    if (TEX & TEX_WRAP) {
+        sx = wrap_arg(sx);
+        sy = wrap_arg(sy);
+    } else {
+        sx = fminf(fmaxf(sx, -1.0f), tw);       // fmaxf(NaN, -1) = -1
+        sy = fminf(fmaxf(sy, -1.0f), th);
+    }
     const float x0 = floorf(sx), y0 = floorf(sy);
     const float fx = sx - x0, fy = sy - y0, gx = 1.0f - fx, gy = 1.0f - fy;     // (sx - x0 is exact unless -1 < sx < 0)
-    const long long ix = (long long)x0, iy = (long long)y0;                      // in [-1, 2^31]
-    const int c0 = (int)min(max(ix, 0ll), (long long)W - 1), c1 = (int)min(max(ix + 1, 0ll), (long long)W - 1);
-    const int r0 = (int)min(max(iy, 0ll), (long long)H - 1), r1 = (int)min(max(iy + 1, 0ll), (long long)H - 1);
+    int c0, c1, r0, r1;
+    if (TEX & TEX_WRAP) {
+        const int ix = (int)x0, iy = (int)y0;                                    // |x0| <= 2^31 - 128
+        c0 = wrap_texel<TEX>(ix, W); c1 = wrap_texel<TEX>(ix + 1, W);
+        r0 = wrap_texel<TEX>(iy, H); r1 = wrap_texel<TEX>(iy + 1, H);
+    } else {
+        const long long ix = (long long)x0, iy = (long long)y0;                  // in [-1, 2^31]
+        c0 = (int)min(max(ix, 0ll), (long long)W - 1); c1 = (int)min(max(ix + 1, 0ll), (long long)W - 1);
+        r0 = (int)min(max(iy, 0ll), (long long)H - 1); r1 = (int)min(max(iy + 1, 0ll), (long long)H - 1);
+    }
     float t00[3], t01[3], t10[3], t11[3];
     texel_bgr(tex, W, r0, c0, t00); texel_bgr(tex, W, r0, c1, t01);
     texel_bgr(tex, W, r1, c0, t10); texel_bgr(tex, W, r1, c1, t11);
@@ -317,6 +356,8 @@ __device__ __forceinline__ const uint32_t *mip_step(const uint32_t *p, int &h, i
 
 // CRB_TEX_TRILINEAR: bilinear samples of levels l0 = floor(lc) and l1 = min(l0 + 1, L-1), blended c0*(1 - fr) + c1*fr,
 // fr = lc - l0.  With fr == 0 that is c0 bit for bit (texels are finite and >= 0), so the second level is not read.
+// Both samples address their own level with TEX's wrap mode.
+template <int TEX>
 __device__ __forceinline__ void sample_trilinear(const Frame &F, float lc, float u, float v, float c[3])
 {
     const int l0 = (int)floorf(lc);
@@ -324,11 +365,11 @@ __device__ __forceinline__ void sample_trilinear(const Frame &F, float lc, float
     int h = F.texH, w = F.texW;
     const uint32_t *p = F.tex;
     for (int l = 0; l < l0; ++l) p = mip_step(p, h, w);
-    sample_bilinear(p, h, w, u, v, c);
+    sample_bilinear<TEX>(p, h, w, u, v, c);
     if (fr != 0.0f) {   // then lc < L-1, so l1 = l0 + 1
         p = mip_step(p, h, w);
         float c1[3];
-        sample_bilinear(p, h, w, u, v, c1);
+        sample_bilinear<TEX>(p, h, w, u, v, c1);
 #pragma unroll
         for (int k = 0; k < 3; ++k) c[k] = c[k] * (1.0f - fr) + c1[k] * fr;
     }
@@ -374,9 +415,13 @@ __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, 
                 ux = (ux - u * wx) / c[2]; vx = (vx - v * wx) / c[2];
                 uy = (uy - u * wy) / c[2]; vy = (vy - v * wy) / c[2];
             }
-            sample_trilinear(F, mip_lod(F, ux, vx, uy, vy), u, v, c);
+            sample_trilinear<TEX>(F, mip_lod(F, ux, vx, uy, vy), u, v, c);
         } else if (TEX & TEX_BILINEAR) {
-            sample_bilinear(F.tex, F.texH, F.texW, u, v, c);
+            sample_bilinear<TEX>(F.tex, F.texH, F.texW, u, v, c);
+        } else if (TEX & TEX_WRAP) {   // row = wrap(floor((1 - v) * th)), col = wrap(floor(u * tw)): the clamp rule's products
+            const int row = wrap_texel<TEX>((int)floorf(wrap_arg((1.0f - v) * (float)F.texH)), F.texH);
+            const int col = wrap_texel<TEX>((int)floorf(wrap_arg(u * (float)F.texW)), F.texW);
+            texel_bgr(F.tex, F.texW, row, col, c);
         } else {   // row = clip(int32((1 - v) * th), 0, th-1), col = clip(int32(u * tw), 0, tw-1); BGR as cv2.imread gives it
             const int row = clipi(f32_to_i32_x86((1.0f - v) * (float)F.texH), 0, F.texH - 1);
             const int col = clipi(f32_to_i32_x86(u * (float)F.texW), 0, F.texW - 1);
@@ -2122,12 +2167,17 @@ void fill_frame(const crb_filler *f, Frame *F, int set = 0)
     F->texW = f->tex_w;
 }
 
-// CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR and CRB_TEX_TRILINEAR are modes of CRB_TEXTURE, which needs a bound texture;
-// CRB_TEX_TRILINEAR needs a bound mip chain and excludes CRB_TEX_BILINEAR
+// CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR, CRB_TEX_TRILINEAR, CRB_TEX_REPEAT and CRB_TEX_MIRROR are modes of CRB_TEXTURE, which
+// needs a bound texture; CRB_TEX_TRILINEAR needs a bound mip chain and excludes CRB_TEX_BILINEAR; the two wrap modes exclude
+// each other
 int check_texture(const crb_filler *f, unsigned flags)
 {
     if ((flags & (CRB_TEX_PERSPECTIVE | CRB_TEX_BILINEAR | CRB_TEX_TRILINEAR)) && !(flags & CRB_TEXTURE))
         return fail(CRB_ERR_INVALID, "CRB_TEX_PERSPECTIVE / CRB_TEX_BILINEAR / CRB_TEX_TRILINEAR need CRB_TEXTURE");
+    if ((flags & (CRB_TEX_REPEAT | CRB_TEX_MIRROR)) && !(flags & CRB_TEXTURE))
+        return fail(CRB_ERR_INVALID, "CRB_TEX_REPEAT / CRB_TEX_MIRROR need CRB_TEXTURE");
+    if ((flags & CRB_TEX_REPEAT) && (flags & CRB_TEX_MIRROR))
+        return fail(CRB_ERR_INVALID, "CRB_TEX_REPEAT and CRB_TEX_MIRROR exclude each other");
     if ((flags & CRB_TEX_BILINEAR) && (flags & CRB_TEX_TRILINEAR))
         return fail(CRB_ERR_INVALID, "CRB_TEX_BILINEAR and CRB_TEX_TRILINEAR exclude each other");
     if ((flags & CRB_TEXTURE) && !f->tex) return fail(CRB_ERR_STATE, "CRB_TEXTURE: no texture bound (crb_bind_texture)");
@@ -2267,28 +2317,34 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     return CRB_OK;
 }
 
-// shading instantiation of a frame: per-vertex colours, or per-pixel texturing with its filter and interpolation
+// shading instantiation of a frame: per-vertex colours, or per-pixel texturing with its filter, interpolation and wrap mode
 int tex_mode(const Frame &F)
 {
     if (!(F.flags & CRB_TEXTURE)) return TEX_NONE;
     const int filter = (F.flags & CRB_TEX_TRILINEAR) ? TEX_TRILINEAR : (F.flags & CRB_TEX_BILINEAR) ? TEX_BILINEAR : TEX_NEAREST;
-    return filter | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
+    const int wrap = (F.flags & CRB_TEX_REPEAT) ? TEX_REPEAT : (F.flags & CRB_TEX_MIRROR) ? TEX_MIRROR : 0;
+    return filter | wrap | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
 }
 
 // Calls fn(std::integral_constant<int, MODE>()) with the frame's tex_mode as a compile-time constant: the one list of the shading
-// instantiations of k_raster and k_shade_atomic
+// instantiations of k_raster and k_shade_atomic (per-vertex, then 3 filters x 2 interpolations x 3 addressing modes)
 template <class Fn>
 void with_tex_mode(const Frame &F, Fn &&fn)
 {
+#define CRB_TEX_CASES(W)                                                                                               \
+    case TEX_NEAREST | (W): fn(std::integral_constant<int, TEX_NEAREST | (W)>()); break;                               \
+    case TEX_NEAREST | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_NEAREST | TEX_PERSP | (W)>()); break;       \
+    case TEX_BILINEAR | (W): fn(std::integral_constant<int, TEX_BILINEAR | (W)>()); break;                             \
+    case TEX_BILINEAR | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_BILINEAR | TEX_PERSP | (W)>()); break;     \
+    case TEX_TRILINEAR | (W): fn(std::integral_constant<int, TEX_TRILINEAR | (W)>()); break;                           \
+    case TEX_TRILINEAR | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_TRILINEAR | TEX_PERSP | (W)>()); break;
     switch (tex_mode(F)) {
-    case TEX_NEAREST: fn(std::integral_constant<int, TEX_NEAREST>()); break;
-    case TEX_NEAREST | TEX_PERSP: fn(std::integral_constant<int, TEX_NEAREST | TEX_PERSP>()); break;
-    case TEX_BILINEAR: fn(std::integral_constant<int, TEX_BILINEAR>()); break;
-    case TEX_BILINEAR | TEX_PERSP: fn(std::integral_constant<int, TEX_BILINEAR | TEX_PERSP>()); break;
-    case TEX_TRILINEAR: fn(std::integral_constant<int, TEX_TRILINEAR>()); break;
-    case TEX_TRILINEAR | TEX_PERSP: fn(std::integral_constant<int, TEX_TRILINEAR | TEX_PERSP>()); break;
+    CRB_TEX_CASES(0)
+    CRB_TEX_CASES(TEX_REPEAT)
+    CRB_TEX_CASES(TEX_MIRROR)
     default: fn(std::integral_constant<int, TEX_NONE>());
     }
+#undef CRB_TEX_CASES
 }
 
 // raster + shade (+ fused clear) of the frame run_prep binned

@@ -127,6 +127,9 @@ class AdvancedPixelBufferFiller:
     bilinear blend of four (CRB_TEX_BILINEAR), or a blend of bilinear samples of the two levels of the texture's mip chain that
     the pixel's footprint in the texture selects (CRB_TEX_TRILINEAR; the chain is built on the device when the texture is bound),
     from texture coordinates interpolated affinely in screen space or perspective-correctly (CRB_TEX_PERSPECTIVE).
+    `texture_wrap="clamp" | "repeat" | "mirror"` -- how those renders address texels of coordinates outside [0, 1]: the border
+    texel (the default), the texture repeated (CRB_TEX_REPEAT), or repeated mirrored every other period (CRB_TEX_MIRROR), on
+    both axes and with every filter.
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -138,18 +141,22 @@ class AdvancedPixelBufferFiller:
     _view_owner = {}      # address of a host mirror handed out by get_*_buffer() -> weak reference to its filler (owner_of_views)
 
     def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None,
-                 texturing="vertex", texture_filter="nearest", perspective_correct=False):
+                 texturing="vertex", texture_filter="nearest", perspective_correct=False, texture_wrap="clamp"):
         if texturing not in ("vertex", "pixel"):
             raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
         if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear", "trilinear"):
             raise ValueError(f"texture_filter must be 'nearest', 'bilinear' or 'trilinear', got {texture_filter!r}")
         if not isinstance(perspective_correct, (bool, np.bool_)):
             raise ValueError(f"perspective_correct must be True or False, got {perspective_correct!r}")
+        if not isinstance(texture_wrap, str) or texture_wrap not in ("clamp", "repeat", "mirror"):
+            raise ValueError(f"texture_wrap must be 'clamp', 'repeat' or 'mirror', got {texture_wrap!r}")
         self._texturing = texturing
         # render flags of every textured frame (kept in the arguments of a frame, so a redraw of it samples the same way)
         self._tex_flags = (_lib.CRB_TEXTURE | (_lib.CRB_TEX_BILINEAR if texture_filter == "bilinear" else 0)
                            | (_lib.CRB_TEX_TRILINEAR if texture_filter == "trilinear" else 0)
-                           | (_lib.CRB_TEX_PERSPECTIVE if perspective_correct else 0))
+                           | (_lib.CRB_TEX_PERSPECTIVE if perspective_correct else 0)
+                           | (_lib.CRB_TEX_REPEAT if texture_wrap == "repeat" else 0)
+                           | (_lib.CRB_TEX_MIRROR if texture_wrap == "mirror" else 0))
         # (source texture, its version, packed uint32 CUDA tensor: [th,tw], or with "trilinear" the whole mip chain) bound to the filler
         self._tex = None
         self._uv = None               # (texture coordinates, their triangle indices, UV-by-triangle CUDA tensor [T,3,3])
@@ -462,8 +469,8 @@ class AdvancedPixelBufferFiller:
         """Render [T,3,3] float32 arrays.  numpy inputs are staged through pinned memory and copied H2D;
         torch CUDA tensors are used in place (device-resident inputs).  `texture` (uint8 [h,w,3], BGR; NumPy or torch):
         per-pixel texturing -- `c` then holds texture coordinates by triangle, [T,3,3] (third component ignored) or
-        [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE), sampled as the constructor's `texture_filter` and
-        `perspective_correct` say."""
+        [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE), sampled as the constructor's `texture_filter`,
+        `perspective_correct` and `texture_wrap` say."""
         torch = self._torch
         flags = _lib.CRB_PATH_ATOMIC if path == "atomic" else 0
         if texture is not None:

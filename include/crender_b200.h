@@ -97,6 +97,24 @@ extern "C" {
                                       colour = c0*(1 - fr) + c1*fr with c0, c1 CRB_TEX_BILINEAR's blend on levels l0, l1.  float32, one
                                       rounding per operation.  Where lc == 0 this is CRB_TEX_BILINEAR bit for bit.  Without CRB_TEXTURE,
                                       or with CRB_TEX_BILINEAR: CRB_ERR_INVALID; no chain bound: CRB_ERR_STATE. */
+#define CRB_TEX_REPEAT 16384u      /* with CRB_TEXTURE: texture coordinates outside [0, 1] repeat the texture (wrap modes, DESIGN 2) */
+#define CRB_TEX_MIRROR 32768u      /* with CRB_TEXTURE: texture coordinates outside [0, 1] repeat it mirrored every other period.
+   The rule of both wrap modes (DESIGN 2 states it word for word the same):
+   Neither bit means clamp, which is the behaviour of CRB_TEXTURE and its filters above, bit for bit. F() is float32; every
+   float operation is one binary32 rounding with no FMA; integer arithmetic is exact.
+   - Index of a float: ifloor(x): if x is NaN or |x| >= 2^31, x := F(0); then k = int(floor(x)), so k and k + 1 fit in int32.
+   - Wrap of an integer index k into [0, n): repeat: k mod n with floor modulo (Python's %, np.mod), in [0, n); mirror:
+     m = k mod 2n, then m if m < n, else 2n - 1 - m (2n can exceed int32).
+   - Nearest: col = wrap(ifloor(u*F(tw)), tw), row = wrap(ifloor((F(1) - v)*F(th)), th) -- the clamp rule's products,
+     floored instead of truncated.  Where 0 <= u*tw < tw and 0 <= (1-v)*th < th both modes pick the clamp texel.
+   - Bilinear: sx = u*F(tw) - F(0.5), sy = (F(1) - v)*F(th) - F(0.5), with no [-1, tw] clamp: NaN or |s| >= 2^31 becomes
+     F(0).  x0 = floor(sx), fx = sx - x0, gx = F(1) - fx; c0 = wrap(int(x0), tw), c1 = wrap(int(x0) + 1, tw); rows alike.
+     The blend is CRB_TEX_BILINEAR's.  Where 0 <= sx <= tw-1 and 0 <= sy <= th-1 this is clamp-bilinear bit for bit; at
+     texel centres it is wrap-nearest.
+   - Trilinear: the level of detail and the chain are unchanged; both level samples use the wrapped bilinear rule, each
+     with its own level's (th_l, tw_l).  Where fr == 0 the second level is still not read.
+   - Both bits are independent of CRB_TEX_PERSPECTIVE and combine with every filter; one mode applies to both axes.
+   - Both bits together, or either without CRB_TEXTURE: CRB_ERR_INVALID on every render entry point. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u
