@@ -136,6 +136,18 @@ struct Frame {
     int texH, texW;
 };
 
+// A Frame with the id outputs (crb_bind_id_buffers, crb_render_views_ids; DESIGN 2): per view slab tri_id [rows,W] int32 and
+// bary [rows,W,3] float32, either of them nullptr when not wanted.  Only the IDS instantiations of k_raster / k_shade_atomic take
+// it: the members follow texW, so every other member keeps its offset, and the kernels without id outputs keep their parameter
+// block (their keybuf / tensor-map parameters would move if Frame itself grew).
+struct FrameIds : Frame {
+    int32_t *triId;
+    float *bary;
+    int idBase;          // tri_id = idBase + the winner's index in the call's [T,3,3] arrays
+};
+template <bool IDS>
+using FrameOf = typename std::conditional<IDS, FrameIds, Frame>::type;
+
 // ------------------------------------------------------------------------------------------------------------
 // device arithmetic shared by every path.  Operation order restates the reference exactly.
 // ------------------------------------------------------------------------------------------------------------
@@ -381,9 +393,11 @@ __device__ __forceinline__ void sample_trilinear(const Frame &F, float lc, float
 // TEX != TEX_NONE (per-pixel texturing, CRB_TEXTURE; an extension, DESIGN 2): the interpolated colour slots hold (u, v, -), or
 // with CRB_TEX_PERSPECTIVE (U, V, W) = (u/z, v/z, 1/z), divided back to u = U/W, v = V/W; the texel they name (nearest) or
 // the bilinear blend of the four around them replaces the colour before the fused Guro pass.  Compiled in only where asked
-// for, so the per-vertex instantiations are the code they were.
-template <int TEX = TEX_NONE>
-__device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, float px, float py, float &z, float c[3], float n[3])
+// for, so the per-vertex instantiations are the code they were.  BC (the id outputs): `bc` receives (b1, b2, b3), the
+// barycentrics everything is interpolated with; compile-time, so that the instantiations without id outputs are the code they were.
+template <int TEX = TEX_NONE, bool BC = false>
+__device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, float px, float py, float &z, float c[3], float n[3],
+                                               float bc[3] = nullptr)
 {
     const float4 A = R[S_A], B = R[S_B], C = R[S_C];
     // x0=A.x y0=A.y x1=A.z y1=A.w x2=B.x y2=B.y z0=B.z z1=B.w z2=C.x  l03=C.y l13=C.z l23=C.w
@@ -391,6 +405,7 @@ __device__ __forceinline__ bool shade_fragment(const Frame &F, const float4 *R, 
     const float n2 = (B.x - A.x) * (py - A.y) - (B.y - A.y) * (px - A.x);
     const float n3 = (A.x - A.z) * (py - A.w) - (A.y - A.w) * (px - A.z);
     const float b1 = n1 / C.y, b2 = n2 / C.z, b3 = n3 / C.w;
+    if constexpr (BC) { bc[0] = b1; bc[1] = b2; bc[2] = b3; }
     if (b1 < 0.0f || b2 < 0.0f || b3 < 0.0f) return false;
     z = (B.z * b1 + B.w * b2) + C.x * b3;
     if (z != z) return false;
@@ -1131,6 +1146,14 @@ struct __align__(64) TMaps {
     CUtensorMap zt, ct, nt;
     unsigned use;
 };
+// ... and of the id outputs, for the IDS instantiations: tri_id [view][row][x] (an int32 array described as float32: TMA copies
+// bits, the clear pattern is 0xFFFFFFFF = -1) and bary [view][row][3x], use bits ID_TRI / ID_BARY
+constexpr unsigned ID_TRI = 8u, ID_BARY = 16u;
+struct TMapsIds : TMaps {
+    CUtensorMap it, bt;
+};
+template <bool IDS>
+using TMapsOf = typename std::conditional<IDS, TMapsIds, TMaps>::type;
 
 __device__ __forceinline__ void tma_store_box(const CUtensorMap *m, const void *smem, int cx, int cy, int cv)
 {
@@ -1194,6 +1217,8 @@ struct __align__(128) TileSmem {
         struct {                              // clear CTAs only: the constant pattern their TMA boxes are stored from
             float z[CLEAR_ROWS * TW];         //   Z_INIT
             float c[CLEAR_ROWS * TW * 3];     //   background colour = 0 (background_color) = the cleared normals: one pattern serves both
+                                              //   (and the cleared barycentrics of the IDS instantiations)
+            unsigned id[CLEAR_ROWS * TW];     //   IDS instantiations: tri_id -1 (last, so z and c keep their offsets)
         } pat;
     } u;
     unsigned long long keys[TH * KEY_STRIDE];
@@ -1251,6 +1276,31 @@ __device__ __forceinline__ void write_clear_tile(const Frame &F, unsigned skip, 
     }
 }
 
+// The same for the id outputs (IDS instantiations): tri_id -1, bary (0, 0, 0)
+template <int NTH>
+__device__ __forceinline__ void write_clear_ids(const FrameIds &F, int view, int x0, int yl0, int tw, int th)
+{
+    const long long slab = (long long)view * F.slabPixels;
+    if (tw == TW && (F.W & 3) == 0) {       // 16-byte stores, as write_clear_tile's
+        const int q = threadIdx.x & 7;
+        for (int r = threadIdx.x >> 3; r < th; r += NTH / 8) {
+            const long long rowpix = slab + (long long)(yl0 + r) * F.W + x0;
+            if (F.triId) reinterpret_cast<int4 *>(F.triId + rowpix)[q] = make_int4(-1, -1, -1, -1);
+            if (F.bary) {
+                float4 *o = reinterpret_cast<float4 *>(F.bary + rowpix * 3);
+                o[q] = make_float4(0.f, 0.f, 0.f, 0.f); o[q + 8] = make_float4(0.f, 0.f, 0.f, 0.f); o[q + 16] = make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        }
+    } else {
+        for (int i = threadIdx.x; i < th * tw; i += NTH) {
+            const int r = i / tw, xx = i % tw;
+            const long long p = slab + (long long)(yl0 + r) * F.W + x0 + xx;
+            if (F.triId) F.triId[p] = -1;
+            if (F.bary) { F.bary[p * 3] = 0.f; F.bary[p * 3 + 1] = 0.f; F.bary[p * 3 + 2] = 0.f; }
+        }
+    }
+}
+
 // Conservative bound of the pixels of one row that can pass `bar_k >= 0`, for one barycentric.
 // Reference (mu:34): num = fl(fl(l1*fl(py-a)) - fl(l2*fl(px-b))), inside <=> !(num/l3 < 0).  With the sign-normalised
 // (l1', l2', d' > 0) form, inside => num' >= -REJ_EPS (k_fill).  num' differs from the real-valued
@@ -1282,9 +1332,10 @@ constexpr unsigned PK_SPAN = 8u;     // FL_SPAN
 constexpr unsigned PK_FAST = 16u;    // FL_SPAN and FL_FDIV: div_rn_by() applies whenever the numerators are >= 2^-40
 constexpr int PK_XA = 8, PK_XB = 14, PK_YT = 20;   // tile-relative rectangle: first x (6 bits), end x (6 bits), first row (5 bits)
 
-// Visibility + deferred shading of one busy tile (n triangles staged at list offset off).
-template <class C, int TEX>
-__device__ __forceinline__ void raster_tile(const Frame &F, TileSmem<C> &S_, const bool clear, const int view,
+// Visibility + deferred shading of one busy tile (n triangles staged at list offset off).  IDS: the winner's id and
+// barycentrics are stored beside the other outputs.
+template <class C, int TEX, bool IDS>
+__device__ __forceinline__ void raster_tile(const FrameOf<IDS> &F, TileSmem<C> &S_, const bool clear, const int view,
                                             const int tx, const int ty, const unsigned n, const unsigned off, const int rowLo, const int rowHi)
 {
     constexpr int RT = C::RT, CH = C::CH, FQ = C::FQ;
@@ -1527,14 +1578,17 @@ __device__ __forceinline__ void raster_tile(const Frame &F, TileSmem<C> &S_, con
         if (yy < rowLo || yy >= th || xx >= tw) continue;
         const unsigned long long key = S.keys[yy * KEY_STRIDE + xx];
         float z = Z_INIT, c[3] = {bg, bg, bg}, nn[3] = {0.f, 0.f, 0.f};
+        int id = -1;
+        float b[3] = {0.f, 0.f, 0.f};
         bool write = clear;
         if (key != KEY_EMPTY) {
             const unsigned tri = ~(unsigned)(key & 0xFFFFFFFFull);
-            float fz, fc[3], fn[3];
-            if (shade_fragment<TEX>(F, recv + (size_t)tri * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn)) {
+            float fz, fc[3], fn[3], fb[3];
+            if (shade_fragment<TEX, IDS>(F, recv + (size_t)tri * SREC, (float)(x0 + xx), (float)(y0 + yy), fz, fc, fn, fb)) {
                 const float zold = clear ? Z_INIT : F.z[pix];
                 if (!(fz > zold)) {  // pyx:223: drawn unless new_z > z_buffer (equal depth overwrites)
                     z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
+                    if constexpr (IDS) { id = F.idBase + (int)tri; b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
                     write = true;
                 }
             }
@@ -1543,6 +1597,10 @@ __device__ __forceinline__ void raster_tile(const Frame &F, TileSmem<C> &S_, con
             if (F.z) F.z[pix] = z;
             if (F.color) { F.color[pix * 3] = c[0]; F.color[pix * 3 + 1] = c[1]; F.color[pix * 3 + 2] = c[2]; }
             if (F.normals) { F.normals[pix * 3] = nn[0]; F.normals[pix * 3 + 1] = nn[1]; F.normals[pix * 3 + 2] = nn[2]; }
+            if constexpr (IDS) {
+                if (F.triId) F.triId[pix] = id;
+                if (F.bary) { F.bary[pix * 3] = b[0]; F.bary[pix * 3 + 1] = b[1]; F.bary[pix * 3 + 2] = b[2]; }
+            }
         }
         if (F.color_u8 && write) {
             unsigned char *o = u8stage ? S.u.u8 + p * 3 : u8_pixel(F, view, yl0 + yy, x0 + xx);
@@ -1562,8 +1620,8 @@ __device__ __forceinline__ void raster_tile(const Frame &F, TileSmem<C> &S_, con
 
 // The fused clear through TMA: one tile = three whole-tile boxes (z, colour, normals) stored from the constant pattern in
 // shared memory; the hardware clips boxes at the image edge.  Called by one lane.
-template <class C>
-__device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C> &S, unsigned t)
+template <class C, bool IDS>
+__device__ __forceinline__ void tma_clear_tile(const TMapsOf<IDS> &M, const TileSmem<C> &S, unsigned t)
 {
     constexpr int CLEAR_ROWS = C::CLEAR_ROWS;
     const int view = (int)(t >> 22), yl0 = (int)((t >> 11) & 2047u) * TH, x0 = (int)(t & 2047u) * TW;
@@ -1572,6 +1630,10 @@ __device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C>
         if (M.use & CRB_BUF_Z) tma_store_box(&M.zt, S.u.pat.z, x0, yl0 + r, view);
         if (M.use & CRB_BUF_COLOR) tma_store_box(&M.ct, S.u.pat.c, x0 * 3, yl0 + r, view);
         if (M.use & CRB_BUF_NORMALS) tma_store_box(&M.nt, S.u.pat.c, x0 * 3, yl0 + r, view);
+        if constexpr (IDS) {
+            if (M.use & ID_TRI) tma_store_box(&M.it, S.u.pat.id, x0, yl0 + r, view);
+            if (M.use & ID_BARY) tma_store_box(&M.bt, S.u.pat.c, x0 * 3, yl0 + r, view);
+        }
     }
 }
 
@@ -1583,8 +1645,8 @@ __device__ __forceinline__ void tma_clear_tile(const TMaps &M, const TileSmem<C>
 // every CTA adopting its share of the empty tiles.
 // Resident CTAs per SM follow the shape (RasterSmall 12 at 40 registers, RasterLarge 8 at up to 64, RasterWide 6 at 40); the
 // static_assert in k_raster ties each shape's shared memory to the residency its launch bounds ask for.
-template <class C, int TEX>
-__global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, const __grid_constant__ TMaps M)
+template <class C, int TEX, bool IDS>
+__global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<IDS> F, const __grid_constant__ TMapsOf<IDS> M)
 {
     constexpr int RT = C::RT, CLEAR_ROWS = C::CLEAR_ROWS;
     static_assert(sizeof(TileSmem<C>) + 1024 <= 233472 / C::MIN_CTAS, "k_raster: shared memory per CTA exceeds the residency its launch bounds assume");
@@ -1609,6 +1671,8 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
             for (int i = threadIdx.x; i < CLEAR_ROWS * TW * 3 / 4; i += RT) {
                 reinterpret_cast<float4 *>(S.u.pat.c)[i] = make_float4(bg, bg, bg, bg);       // (bg is 0.0f: also the normals' pattern)
                 if (i < CLEAR_ROWS * TW / 4) reinterpret_cast<float4 *>(S.u.pat.z)[i] = make_float4(Z_INIT, Z_INIT, Z_INIT, Z_INIT);
+                if constexpr (IDS)
+                    if (i < CLEAR_ROWS * TW / 4) reinterpret_cast<int4 *>(S.u.pat.id)[i] = make_int4(-1, -1, -1, -1);
             }
             fence_async_smem();
             __syncthreads();
@@ -1616,7 +1680,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
                 while (e < ne) {
                     const unsigned en = e + stride;
                     const unsigned tn = en < ne ? F.empty[en] : 0u;
-                    tma_clear_tile(M, S, t);
+                    tma_clear_tile<C, IDS>(M, S, t);
                     e = en; t = tn;
                 }
                 tma_commit();
@@ -1652,6 +1716,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
             const unsigned t = F.empty[e];
             const int view = (int)(t >> 22), ty = (int)((t >> 11) & 2047u), tx = (int)(t & 2047u);
             write_clear_tile<RT>(F, 0u, view, tx * TW, ty * TH, min(TW, F.W - tx * TW), min(TH, F.row1 - F.row0 - ty * TH));
+            if constexpr (IDS) write_clear_ids<RT>(F, view, tx * TW, ty * TH, min(TW, F.W - tx * TW), min(TH, F.row1 - F.row0 - ty * TH));
         }
     }
     PH(0);
@@ -1659,7 +1724,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const Frame F, co
         const uint4 cur = rec;
         if (cta != first) __syncthreads();                  // the previous tile is done with shared memory
         if (cta + stride < nb) rec = lst[cta + stride];     // the next tile's record arrives while this one is rasterized
-        raster_tile<C, TEX>(F, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
+        raster_tile<C, TEX, IDS>(F, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
                     (int)(cur.w & 255u), (int)(cur.w >> 8));
     }
 }
@@ -1715,24 +1780,27 @@ __global__ void __launch_bounds__(NT) k_raster_atomic(const Frame F, unsigned lo
     }
 }
 
-template <int TEX>
-__global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned long long *keybuf)
+template <int TEX, bool IDS>
+__global__ void __launch_bounds__(NT) k_shade_atomic(const FrameOf<IDS> F, unsigned long long *keybuf)
 {
     const long long pix = (long long)blockIdx.x * NT + threadIdx.x;
     if (pix >= F.slabPixels) return;
     const unsigned long long key = keybuf[pix];
     const bool clear = (F.flags & CRB_CLEAR_FIRST) != 0;
     float z = Z_INIT, c[3] = {0.f, 0.f, 0.f}, nn[3] = {0.f, 0.f, 0.f};
+    int id = -1;
+    float b[3] = {0.f, 0.f, 0.f};
     bool write = clear;
     if (key != KEY_EMPTY) {
         keybuf[pix] = KEY_EMPTY;
         const unsigned tri = ~(unsigned)(key & 0xFFFFFFFFull);
         const int y = F.row0 + (int)(pix / F.W), x = (int)(pix % F.W);
-        float fz, fc[3], fn[3];
-        if (shade_fragment<TEX>(F, F.shrec + (size_t)tri * SREC, (float)x, (float)y, fz, fc, fn)) {
+        float fz, fc[3], fn[3], fb[3];
+        if (shade_fragment<TEX, IDS>(F, F.shrec + (size_t)tri * SREC, (float)x, (float)y, fz, fc, fn, fb)) {
             const float zold = clear ? Z_INIT : F.z[pix];
             if (!(fz > zold)) {
                 z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
+                if constexpr (IDS) { id = F.idBase + (int)tri; b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
                 write = true;
             }
         }
@@ -1741,6 +1809,10 @@ __global__ void __launch_bounds__(NT) k_shade_atomic(const Frame F, unsigned lon
     F.z[pix] = z;
     F.color[pix * 3] = c[0]; F.color[pix * 3 + 1] = c[1]; F.color[pix * 3 + 2] = c[2];
     F.normals[pix * 3] = nn[0]; F.normals[pix * 3 + 1] = nn[1]; F.normals[pix * 3 + 2] = nn[2];
+    if constexpr (IDS) {
+        if (F.triId) F.triId[pix] = id;
+        if (F.bary) { F.bary[pix * 3] = b[0]; F.bary[pix * 3 + 1] = b[1]; F.bary[pix * 3 + 2] = b[2]; }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1789,6 +1861,16 @@ __global__ void __launch_bounds__(NT) k_init_buffers(float *z, float *color, flo
         color[i] = 0.0f;
         normals[i] = 0.0f;
         if (i < pixels) z[i] = Z_INIT;
+    }
+}
+
+// crb_init_buffers on bound id outputs: tri_id -1, bary 0 (either may be NULL)
+__global__ void __launch_bounds__(NT) k_init_ids(int32_t *triId, float *bary, long long pixels)
+{
+    const long long stride = (long long)gridDim.x * NT, n = bary ? pixels * 3 : pixels;
+    for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < n; i += stride) {
+        if (bary) bary[i] = 0.0f;
+        if (triId && i < pixels) triId[i] = -1;
     }
 }
 
@@ -2055,6 +2137,9 @@ struct crb_filler {
     const uint32_t *tex;   // crb_bind_texture: packed texels (caller-owned device memory), NULL = none
     int tex_h, tex_w;
     int tex_levels;        // crb_bind_texture_mips: levels of the bound chain; 0 = a single level (crb_bind_texture)
+    int32_t *tri_id;       // crb_bind_id_buffers: id outputs of crb_render / crb_render_host / crb_init_buffers (NULL = not wanted)
+    float *bary;
+    int id_base;
 };
 
 namespace {
@@ -2167,6 +2252,22 @@ void fill_frame(const crb_filler *f, Frame *F, int set = 0)
     F->texW = f->tex_w;
 }
 
+// The filler's bound id outputs (crb_render, crb_render_host); crb_render_views_ids sets its slabs itself
+void fill_ids(const crb_filler *f, FrameIds *F)
+{
+    F->triId = f->tri_id;
+    F->bary = f->bary;
+    F->idBase = f->id_base;
+}
+
+// tri_id = base + t must fit int32 for every t < T (-1 is reserved: base >= 0 is checked where it is bound)
+int check_id_range(long long base, int64_t T)
+{
+    if (base + T - 1 > (long long)INT32_MAX)
+        return fail(CRB_ERR_INVALID, "id base %lld + T %lld - 1 exceeds INT32_MAX", base, (long long)T);
+    return CRB_OK;
+}
+
 // CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR, CRB_TEX_TRILINEAR, CRB_TEX_REPEAT and CRB_TEX_MIRROR are modes of CRB_TEXTURE, which
 // needs a bound texture; CRB_TEX_TRILINEAR needs a bound mip chain and excludes CRB_TEX_BILINEAR; the two wrap modes exclude
 // each other
@@ -2215,7 +2316,7 @@ EncodeTiledFn encode_tiled_fn()
 }
 
 // [views][rows][W*comps] float32, boxes of box_rows x (TW*comps).  Returns false if the layout cannot be described.
-bool encode_map(CUtensorMap *m, float *base, int comps, const Frame &F, int box_rows)
+bool encode_map(CUtensorMap *m, void *base, int comps, const Frame &F, int box_rows)
 {
     EncodeTiledFn fn = encode_tiled_fn();
     const long long rows = F.row1 - F.row0;
@@ -2228,13 +2329,16 @@ bool encode_map(CUtensorMap *m, float *base, int comps, const Frame &F, int box_
               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// All or nothing: every non-NULL output array gets a map, or the launch uses plain stores.
-unsigned encode_maps(TMaps *M, const Frame &F, int clear_rows)
+// All or nothing: every non-NULL output array gets a map, or the launch uses plain stores.  The id outputs' maps are encoded
+// only where they are bound.
+unsigned encode_maps(TMapsIds *M, const FrameIds &F, int clear_rows)
 {
     unsigned use = 0;
     if (F.z) { if (!encode_map(&M->zt, F.z, 1, F, clear_rows)) return 0u; use |= CRB_BUF_Z; }
     if (F.color) { if (!encode_map(&M->ct, F.color, 3, F, clear_rows)) return 0u; use |= CRB_BUF_COLOR; }
     if (F.normals) { if (!encode_map(&M->nt, F.normals, 3, F, clear_rows)) return 0u; use |= CRB_BUF_NORMALS; }
+    if (F.triId) { if (!encode_map(&M->it, F.triId, 1, F, clear_rows)) return 0u; use |= ID_TRI; }
+    if (F.bary) { if (!encode_map(&M->bt, F.bary, 3, F, clear_rows)) return 0u; use |= ID_BARY; }
     return use;
 }
 
@@ -2326,29 +2430,35 @@ int tex_mode(const Frame &F)
     return filter | wrap | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
 }
 
-// Calls fn(std::integral_constant<int, MODE>()) with the frame's tex_mode as a compile-time constant: the one list of the shading
-// instantiations of k_raster and k_shade_atomic (per-vertex, then 3 filters x 2 interpolations x 3 addressing modes)
+// Calls fn(std::integral_constant<int, MODE>(), std::bool_constant<IDS>()) with the frame's tex_mode and whether it has id outputs
+// as compile-time constants: the one list of the shading instantiations of k_raster and k_shade_atomic (per-vertex, then
+// 3 filters x 2 interpolations x 3 addressing modes; each without and with id outputs)
 template <class Fn>
-void with_tex_mode(const Frame &F, Fn &&fn)
+void with_shade_mode(const FrameIds &F, Fn &&fn)
 {
+    const bool ids = F.triId || F.bary;
+    auto go = [&](auto mode) {
+        if (ids) fn(mode, std::true_type());
+        else fn(mode, std::false_type());
+    };
 #define CRB_TEX_CASES(W)                                                                                               \
-    case TEX_NEAREST | (W): fn(std::integral_constant<int, TEX_NEAREST | (W)>()); break;                               \
-    case TEX_NEAREST | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_NEAREST | TEX_PERSP | (W)>()); break;       \
-    case TEX_BILINEAR | (W): fn(std::integral_constant<int, TEX_BILINEAR | (W)>()); break;                             \
-    case TEX_BILINEAR | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_BILINEAR | TEX_PERSP | (W)>()); break;     \
-    case TEX_TRILINEAR | (W): fn(std::integral_constant<int, TEX_TRILINEAR | (W)>()); break;                           \
-    case TEX_TRILINEAR | TEX_PERSP | (W): fn(std::integral_constant<int, TEX_TRILINEAR | TEX_PERSP | (W)>()); break;
+    case TEX_NEAREST | (W): go(std::integral_constant<int, TEX_NEAREST | (W)>()); break;                               \
+    case TEX_NEAREST | TEX_PERSP | (W): go(std::integral_constant<int, TEX_NEAREST | TEX_PERSP | (W)>()); break;       \
+    case TEX_BILINEAR | (W): go(std::integral_constant<int, TEX_BILINEAR | (W)>()); break;                             \
+    case TEX_BILINEAR | TEX_PERSP | (W): go(std::integral_constant<int, TEX_BILINEAR | TEX_PERSP | (W)>()); break;     \
+    case TEX_TRILINEAR | (W): go(std::integral_constant<int, TEX_TRILINEAR | (W)>()); break;                           \
+    case TEX_TRILINEAR | TEX_PERSP | (W): go(std::integral_constant<int, TEX_TRILINEAR | TEX_PERSP | (W)>()); break;
     switch (tex_mode(F)) {
     CRB_TEX_CASES(0)
     CRB_TEX_CASES(TEX_REPEAT)
     CRB_TEX_CASES(TEX_MIRROR)
-    default: fn(std::integral_constant<int, TEX_NONE>());
+    default: go(std::integral_constant<int, TEX_NONE>());
     }
 #undef CRB_TEX_CASES
 }
 
 // raster + shade (+ fused clear) of the frame run_prep binned
-int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
+int run_raster(crb_filler *f, FrameIds &F, cudaStream_t st, int slot)
 {
     int rc;
     slot &= 7;                                   // busy-tile statistics are kept per position in a batch of launches
@@ -2378,7 +2488,7 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     }
     const int clear_rows = shape == 2 ? RasterSmall::CLEAR_ROWS : shape == 3 ? RasterWide::CLEAR_ROWS : RasterLarge::CLEAR_ROWS;
     const int min_ctas = shape == 2 ? RasterSmall::MIN_CTAS : shape == 3 ? RasterWide::MIN_CTAS : RasterLarge::MIN_CTAS;
-    TMaps M;
+    TMapsIds M;
     memset(&M, 0, sizeof(M));
     const bool clear = (F.flags & CRB_CLEAR_FIRST) != 0;
     if (f->use_tma && clear && !(F.W & 3) && !F.color_u8) M.use = encode_maps(&M, F, clear_rows);
@@ -2406,11 +2516,14 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     long long gR = gL + gH;
     if (M.use) gR = (long long)CE * ((gR + CE - 2) / (CE - 1));     // CE - 1 rasterizing CTAs + one clear CTA per group of CE (see k_raster)
     if (prof) CU(cudaEventRecord(f->prof_ev[2 * f->prof_n], st));
-    with_tex_mode(F, [&](auto mode) {
+    with_shade_mode(F, [&](auto mode, auto ids) {
         constexpr int TEX = decltype(mode)::value;
-        if (shape == 2) k_raster<RasterSmall, TEX><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(F, M);
-        else if (shape == 3) k_raster<RasterWide, TEX><<<(unsigned)gR, RasterWide::RT, 0, st>>>(F, M);
-        else k_raster<RasterLarge, TEX><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(F, M);
+        constexpr bool IDS = decltype(ids)::value;
+        const FrameOf<IDS> &FK = F;          // without id outputs: the Frame part only
+        const TMapsOf<IDS> &MK = M;
+        if (shape == 2) k_raster<RasterSmall, TEX, IDS><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(FK, MK);
+        else if (shape == 3) k_raster<RasterWide, TEX, IDS><<<(unsigned)gR, RasterWide::RT, 0, st>>>(FK, MK);
+        else k_raster<RasterLarge, TEX, IDS><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(FK, MK);
     });
     if ((rc = launch_check(f, "k_raster"))) return rc;
     if (prof) {
@@ -2420,13 +2533,13 @@ int run_raster(crb_filler *f, Frame &F, cudaStream_t st, int slot)
     return CRB_OK;
 }
 
-int run_tiled(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
+int run_tiled(crb_filler *f, FrameIds &F, cudaStream_t st, int slot = 0)
 {
     int rc = run_prep(f, F, st, slot);
     return rc ? rc : run_raster(f, F, st, slot);
 }
 
-int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
+int run_atomic(crb_filler *f, FrameIds &F, cudaStream_t st)
 {
     int rc;
     if (F.nViews != 1 || F.views) return fail(CRB_ERR_INVALID, "CRB_PATH_ATOMIC supports single-view renders only");
@@ -2447,7 +2560,11 @@ int run_atomic(crb_filler *f, Frame &F, cudaStream_t st)
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
     }
     const unsigned gS = (unsigned)((F.slabPixels + NT - 1) / NT);
-    with_tex_mode(F, [&](auto mode) { k_shade_atomic<decltype(mode)::value><<<gS, NT, 0, st>>>(F, f->keybuf); });
+    with_shade_mode(F, [&](auto mode, auto ids) {
+        constexpr bool IDS = decltype(ids)::value;
+        const FrameOf<IDS> &FK = F;
+        k_shade_atomic<decltype(mode)::value, IDS><<<gS, NT, 0, st>>>(FK, f->keybuf);
+    });
     return launch_check(f, "k_shade_atomic");
 }
 
@@ -2811,7 +2928,20 @@ int crb_init_buffers(crb_filler *f, void *stream)
     const long long px = (long long)(f->row1 - f->row0) * f->w;
     if (px == 0) return CRB_OK;
     k_init_buffers<<<1184, NT, 0, (cudaStream_t)stream>>>(f->z, f->color, f->normals, px);
-    return launch_check(f, "k_init_buffers");
+    int rc = launch_check(f, "k_init_buffers");
+    if (rc || (!f->tri_id && !f->bary)) return rc;
+    k_init_ids<<<1184, NT, 0, (cudaStream_t)stream>>>(f->tri_id, f->bary, px);
+    return launch_check(f, "k_init_ids");
+}
+
+int crb_bind_id_buffers(crb_filler *f, int32_t *tri_id, float *bary, int32_t base)
+{
+    if (check_filler(f)) return CRB_ERR_INVALID;
+    if (base < 0) return fail(CRB_ERR_INVALID, "id base %d < 0 (-1 is reserved for pixels nothing covers)", (int)base);
+    if ((reinterpret_cast<uintptr_t>(tri_id) | reinterpret_cast<uintptr_t>(bary)) & 15u)
+        return fail(CRB_ERR_INVALID, "id buffers must be 16-byte aligned");
+    f->tri_id = tri_id; f->bary = bary; f->id_base = base;
+    return CRB_OK;
 }
 
 int crb_render(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, unsigned flags, void *stream)
@@ -2820,11 +2950,13 @@ int crb_render(crb_filler *f, const float *v, const float *c, const float *n, in
     if (!f->z || !f->color || !f->normals) return fail(CRB_ERR_STATE, "buffers not bound");
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
+    if (f->tri_id) { int irc = check_id_range(f->id_base, T); if (irc) return irc; }
     CU(cudaSetDevice(f->device));
     { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
     if ((long long)(f->row1 - f->row0) * f->w == 0) return CRB_OK;
-    Frame F;
+    FrameIds F;
     fill_frame(f, &F);
+    fill_ids(f, &F);
     F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEX_FLAGS);
     F.v = v; F.c = c; F.n = n;
     F.z = f->z; F.color = f->color; F.normals = f->normals;
@@ -3140,6 +3272,14 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
                      int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
                      unsigned flags, const float light[3], void *stream)
 {
+    return crb_render_views_ids(f, v, c, n, T, views, n_views, z_out, color_out, normals_out, color_u8_out, nullptr, nullptr,
+                                flags, light, stream);
+}
+
+int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views,
+                         int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
+                         int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream)
+{
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (n_views < 0) return fail(CRB_ERR_INVALID, "negative size");
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
@@ -3147,8 +3287,10 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
     if (flags & CRB_PATH_ATOMIC) return fail(CRB_ERR_INVALID, "CRB_PATH_ATOMIC supports single-view renders only");
     if ((flags & CRB_GURO) && !light) return fail(CRB_ERR_INVALID, "CRB_GURO needs a light direction");
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
-    if ((reinterpret_cast<uintptr_t>(z_out) | reinterpret_cast<uintptr_t>(color_out) | reinterpret_cast<uintptr_t>(normals_out)) & 15u)
+    if ((reinterpret_cast<uintptr_t>(z_out) | reinterpret_cast<uintptr_t>(color_out) | reinterpret_cast<uintptr_t>(normals_out) |
+         reinterpret_cast<uintptr_t>(tri_id_out) | reinterpret_cast<uintptr_t>(bary_out)) & 15u)
         return fail(CRB_ERR_INVALID, "output slabs must be 16-byte aligned");
+    if (tri_id_out) { int irc = check_id_range(0, T); if (irc) return irc; }
     if (f->u8x_n && color_u8_out) return fail(CRB_ERR_INVALID, "color_u8_out must be NULL while a row exchange is set (crb_set_u8_exchange)");
     if (f->u8x_n && f->u8x_n * f->u8x_rows != f->row1 - f->row0) return fail(CRB_ERR_STATE, "row exchange bands do not cover the filler's rows");
     CU(cudaSetDevice(f->device));
@@ -3173,8 +3315,11 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
     int i = 0, last_set = 0;
     for (int v0 = 0; v0 < n_views; v0 += f->maxViews, ++i) {
         const int set = pipe ? (int)(f->launch_seq++ & 1u) : 0;
-        Frame F;
+        FrameIds F;
         fill_frame(f, &F, set);
+        F.triId = tri_id_out ? tri_id_out + (size_t)v0 * slab : nullptr;    // views index the base mesh: base 0
+        F.bary = bary_out ? bary_out + (size_t)v0 * slab * 3 : nullptr;
+        F.idBase = 0;
         F.T = T; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
         F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;

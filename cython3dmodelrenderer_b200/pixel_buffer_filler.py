@@ -130,6 +130,10 @@ class AdvancedPixelBufferFiller:
     `texture_wrap="clamp" | "repeat" | "mirror"` -- how those renders address texels of coordinates outside [0, 1]: the border
     texel (the default), the texture repeated (CRB_TEX_REPEAT), or repeated mirrored every other period (CRB_TEX_MIRROR), on
     both axes and with every filter.
+    `triangle_ids=True` / `barycentrics=True` -- the filler also keeps an int32 [rows,w] buffer of the triangle visible at each
+    pixel (`id_base` of the render call + its index in the call's arrays; -1 where nothing was drawn) and a float32 [rows,w,3]
+    buffer of its screen-space barycentrics there (crb_bind_id_buffers, DESIGN 2); read them with get_triangle_id_buffer() /
+    get_barycentric_buffer() or device_id_buffers().  With `out_ptrs` these two buffers are the filler's own.
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -141,7 +145,8 @@ class AdvancedPixelBufferFiller:
     _view_owner = {}      # address of a host mirror handed out by get_*_buffer() -> weak reference to its filler (owner_of_views)
 
     def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None,
-                 texturing="vertex", texture_filter="nearest", perspective_correct=False, texture_wrap="clamp"):
+                 texturing="vertex", texture_filter="nearest", perspective_correct=False, texture_wrap="clamp",
+                 triangle_ids=False, barycentrics=False):
         if texturing not in ("vertex", "pixel"):
             raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
         if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear", "trilinear"):
@@ -150,6 +155,9 @@ class AdvancedPixelBufferFiller:
             raise ValueError(f"perspective_correct must be True or False, got {perspective_correct!r}")
         if not isinstance(texture_wrap, str) or texture_wrap not in ("clamp", "repeat", "mirror"):
             raise ValueError(f"texture_wrap must be 'clamp', 'repeat' or 'mirror', got {texture_wrap!r}")
+        for name, val in (("triangle_ids", triangle_ids), ("barycentrics", barycentrics)):
+            if not isinstance(val, (bool, np.bool_)):
+                raise ValueError(f"{name} must be True or False, got {val!r}")
         self._texturing = texturing
         # render flags of every textured frame (kept in the arguments of a frame, so a redraw of it samples the same way)
         self._tex_flags = (_lib.CRB_TEXTURE | (_lib.CRB_TEX_BILINEAR if texture_filter == "bilinear" else 0)
@@ -187,6 +195,18 @@ class AdvancedPixelBufferFiller:
                 self._normals = wrap_device_pointer(torch, out_ptrs[2], (rows, self.w, 3), self._dev)
             check(self._L.crb_bind_buffers(self._handle, self._z.data_ptr(), self._color.data_ptr(),
                                            self._normals.data_ptr()))
+            # id outputs: always the filler's own memory.  Fresh-filler values (-1, 0) come with the first frame's clear, or --
+            # caller buffers taken as they are -- right here
+            self._tri_id = torch.empty((rows, self.w), dtype=torch.int32, device=self._dev) if triangle_ids else None
+            self._bary = torch.empty((rows, self.w, 3), dtype=torch.float32, device=self._dev) if barycentrics else None
+            if out_ptrs is not None:
+                if self._tri_id is not None:
+                    self._tri_id.fill_(-1)
+                if self._bary is not None:
+                    self._bary.zero_()
+            self._id_base = 0
+            if triangle_ids or barycentrics:
+                check(self._L.crb_bind_id_buffers(self._handle, self._ptr_or_none(self._tri_id), self._ptr_or_none(self._bary), 0))
         self._ws = None
         self._ws_T = -1
         self._ws_views = 1
@@ -223,6 +243,19 @@ class AdvancedPixelBufferFiller:
                 self._handle = None
         except Exception:
             pass
+
+    @staticmethod
+    def _ptr_or_none(t):
+        return None if t is None else t.data_ptr()
+
+    def _check_id_base(self, id_base, T):
+        """The id_base of a render call: an int >= 0 with id_base + T - 1 <= INT32_MAX (-1 is reserved)."""
+        if isinstance(id_base, (bool, np.bool_)) or not isinstance(id_base, (int, np.integer)):
+            raise ValueError(f"id_base must be an int, got {id_base!r}")
+        id_base = int(id_base)
+        if id_base < 0 or id_base + int(T) - 1 > 2 ** 31 - 1:
+            raise ValueError(f"id_base must be >= 0 with id_base + T - 1 <= 2**31 - 1, got id_base={id_base}, T={int(T)}")
+        return id_base
 
     def _stream(self):
         return ctypes.c_void_p(self._torch.cuda.current_stream(self._dev).cuda_stream)
@@ -346,21 +379,22 @@ class AdvancedPixelBufferFiller:
         """pyx:80-81"""
         return self.h, self.w
 
-    def render_model(self, model, prefetch=True):
+    def render_model(self, model, prefetch=True, id_base=0):
         """pyx:92-104.  Reads model._vertices_by_triangles / _colors_by_triangles / _normals_by_triangles
         ([T,3,3] float32), never mutates them, composites into the persistent buffers.  (`prefetch=False`, not in the
         reference: do not start downloading the buffers the previous frame's caller fetched -- renderer.Renderer lights the
-        colour buffer on the device first.)"""
+        colour buffer on the device first.  `id_base`, not in the reference: added to the triangle index written to the
+        triangle-id buffer, so that the models composited into one frame get ranges of their own.)"""
         if self._texturing == "pixel":
-            return self._render_model_textured(model, prefetch)
+            return self._render_model_textured(model, prefetch, id_base)
         v = _check_tri_array(getattr(model, "_vertices_by_triangles"), "vertices")
         c = _check_tri_array(getattr(model, "_colors_by_triangles"), "colors")
         n = _check_tri_array(getattr(model, "_normals_by_triangles"), "normals")
         if not (v.shape[0] == c.shape[0] == n.shape[0]):
             raise IndexError("Out of bounds on buffer access (axis 0)")   # what the bounds-checked memoryviews raise
-        self.render_arrays(v, c, n, prefetch=prefetch)
+        self.render_arrays(v, c, n, prefetch=prefetch, id_base=id_base)
 
-    def _render_model_textured(self, model, prefetch):
+    def _render_model_textured(self, model, prefetch, id_base=0):
         """render_model with texturing="pixel": vertices and normals by triangle as upstream, and -- in place of the colours --
         the texture coordinates by triangle, gathered on the device, with the model's texture bound.  Both are made once per
         model (cached on the identity of `_texture_coords`, `_triangles_texture_coords` and `_texture`, which Model never
@@ -394,7 +428,7 @@ class AdvancedPixelBufferFiller:
             self._uv = u = (vt, tri, uv)
         if not (v.shape[0] == u[2].shape[0] == n.shape[0]):
             raise IndexError("Out of bounds on buffer access (axis 0)")
-        self.render_arrays(v, u[2], n, prefetch=prefetch, texture=tex)
+        self.render_arrays(v, u[2], n, prefetch=prefetch, texture=tex, id_base=id_base)
 
     def _bind_texture(self, texture):
         """Packs (crb_pack_texture) and binds (crb_bind_texture) `texture` -- with texture_filter="trilinear" its mip chain
@@ -454,6 +488,35 @@ class AdvancedPixelBufferFiller:
         """pyx:252-253"""
         return self._get("z", _lib.CRB_BUF_Z)
 
+    # ---------------------------------------------------------------------------------------- id outputs
+    def _id_tensor(self, name):
+        t = {"triangle_ids": self._tri_id, "barycentrics": self._bary}[name]
+        if t is None:
+            raise ValueError(f"this filler was not built with {name}=True")
+        return t
+
+    def get_triangle_id_buffer(self):
+        """int32 [rows,w]: id_base + index of the triangle visible at each pixel, -1 where nothing was drawn.  A synchronised
+        copy, not a live view: nothing upstream writes through it."""
+        t = self._id_tensor("triangle_ids")
+        self.device_id_buffers()
+        return t.cpu().numpy()
+
+    def get_barycentric_buffer(self):
+        """float32 [rows,w,3]: the screen-space barycentrics (mu:5-34) of that triangle at each pixel, 0 where nothing was
+        drawn.  A synchronised copy, not a live view."""
+        t = self._id_tensor("barycentrics")
+        self.device_id_buffers()
+        return t.cpu().numpy()
+
+    def device_id_buffers(self):
+        """(triangle ids, barycentrics) torch CUDA tensors -- None for the one this filler was not built with."""
+        if self._tri_id is None and self._bary is None:
+            raise ValueError("this filler was built with neither triangle_ids=True nor barycentrics=True")
+        self._validate()
+        self._materialize_clear()
+        return self._tri_id, self._bary
+
     # ---------------------------------------------------------------------------------------- extensions
     def clear(self):
         """Fresh-filler state (pyx:65-67).  The reference has no reset (a new filler per frame is its idiom,
@@ -465,12 +528,12 @@ class AdvancedPixelBufferFiller:
             self._stale[name] = True
         self._exposed.clear()   # arrays handed out earlier are detached until fetched again
 
-    def render_arrays(self, v, c, n, path="tiled", check_status=True, prefetch=True, texture=None):
+    def render_arrays(self, v, c, n, path="tiled", check_status=True, prefetch=True, texture=None, id_base=0):
         """Render [T,3,3] float32 arrays.  numpy inputs are staged through pinned memory and copied H2D;
         torch CUDA tensors are used in place (device-resident inputs).  `texture` (uint8 [h,w,3], BGR; NumPy or torch):
         per-pixel texturing -- `c` then holds texture coordinates by triangle, [T,3,3] (third component ignored) or
         [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE), sampled as the constructor's `texture_filter`,
-        `perspective_correct` and `texture_wrap` say."""
+        `perspective_correct` and `texture_wrap` say.  `id_base`: added to the triangle index in the triangle-id buffer."""
         torch = self._torch
         flags = _lib.CRB_PATH_ATOMIC if path == "atomic" else 0
         if texture is not None:
@@ -494,6 +557,7 @@ class AdvancedPixelBufferFiller:
             # that vertex simply gets IEEE inf / NaN coordinates like on the device-resident path -- stated divergence, DESIGN 2)
             v, c, n = (np.asarray(a) for a in (v, c, n))
             T = v.shape[0]
+        id_base = self._check_id_base(id_base, T)
         self._validate()                 # an earlier frame this one composites onto must have been drawn
         if texture is not None:
             self._bind_texture(texture)
@@ -521,7 +585,7 @@ class AdvancedPixelBufferFiller:
             s[1, :T] = c
             s[2, :T] = n
             v = c = n = None
-        args = (on_device, v, c, n, T, flags)
+        args = (on_device, v, c, n, T, flags, id_base)
         self._queue_render(*args)
         self._prefetched.clear()
         want = self._fetched if self._fetched is not None else type(self)._fetched_by_previous
@@ -549,8 +613,12 @@ class AdvancedPixelBufferFiller:
             if name in self._exposed:
                 self._get(name, bit)
 
-    def _queue_render(self, on_device, v, c, n, T, flags):
+    def _queue_render(self, on_device, v, c, n, T, flags, id_base=0):
         """Queues one frame (upload of the staged host arrays if any, kernels, status words) on the current stream."""
+        if (self._tri_id is not None or self._bary is not None) and id_base != self._id_base:
+            check(self._L.crb_bind_id_buffers(self._handle, self._ptr_or_none(self._tri_id), self._ptr_or_none(self._bary),
+                                              id_base))
+            self._id_base = id_base
         if on_device:
             check(self._L.crb_render(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, flags, self._stream()))
         elif flags & (_lib.CRB_HOST_PAGEABLE | _lib.CRB_SYNC_UPLOAD):
@@ -598,7 +666,7 @@ class AdvancedPixelBufferFiller:
 
     def render_views(self, v, c, n, views, z_out=None, color_out=None, normals_out=None, color_u8_out=None,
                      want=("z", "color", "normals"), guro_light=None, chunk=32, check_status=True, defer_join=False,
-                     u8_exchange=None, texture=None):
+                     u8_exchange=None, texture=None, triangle_id_out=None, barycentrics_out=None):
         """Batched multi-view render (config C5): every view gets fresh-filler buffers in its own slab.
 
         v, c, n: torch CUDA float32 [T,3,3] (device-resident base mesh);  views: [V,16] float32 (numpy or CUDA tensor,
@@ -612,6 +680,9 @@ class AdvancedPixelBufferFiller:
         local array -- the view-sharded render and its delivery in one kernel (crb_set_u8_exchange).
         `texture` (uint8 [h,w,3], BGR): per-pixel texturing -- `c` holds texture coordinates by triangle, [T,3,3] or
         [T,3,2], host or CUDA (see render_arrays).
+        `"triangle_id"` / `"barycentrics"` in `want` (or a tensor passed as `triangle_id_out` / `barycentrics_out`) adds the id
+        outputs of every view: int32 [V,rows,w], the index of the visible triangle in the base mesh (-1: none), and float32
+        [V,rows,w,3], its screen-space barycentrics (crb_render_views_ids).
         Returns a dict of the produced tensors."""
         torch = self._torch
         if texture is not None:
@@ -640,6 +711,8 @@ class AdvancedPixelBufferFiller:
         z_out = slab("z", z_out, (V, rows, self.w), torch.float32)
         color_out = slab("color", color_out, (V, rows, self.w, 3), torch.float32)
         normals_out = slab("normals", normals_out, (V, rows, self.w, 3), torch.float32)
+        triangle_id_out = slab("triangle_id", triangle_id_out, (V, rows, self.w), torch.int32)
+        barycentrics_out = slab("barycentrics", barycentrics_out, (V, rows, self.w, 3), torch.float32)
         if color_u8_out is True:
             color_u8_out = torch.empty((V, rows, self.w, 3), dtype=torch.uint8, device=self._dev)
         if color_u8_out is not None:
@@ -669,17 +742,22 @@ class AdvancedPixelBufferFiller:
             check(self._L.crb_set_u8_exchange(self._handle, len(bases), int(hb), arr))
         try:
             return self._render_views_loop(v, c, n, T, views, V, z_out, color_out, normals_out, color_u8_out, flags, light,
-                                           check_status, out, ptr)
+                                           check_status, out, ptr, triangle_id_out, barycentrics_out)
         finally:
             if u8_exchange is not None:
                 check(self._L.crb_set_u8_exchange(self._handle, 0, 0, None))
 
     def _render_views_loop(self, v, c, n, T, views, V, z_out, color_out, normals_out, color_u8_out, flags, light, check_status,
-                           out, ptr):
+                           out, ptr, tri_id_out=None, bary_out=None):
         while True:
-            check(self._L.crb_render_views(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, views.data_ptr(), V,
-                                           ptr(z_out), ptr(color_out), ptr(normals_out), ptr(color_u8_out), flags, light,
-                                           self._stream()))
+            if tri_id_out is None and bary_out is None:
+                check(self._L.crb_render_views(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, views.data_ptr(), V,
+                                               ptr(z_out), ptr(color_out), ptr(normals_out), ptr(color_u8_out), flags, light,
+                                               self._stream()))
+            else:
+                check(self._L.crb_render_views_ids(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, views.data_ptr(), V,
+                                                   ptr(z_out), ptr(color_out), ptr(normals_out), ptr(color_u8_out),
+                                                   ptr(tri_id_out), ptr(bary_out), flags, light, self._stream()))
             if not check_status:
                 break
             need, cap = ctypes.c_int64(), ctypes.c_int64()

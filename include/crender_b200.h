@@ -186,8 +186,34 @@ int crb_bind_workspace(crb_filler *f, void *workspace, size_t bytes, int64_t max
 int crb_alloc_owned(crb_filler *f, int64_t max_triangles, int max_views, int64_t pair_capacity);
 int crb_device_buffers(const crb_filler *f, float **z, float **color, float **normals);
 
-/* z = 1e6, colour = 0, normals = 0 (pyx:65-67), asynchronous on `stream`. */
+/* z = 1e6, colour = 0, normals = 0 (pyx:65-67), asynchronous on `stream`.  Bound id outputs (crb_bind_id_buffers) are reset
+ * too: tri_id = -1, bary = (+0, +0, +0). */
 int crb_init_buffers(crb_filler *f, void *stream);
+
+/* ---- id outputs: which triangle is visible at each pixel, and its barycentrics there (an extension) -------------------------
+ * The rule (DESIGN 2 states it word for word the same):
+ *   - tri_id: int32 [rows, w].  At every pixel where a render call writes z, colour and normals, tri_id = base + t.  t is the
+ *     index, in that call's [T,3,3] arrays, of the winning triangle: the smallest depth wins; among equal depths the highest
+ *     index wins -- the reference's last writer (`!(new_z > z_buffer)`, an equal depth overwrites).  tri_id is written exactly
+ *     where, and exactly when, the call writes the other buffers; pixels the call does not write keep their value.  In a fresh
+ *     frame (CRB_CLEAR_FIRST, or crb_init_buffers) pixels nothing covers get -1.
+ *   - bary: float32 [rows, w, 3], (b1, b2, b3): the three barycentrics of mu:5-34 that this pixel's z, normals and colour slots
+ *     are interpolated with, px and py the integer pixel coordinates as float32, one rounding per operation, no FMA.  Pixels
+ *     nothing covers in a fresh frame get (+0, +0, +0).  These are screen-space barycentrics, also for CRB_TEX_PERSPECTIVE
+ *     renders (whose texture coordinates are interpolated perspective-correctly from them).
+ *   - Neither output depends on the texturing mode, CRB_GURO or the rasterizer shape; turning them on changes no bit of z,
+ *     colour, normals or the uint8 image.
+ *   - Batched views (crb_render_views_ids): t indexes the base mesh and base is 0; each view's slab is fresh, like the others.
+ *   - Bands (crb_set_band): rows [row0, row1) only, like the other buffers; the concatenated bands equal the full frame.
+ *   - base < 0, or base + T - 1 > INT32_MAX: CRB_ERR_INVALID (-1 is reserved).
+ *   - A frame that overflows the pair list (CRB_ERR_OVERFLOW) leaves the id outputs untouched, like the other buffers.
+ *   - crb_render_image_host writes no id outputs, and leaves bound id buffers untouched. */
+
+/* DEVICE pointers laid out like the bound buffers: tri_id [rows,w] int32, bary [rows,w,3] float32, each 16-byte aligned.  Either
+ * may be NULL (not wanted); both NULL unbinds.  crb_render, crb_render_host (on the device: its download_mask does not cover
+ * them), the atomic path and crb_init_buffers write them; crb_render_views does not.  Host only: rebinding to change `base`
+ * between calls queues nothing.  CRB_ERR_INVALID for base < 0 or a misaligned pointer. */
+int crb_bind_id_buffers(crb_filler *f, int32_t *tri_id, float *bary, int32_t base);
 
 /* ---- per-pixel texturing (CRB_TEXTURE) ----------------------------------------------------------------------- */
 
@@ -272,6 +298,13 @@ int crb_sync(crb_filler *f, void *stream);
 int crb_render_views(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views /* NULL: one untransformed view */,
                      int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
                      unsigned flags, const float light[3], void *stream);
+
+/* crb_render_views plus the id outputs of every view (rule above): tri_id_out [n_views,rows,w] int32 and bary_out
+ * [n_views,rows,w,3] float32, DEVICE, 16-byte aligned, each may be NULL (crb_render_views is this call with both NULL).  tri_id
+ * indexes the base mesh (base 0).  The filler's bound id buffers are not used. */
+int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views,
+                         int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
+                         int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream);
 
 /* Row exchange of the uint8 image (SURVEY 8e, config C5 "view-sharded ... with NCCL gather"; no reference counterpart --
  * run.py is one process).  While n_bands > 0, crb_render_views writes run.py:26's flipped uint8 image of its views NOT into
