@@ -145,8 +145,13 @@ struct FrameIds : Frame {
     float *bary;
     int idBase;          // tri_id = idBase + the winner's index in the call's [T,3,3] arrays
 };
-template <bool IDS>
-using FrameOf = typename std::conditional<IDS, FrameIds, Frame>::type;
+// What the shading pass of k_raster / k_shade_atomic writes, fixed at compile time: the float32 buffers and the uint8 image
+// (OUT_PLAIN), those plus the id outputs (OUT_IDS), or only the supersampled uint8 image, each s x s block of samples resolved
+// into one pixel (OUT_SS, CRB_SS2 / CRB_SS4; k_raster only, s read from F.flags).
+enum OutKind { OUT_PLAIN = 0, OUT_IDS = 1, OUT_SS = 2 };
+constexpr unsigned CRB_SS_FLAGS = CRB_SS2 | CRB_SS4;
+template <int OUT>
+using FrameOf = typename std::conditional<OUT == OUT_IDS, FrameIds, Frame>::type;
 
 // ------------------------------------------------------------------------------------------------------------
 // device arithmetic shared by every path.  Operation order restates the reference exactly.
@@ -1152,8 +1157,8 @@ constexpr unsigned ID_TRI = 8u, ID_BARY = 16u;
 struct TMapsIds : TMaps {
     CUtensorMap it, bt;
 };
-template <bool IDS>
-using TMapsOf = typename std::conditional<IDS, TMapsIds, TMaps>::type;
+template <int OUT>
+using TMapsOf = typename std::conditional<OUT == OUT_IDS, TMapsIds, TMaps>::type;
 
 __device__ __forceinline__ void tma_store_box(const CUtensorMap *m, const void *smem, int cx, int cy, int cv)
 {
@@ -1220,6 +1225,10 @@ struct __align__(128) TileSmem {
                                               //   (and the cleared barycentrics of the IDS instantiations)
             unsigned id[CLEAR_ROWS * TW];     //   IDS instantiations: tri_id -1 (last, so z and c keep their offsets)
         } pat;
+        struct {                              // OUT_SS instantiations (shade_resolved), at most s = 2 columns per output pixel:
+            float part[TH * (TW / 2) * 3];    //   each sample row's horizontal sums of s samples, [row][output column][channel]
+            unsigned char img[(TH / 2) * (TW / 2) * 3];   //   the resolved uint8 block in tile order (the stores flip the rows)
+        } ss;
     } u;
     unsigned long long keys[TH * KEY_STRIDE];
     unsigned warp_sums[RT / 32];
@@ -1301,6 +1310,102 @@ __device__ __forceinline__ void write_clear_ids(const FrameIds &F, int view, int
     }
 }
 
+// ---- supersampled images (OUT_SS: CRB_SS2 / CRB_SS4, DESIGN 2) ---------------------------------------------------------------
+// The frame is rasterized and shaded on the s x s sample grid (the filler's h x w); each s x s block of samples resolves into one
+// pixel of the flipped uint8 image [rows/s, W/s, 3].  rows and W are multiples of s, and s divides TH, TW and the 8-row bands of
+// split tiles, so every block lies inside one CTA's rows of one tile.  Image-only, full-frame, fresh frames (no band, no row
+// exchange): crb_render_views checks that.
+__device__ __forceinline__ int ss_factor(const Frame &F) { return (F.flags & CRB_SS4) ? 4 : 2; }
+
+// Address of output pixel (xo, output row oy counted from the bottom like the sample rows) of view `view`
+__device__ __forceinline__ unsigned char *u8_resolved_pixel(const Frame &F, int s, int view, int oy, int xo)
+{
+    const int rowsO = (F.row1 - F.row0) / s, Wo = F.W / s;
+    return F.color_u8 + ((long long)view * (F.slabPixels / (s * s)) + (long long)(rowsO - 1 - oy) * Wo + xo) * 3;
+}
+
+// Whole output rows of a full tile (3 * TW/s bytes) leave as three stores of TW/s bytes where the image rows allow: W % TW == 0
+// makes every row start a multiple of TW/s bytes (3 is odd)
+__device__ __forceinline__ bool resolved_rows_vec(const Frame &F, int s, int tw)
+{
+    return tw == TW && F.W % TW == 0 && !(reinterpret_cast<uintptr_t>(F.color_u8) & (uintptr_t)(TW / s - 1));
+}
+
+// An empty tile's block of the resolved image: background 0 resolves to 0
+template <int NTH>
+__device__ __forceinline__ void write_clear_resolved(const Frame &F, int view, int x0, int yl0, int tw, int th)
+{
+    const int s = ss_factor(F), oyb = yl0 / s, xo = x0 / s, orows = th / s;
+    if (resolved_rows_vec(F, s, tw)) {
+        for (int i = threadIdx.x; i < orows * 3; i += NTH) {
+            unsigned char *o = u8_resolved_pixel(F, s, view, oyb + i / 3, xo) + (i % 3) * (TW / s);
+            if (s == 2) *reinterpret_cast<uint4 *>(o) = make_uint4(0u, 0u, 0u, 0u);
+            else *reinterpret_cast<uint2 *>(o) = make_uint2(0u, 0u);
+        }
+    } else {
+        const int rowB = tw / s * 3;
+        for (int i = threadIdx.x; i < orows * rowB; i += NTH) u8_resolved_pixel(F, s, view, oyb + i / rowB, xo)[i % rowB] = 0;
+    }
+}
+
+// Shading epilogue of a busy tile's rows [rowLo, th) in an OUT_SS instantiation (the keys hold the tile's winners).  The colour of
+// every sample is what the frame would hold there (lit if CRB_GURO, background 0); per channel the s x s block sums as a fixed
+// pairwise tree, first along each sample row -- (a + b), ((a + b) + (c + d)) -- with warp shuffles (lane = sample column), then
+// across the staged row sums the same way; times F(1/s^2) (exact), truncated like .astype('uint8'), rows flipped.
+template <class C, int TEX>
+__device__ __forceinline__ void shade_resolved(const Frame &F, TileSmem<C> &S, const int view, const int x0, const int y0,
+                                               const int yl0, const int tw, const int th, const int rowLo, const unsigned tid)
+{
+    constexpr int RT = C::RT, RS = (TW / 2) * 3;     // RS: floats of one sample row's sums
+    static_assert(sizeof(S.u.ss) <= sizeof(S.u.st), "the resolve's staging must not grow the tile's shared memory");
+    const unsigned lane = tid & 31u;
+    const int s = ss_factor(F);
+    const float bg = background_color(F);
+    const float4 *recv = F.shrec + (long long)view * F.T * SREC;
+    for (int yy = rowLo + (int)(tid >> 5); yy < th; yy += RT / 32) {      // warp-uniform rows: every lane takes part in the shuffles
+        const unsigned long long key = S.keys[yy * KEY_STRIDE + lane];    // (columns >= tw hold no fragment: their keys stay empty)
+        float c[3] = {bg, bg, bg};
+        if (key != KEY_EMPTY) {
+            float fz, fc[3], fn[3];
+            if (shade_fragment<TEX>(F, recv + (size_t)~(unsigned)(key & 0xFFFFFFFFull) * SREC, (float)(x0 + (int)lane),
+                                    (float)(y0 + yy), fz, fc, fn) && !(fz > Z_INIT)) {   // drawn unless new_z > the fresh z (pyx:223)
+                c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2];
+            }
+        }
+        for (int d = 1; d < s; d <<= 1) {                // lane j*s ends with the tree sum of columns [j*s, j*s + s)
+            c[0] = c[0] + __shfl_down_sync(0xFFFFFFFFu, c[0], d);
+            c[1] = c[1] + __shfl_down_sync(0xFFFFFFFFu, c[1], d);
+            c[2] = c[2] + __shfl_down_sync(0xFFFFFFFFu, c[2], d);
+        }
+        if ((lane & (unsigned)(s - 1)) == 0u) {
+            float *p = S.u.ss.part + yy * RS + (int)lane / s * 3;
+            p[0] = c[0]; p[1] = c[1]; p[2] = c[2];
+        }
+    }
+    __syncthreads();
+    const int so3 = TW / s * 3, rowB = tw / s * 3, oy0 = rowLo / s, oy1 = th / s, oyb = yl0 / s, xo = x0 / s;
+    const float scale = s == 4 ? 0.0625f : 0.25f;
+    const bool vec = resolved_rows_vec(F, s, tw);
+    for (int i = tid; i < (oy1 - oy0) * rowB; i += RT) {
+        const int oy = oy0 + i / rowB, e = i - (i / rowB) * rowB;          // e = output column * 3 + channel
+        const float *p = S.u.ss.part + oy * s * RS + e;
+        const float sum = s == 2 ? p[0] + p[RS] : (p[0] + p[RS]) + (p[2 * RS] + p[3 * RS]);
+        const unsigned char u = to_u8(sum * scale);
+        if (vec) S.u.ss.img[oy * so3 + e] = u;
+        else u8_resolved_pixel(F, s, view, oyb + oy, xo)[e] = u;
+    }
+    if (vec) {
+        __syncthreads();
+        for (int i = tid; i < (oy1 - oy0) * 3; i += RT) {
+            const int oy = oy0 + i / 3, q = i % 3;
+            unsigned char *o = u8_resolved_pixel(F, s, view, oyb + oy, xo) + q * (TW / s);
+            const unsigned char *src = S.u.ss.img + oy * so3 + q * (TW / s);
+            if (s == 2) *reinterpret_cast<uint4 *>(o) = *reinterpret_cast<const uint4 *>(src);
+            else *reinterpret_cast<uint2 *>(o) = *reinterpret_cast<const uint2 *>(src);
+        }
+    }
+}
+
 // Conservative bound of the pixels of one row that can pass `bar_k >= 0`, for one barycentric.
 // Reference (mu:34): num = fl(fl(l1*fl(py-a)) - fl(l2*fl(px-b))), inside <=> !(num/l3 < 0).  With the sign-normalised
 // (l1', l2', d' > 0) form, inside => num' >= -REJ_EPS (k_fill).  num' differs from the real-valued
@@ -1334,11 +1439,12 @@ constexpr int PK_XA = 8, PK_XB = 14, PK_YT = 20;   // tile-relative rectangle: f
 
 // Visibility + deferred shading of one busy tile (n triangles staged at list offset off).  IDS: the winner's id and
 // barycentrics are stored beside the other outputs.
-template <class C, int TEX, bool IDS>
-__device__ __forceinline__ void raster_tile(const FrameOf<IDS> &F, TileSmem<C> &S_, const bool clear, const int view,
+template <class C, int TEX, int OUT>
+__device__ __forceinline__ void raster_tile(const FrameOf<OUT> &F, TileSmem<C> &S_, const bool clear, const int view,
                                             const int tx, const int ty, const unsigned n, const unsigned off, const int rowLo, const int rowHi)
 {
     constexpr int RT = C::RT, CH = C::CH, FQ = C::FQ;
+    constexpr bool IDS = OUT == OUT_IDS;
     typedef TileSmem<C> TS;
     // The address of the CTA's shared memory goes through an empty asm: under the 40-register cap the compiler otherwise re-derives
     // the shared-window base (S2R SR_CgaCtaId + LEA) inside the exact and the shading loops instead of keeping it; an opaque
@@ -1560,6 +1666,10 @@ __device__ __forceinline__ void raster_tile(const FrameOf<IDS> &F, TileSmem<C> &
     }
     __syncthreads();
     PH(6);
+    if constexpr (OUT == OUT_SS) {
+        shade_resolved<C, TEX>(F, S, view, x0, y0, yl0, tw, th, rowLo, tid);
+        return;
+    }
 
     // ---- deferred shading of the winners ---------------------------------------------------------------------
     const long long slab = (long long)view * F.slabPixels;
@@ -1620,9 +1730,10 @@ __device__ __forceinline__ void raster_tile(const FrameOf<IDS> &F, TileSmem<C> &
 
 // The fused clear through TMA: one tile = three whole-tile boxes (z, colour, normals) stored from the constant pattern in
 // shared memory; the hardware clips boxes at the image edge.  Called by one lane.
-template <class C, bool IDS>
-__device__ __forceinline__ void tma_clear_tile(const TMapsOf<IDS> &M, const TileSmem<C> &S, unsigned t)
+template <class C, int OUT>
+__device__ __forceinline__ void tma_clear_tile(const TMapsOf<OUT> &M, const TileSmem<C> &S, unsigned t)
 {
+    constexpr bool IDS = OUT == OUT_IDS;
     constexpr int CLEAR_ROWS = C::CLEAR_ROWS;
     const int view = (int)(t >> 22), yl0 = (int)((t >> 11) & 2047u) * TH, x0 = (int)(t & 2047u) * TW;
 #pragma unroll
@@ -1645,10 +1756,11 @@ __device__ __forceinline__ void tma_clear_tile(const TMapsOf<IDS> &M, const Tile
 // every CTA adopting its share of the empty tiles.
 // Resident CTAs per SM follow the shape (RasterSmall 12 at 40 registers, RasterLarge 8 at up to 64, RasterWide 6 at 40); the
 // static_assert in k_raster ties each shape's shared memory to the residency its launch bounds ask for.
-template <class C, int TEX, bool IDS>
-__global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<IDS> F, const __grid_constant__ TMapsOf<IDS> M)
+template <class C, int TEX, int OUT>
+__global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<OUT> F, const __grid_constant__ TMapsOf<OUT> M)
 {
     constexpr int RT = C::RT, CLEAR_ROWS = C::CLEAR_ROWS;
+    constexpr bool IDS = OUT == OUT_IDS;
     static_assert(sizeof(TileSmem<C>) + 1024 <= 233472 / C::MIN_CTAS, "k_raster: shared memory per CTA exceeds the residency its launch bounds assume");
     __shared__ TileSmem<C> S;
     PH_DECL
@@ -1680,7 +1792,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<IDS
                 while (e < ne) {
                     const unsigned en = e + stride;
                     const unsigned tn = en < ne ? F.empty[en] : 0u;
-                    tma_clear_tile<C, IDS>(M, S, t);
+                    tma_clear_tile<C, OUT>(M, S, t);
                     e = en; t = tn;
                 }
                 tma_commit();
@@ -1715,6 +1827,10 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<IDS
         for (unsigned e = bidx; e < ne; e += Gb) {
             const unsigned t = F.empty[e];
             const int view = (int)(t >> 22), ty = (int)((t >> 11) & 2047u), tx = (int)(t & 2047u);
+            if constexpr (OUT == OUT_SS) {
+                write_clear_resolved<RT>(F, view, tx * TW, ty * TH, min(TW, F.W - tx * TW), min(TH, F.row1 - F.row0 - ty * TH));
+                continue;
+            }
             write_clear_tile<RT>(F, 0u, view, tx * TW, ty * TH, min(TW, F.W - tx * TW), min(TH, F.row1 - F.row0 - ty * TH));
             if constexpr (IDS) write_clear_ids<RT>(F, view, tx * TW, ty * TH, min(TW, F.W - tx * TW), min(TH, F.row1 - F.row0 - ty * TH));
         }
@@ -1724,7 +1840,7 @@ __global__ void __launch_bounds__(C::RT, C::MIN_CTAS) k_raster(const FrameOf<IDS
         const uint4 cur = rec;
         if (cta != first) __syncthreads();                  // the previous tile is done with shared memory
         if (cta + stride < nb) rec = lst[cta + stride];     // the next tile's record arrives while this one is rasterized
-        raster_tile<C, TEX, IDS>(F, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
+        raster_tile<C, TEX, OUT>(F, S, clear, (int)(cur.x >> 22), (int)(cur.x & 2047u), (int)((cur.x >> 11) & 2047u), cur.y, cur.z,
                     (int)(cur.w & 255u), (int)(cur.w >> 8));
     }
 }
@@ -1780,9 +1896,11 @@ __global__ void __launch_bounds__(NT) k_raster_atomic(const Frame F, unsigned lo
     }
 }
 
-template <int TEX, bool IDS>
-__global__ void __launch_bounds__(NT) k_shade_atomic(const FrameOf<IDS> F, unsigned long long *keybuf)
+template <int TEX, int OUT>
+__global__ void __launch_bounds__(NT) k_shade_atomic(const FrameOf<OUT> F, unsigned long long *keybuf)
 {
+    constexpr bool IDS = OUT == OUT_IDS;
+    static_assert(OUT != OUT_SS, "supersampled images come from the tiled path only");
     const long long pix = (long long)blockIdx.x * NT + threadIdx.x;
     if (pix >= F.slabPixels) return;
     const unsigned long long key = keybuf[pix];
@@ -1996,6 +2114,24 @@ __global__ void __launch_bounds__(NT) k_color_u8_flipped(const float *color, uns
     for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < n; i += stride) {
         const long long r = i / rowElems, e = i % rowElems;
         out[(rows - 1 - r) * rowElems + e] = to_u8(color[i]);
+    }
+}
+
+// The resolve of CRB_SS2 / CRB_SS4 (DESIGN 2) over a float32 colour buffer [rowsO*s, Wo*s, 3]: one output element per thread, the
+// same pairwise trees as shade_resolved (along each sample row, then across the rows), times F(1/s^2), run.py:26's truncation, flip
+__global__ void __launch_bounds__(NT) k_color_u8_resolved(const float *color, unsigned char *out, int rowsO, int Wo, int s)
+{
+    const long long rowElems = (long long)Wo * 3, n = (long long)rowsO * rowElems, stride = (long long)gridDim.x * NT;
+    const long long inRow = rowElems * s;                       // floats of one sample row
+    const float scale = s == 4 ? 0.0625f : 0.25f;
+    for (long long i = (long long)blockIdx.x * NT + threadIdx.x; i < n; i += stride) {
+        const long long r = i / rowElems, e = i % rowElems, x = e / 3, k = e % 3;
+        const float *p = color + r * s * inRow + x * s * 3 + k;
+        float rs[4];
+        for (int m = 0; m < s; ++m, p += inRow)
+            rs[m] = s == 2 ? p[0] + p[3] : (p[0] + p[3]) + (p[6] + p[9]);
+        const float sum = s == 2 ? rs[0] + rs[1] : (rs[0] + rs[1]) + (rs[2] + rs[3]);
+        out[(rowsO - 1 - r) * rowElems + e] = to_u8(sum * scale);
     }
 }
 
@@ -2430,16 +2566,17 @@ int tex_mode(const Frame &F)
     return filter | wrap | ((F.flags & CRB_TEX_PERSPECTIVE) ? TEX_PERSP : 0);
 }
 
-// Calls fn(std::integral_constant<int, MODE>(), std::bool_constant<IDS>()) with the frame's tex_mode and whether it has id outputs
+// Calls fn(std::integral_constant<int, MODE>(), std::integral_constant<int, OUT>()) with the frame's tex_mode and its OutKind
 // as compile-time constants: the one list of the shading instantiations of k_raster and k_shade_atomic (per-vertex, then
-// 3 filters x 2 interpolations x 3 addressing modes; each without and with id outputs)
+// 3 filters x 2 interpolations x 3 addressing modes; each without and with id outputs, and -- k_raster only -- resolved)
 template <class Fn>
 void with_shade_mode(const FrameIds &F, Fn &&fn)
 {
-    const bool ids = F.triId || F.bary;
+    const bool ids = F.triId || F.bary, ss = (F.flags & CRB_SS_FLAGS) != 0;
     auto go = [&](auto mode) {
-        if (ids) fn(mode, std::true_type());
-        else fn(mode, std::false_type());
+        if (ss) fn(mode, std::integral_constant<int, OUT_SS>());
+        else if (ids) fn(mode, std::integral_constant<int, OUT_IDS>());
+        else fn(mode, std::integral_constant<int, OUT_PLAIN>());
     };
 #define CRB_TEX_CASES(W)                                                                                               \
     case TEX_NEAREST | (W): go(std::integral_constant<int, TEX_NEAREST | (W)>()); break;                               \
@@ -2516,14 +2653,14 @@ int run_raster(crb_filler *f, FrameIds &F, cudaStream_t st, int slot)
     long long gR = gL + gH;
     if (M.use) gR = (long long)CE * ((gR + CE - 2) / (CE - 1));     // CE - 1 rasterizing CTAs + one clear CTA per group of CE (see k_raster)
     if (prof) CU(cudaEventRecord(f->prof_ev[2 * f->prof_n], st));
-    with_shade_mode(F, [&](auto mode, auto ids) {
+    with_shade_mode(F, [&](auto mode, auto out) {
         constexpr int TEX = decltype(mode)::value;
-        constexpr bool IDS = decltype(ids)::value;
-        const FrameOf<IDS> &FK = F;          // without id outputs: the Frame part only
-        const TMapsOf<IDS> &MK = M;
-        if (shape == 2) k_raster<RasterSmall, TEX, IDS><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(FK, MK);
-        else if (shape == 3) k_raster<RasterWide, TEX, IDS><<<(unsigned)gR, RasterWide::RT, 0, st>>>(FK, MK);
-        else k_raster<RasterLarge, TEX, IDS><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(FK, MK);
+        constexpr int OUT = decltype(out)::value;
+        const FrameOf<OUT> &FK = F;          // without id outputs: the Frame part only
+        const TMapsOf<OUT> &MK = M;
+        if (shape == 2) k_raster<RasterSmall, TEX, OUT><<<(unsigned)gR, RasterSmall::RT, 0, st>>>(FK, MK);
+        else if (shape == 3) k_raster<RasterWide, TEX, OUT><<<(unsigned)gR, RasterWide::RT, 0, st>>>(FK, MK);
+        else k_raster<RasterLarge, TEX, OUT><<<(unsigned)gR, RasterLarge::RT, 0, st>>>(FK, MK);
     });
     if ((rc = launch_check(f, "k_raster"))) return rc;
     if (prof) {
@@ -2560,10 +2697,11 @@ int run_atomic(crb_filler *f, FrameIds &F, cudaStream_t st)
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
     }
     const unsigned gS = (unsigned)((F.slabPixels + NT - 1) / NT);
-    with_shade_mode(F, [&](auto mode, auto ids) {
-        constexpr bool IDS = decltype(ids)::value;
-        const FrameOf<IDS> &FK = F;
-        k_shade_atomic<decltype(mode)::value, IDS><<<gS, NT, 0, st>>>(FK, f->keybuf);
+    with_shade_mode(F, [&](auto mode, auto out) {
+        constexpr int OUT = decltype(out)::value;
+        const FrameOf<OUT> &FK = F;
+        // (no resolved frame gets here: crb_render refuses CRB_SS2 / CRB_SS4, crb_render_views the atomic path)
+        if constexpr (OUT != OUT_SS) k_shade_atomic<decltype(mode)::value, OUT><<<gS, NT, 0, st>>>(FK, f->keybuf);
     });
     return launch_check(f, "k_shade_atomic");
 }
@@ -2947,6 +3085,7 @@ int crb_bind_id_buffers(crb_filler *f, int32_t *tri_id, float *bary, int32_t bas
 int crb_render(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, unsigned flags, void *stream)
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
+    if (flags & CRB_SS_FLAGS) return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: supersampled images come from crb_render_views only");
     if (!f->z || !f->color || !f->normals) return fail(CRB_ERR_STATE, "buffers not bound");
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
@@ -3146,6 +3285,7 @@ static int render_host_once(crb_filler *f, const float *v, const float *c, const
                             unsigned download_mask, float *z_out, float *color_out, float *normals_out, void *stream)
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
+    if (flags & CRB_SS_FLAGS) return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: supersampled images come from crb_render_views only");
     { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     CU(cudaSetDevice(f->device));
@@ -3293,6 +3433,15 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
     if (tri_id_out) { int irc = check_id_range(0, T); if (irc) return irc; }
     if (f->u8x_n && color_u8_out) return fail(CRB_ERR_INVALID, "color_u8_out must be NULL while a row exchange is set (crb_set_u8_exchange)");
     if (f->u8x_n && f->u8x_n * f->u8x_rows != f->row1 - f->row0) return fail(CRB_ERR_STATE, "row exchange bands do not cover the filler's rows");
+    const unsigned ss = flags & CRB_SS_FLAGS;
+    const int s = ss == CRB_SS4 ? 4 : ss == CRB_SS2 ? 2 : 1;
+    if (ss) {
+        if (ss == CRB_SS_FLAGS) return fail(CRB_ERR_INVALID, "CRB_SS2 and CRB_SS4 are exclusive");
+        if (!color_u8_out || z_out || color_out || normals_out || tri_id_out || bary_out)
+            return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: image-only frames (color_u8_out and no float32 or id output)");
+        if (f->row0 != 0 || f->row1 != f->h) return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: not for band fillers (crb_set_band)");
+        if ((f->row1 - f->row0) % s || f->w % s) return fail(CRB_ERR_INVALID, "CRB_SS%d: rows %d and width %d must be multiples of %d", s, f->row1 - f->row0, f->w, s);
+    }
     CU(cudaSetDevice(f->device));
     const long long slab = (long long)(f->row1 - f->row0) * f->w;
     if (slab == 0) return CRB_OK;
@@ -3321,13 +3470,13 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
         F.bary = bary_out ? bary_out + (size_t)v0 * slab * 3 : nullptr;
         F.idBase = 0;
         F.T = T; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
-        F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS)) | CRB_CLEAR_FIRST;
+        F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;
         F.views = views ? views + (size_t)v0 * 16 : nullptr;
         F.z = z_out ? z_out + (size_t)v0 * slab : nullptr;
         F.color = color_out ? color_out + (size_t)v0 * slab * 3 : nullptr;
         F.normals = normals_out ? normals_out + (size_t)v0 * slab * 3 : nullptr;
-        F.color_u8 = color_u8_out ? color_u8_out + (size_t)v0 * slab * 3 : nullptr;
+        F.color_u8 = color_u8_out ? color_u8_out + (size_t)v0 * (slab / (s * s)) * 3 : nullptr;   // (resolved: W/s x rows/s per view)
         if (f->u8x_n) {      // row exchange: the uint8 image leaves through the receive buffers of the row bands
             F.u8xN = f->u8x_n; F.u8xRows = f->u8x_rows;
             for (int d = 0; d < f->u8x_n; ++d) F.u8x[d] = f->u8x[d] + (size_t)v0 * f->u8x_rows * f->w * 3;
@@ -3390,9 +3539,10 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
     if (rc) return rc;
     // one untransformed view, no float32 output: the rasterizer writes the flipped uint8 image itself
     rc = crb_render_views(f, f->stage_v, f->stage_c, f->stage_n, T, nullptr, 1, nullptr, nullptr, nullptr, image_dev,
-                          flags & (CRB_GURO | CRB_TEX_FLAGS), light, stream);
+                          flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS), light, stream);
     if (rc) return rc;
-    const size_t bytes = (size_t)(f->row1 - f->row0) * f->w * 3;
+    const int s = (flags & CRB_SS4) ? 4 : (flags & CRB_SS2) ? 2 : 1;
+    const size_t bytes = (size_t)((f->row1 - f->row0) / s) * (f->w / s) * 3;
     if (bytes) CU(cudaMemcpyAsync(image_host, image_dev, bytes, cudaMemcpyDeviceToHost, st));
     if (status_pinned) {
         rc = crb_status_async(f, status_pinned, stream);
@@ -3434,6 +3584,21 @@ int crb_color_u8_flipped(crb_filler *f, uint8_t *out_u8, void *stream)
     if ((long long)(f->row1 - f->row0) * f->w == 0) return CRB_OK;
     k_color_u8_flipped<<<1184, NT, 0, (cudaStream_t)stream>>>(f->color, out_u8, f->row1 - f->row0, f->w);
     return launch_check(f, "k_color_u8_flipped");
+}
+
+int crb_color_u8_resolved(crb_filler *f, int s, uint8_t *out_u8, void *stream)
+{
+    if (check_filler(f) || !out_u8) return fail(CRB_ERR_INVALID, "NULL argument");
+    if (s != 1 && s != 2 && s != 4) return fail(CRB_ERR_INVALID, "supersampling factor %d is not 1, 2 or 4", s);
+    if (s == 1) return crb_color_u8_flipped(f, out_u8, stream);
+    if (f->row0 != 0 || f->row1 != f->h) return fail(CRB_ERR_INVALID, "crb_color_u8_resolved: not for band fillers (crb_set_band)");
+    if (f->h % s || f->w % s) return fail(CRB_ERR_INVALID, "crb_color_u8_resolved: rows %d and width %d must be multiples of %d", f->h, f->w, s);
+    if (!f->color) return fail(CRB_ERR_STATE, "buffers not bound");
+    CU(cudaSetDevice(f->device));
+    { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
+    if ((long long)f->h * f->w == 0) return CRB_OK;
+    k_color_u8_resolved<<<1184, NT, 0, (cudaStream_t)stream>>>(f->color, out_u8, f->h / s, f->w / s, s);
+    return launch_check(f, "k_color_u8_resolved");
 }
 
 int crb_download(crb_filler *f, unsigned mask, float *z_host, float *color_host, float *normals_host, void *stream)

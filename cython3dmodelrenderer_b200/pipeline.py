@@ -15,7 +15,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import check
-from .pixel_buffer_filler import AdvancedPixelBufferFiller, _check_tri_array
+from .pixel_buffer_filler import SS_FLAGS, AdvancedPixelBufferFiller, _check_supersample, _check_tri_array
 
 _BITS = {"z": _lib.CRB_BUF_Z, "color": _lib.CRB_BUF_COLOR, "normals": _lib.CRB_BUF_NORMALS}
 
@@ -142,23 +142,26 @@ class HostImagePipeline:
     fused launch sequence (fresh-filler clear + rasterizer + shading with the light applied + truncation to uint8 + row
     flip, written by the rasterizer itself: no float32 buffer is produced at all), one D2H copy of h*w*3 bytes and of the
     status words.  `depth` frames are in flight.  Inputs: a pinned float32 tensor [3,T,3,3] = (vertices, colours, normals)
-    by triangles, not to be modified before `result`.  (The per-frame host work matters: at 10 k images/s the submitting
-    thread is the bottleneck if a frame costs it more than a few dozen microseconds.)"""
+    by triangles, not to be modified before `result`.  `supersample=2 | 4`: the image is anti-aliased -- its fillers render
+    (s*h, s*w) samples and the rasterizer resolves each s x s block into one pixel of the [h,w,3] image (CRB_SS2 / CRB_SS4).
+    (The per-frame host work matters: at 10 k images/s the submitting thread is the bottleneck if a frame costs it more than
+    a few dozen microseconds.)"""
 
-    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, depth=3, device=None, light=None):
+    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, depth=3, device=None, light=None, supersample=1):
         if depth < 1:
             raise ValueError("depth must be >= 1")
-        self._flags, self._light = 0, None
+        ss = _check_supersample(supersample)
+        self._flags, self._light = SS_FLAGS[ss], None
         if light is not None:
             # GuroIllumination.__init__ (guro_illumination.py:17-18): negate, then normalise, in float32
             l = -np.asarray(light, dtype="float32")
             l = l / np.linalg.norm(l)
             self._light = (ctypes.c_float * 3)(*[float(x) for x in l])
-            self._flags = _lib.CRB_GURO
+            self._flags |= _lib.CRB_GURO
         self.slots = []
         for _ in range(depth):
             s = _Slot()
-            s.filler = AdvancedPixelBufferFiller(h, w, fov=fov, z_near=z_near, z_far=z_far, device=device)
+            s.filler = AdvancedPixelBufferFiller(ss * h, ss * w, fov=fov, z_near=z_near, z_far=z_far, device=device)
             torch = s.filler._torch
             dev = s.filler._dev
             s.stream = torch.cuda.Stream(device=dev)

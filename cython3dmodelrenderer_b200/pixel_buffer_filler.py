@@ -35,6 +35,16 @@ def _check_texture(texture):
     return texture
 
 
+SS_FLAGS = {1: 0, 2: _lib.CRB_SS2, 4: _lib.CRB_SS4}
+
+
+def _check_supersample(s):
+    """A supersampling factor: 1 (one sample per pixel), 2 or 4 (s x s samples resolved into each pixel, CRB_SS2 / CRB_SS4)."""
+    if isinstance(s, (bool, np.bool_)) or not isinstance(s, (int, np.integer)) or int(s) not in SS_FLAGS:
+        raise ValueError(f"supersample must be 1, 2 or 4, got {s!r}")
+    return int(s)
+
+
 def _check_tri_array(a, name):
     """Same acceptance rules as the reference's `float[:, :, :]` memoryviews (pyx:94-96)."""
     if a is None:
@@ -655,18 +665,28 @@ class AdvancedPixelBufferFiller:
         self._stale["color"] = True
         self._prefetched.discard("color")
 
-    def color_u8_flipped(self):
-        """run.py:26 `image[::-1].astype('uint8')` computed on device; returns a torch CUDA uint8 tensor."""
+    def color_u8_flipped(self, supersample=1):
+        """run.py:26 `image[::-1].astype('uint8')` computed on device; returns a torch CUDA uint8 tensor.  `supersample=2 | 4`:
+        the colour buffer holds s x s samples per pixel, resolved like render_views(supersample=s) into [h/s, w/s, 3]
+        (crb_color_u8_resolved) -- e.g. after Renderer's lighting of a filler built at s times the image size."""
+        ss = _check_supersample(supersample)
+        rows = self.row1 - self.row0
+        if ss > 1 and (rows != self.h or rows % ss or self.w % ss):
+            raise ValueError(f"supersample={ss} needs a full-frame filler whose size is a multiple of {ss}, got rows "
+                             f"[{self.row0}, {self.row1}) of {self.h} x {self.w}")
         self._validate()
         self._materialize_clear()
         self._push_exposed()
-        out = self._torch.empty((self.row1 - self.row0, self.w, 3), dtype=self._torch.uint8, device=self._dev)
-        check(self._L.crb_color_u8_flipped(self._handle, out.data_ptr(), self._stream()))
+        out = self._torch.empty((rows // ss, self.w // ss, 3), dtype=self._torch.uint8, device=self._dev)
+        if ss == 1:
+            check(self._L.crb_color_u8_flipped(self._handle, out.data_ptr(), self._stream()))
+        else:
+            check(self._L.crb_color_u8_resolved(self._handle, ss, out.data_ptr(), self._stream()))
         return out
 
     def render_views(self, v, c, n, views, z_out=None, color_out=None, normals_out=None, color_u8_out=None,
-                     want=("z", "color", "normals"), guro_light=None, chunk=32, check_status=True, defer_join=False,
-                     u8_exchange=None, texture=None, triangle_id_out=None, barycentrics_out=None):
+                     want=None, guro_light=None, chunk=32, check_status=True, defer_join=False,
+                     u8_exchange=None, texture=None, triangle_id_out=None, barycentrics_out=None, supersample=1):
         """Batched multi-view render (config C5): every view gets fresh-filler buffers in its own slab.
 
         v, c, n: torch CUDA float32 [T,3,3] (device-resident base mesh);  views: [V,16] float32 (numpy or CUDA tensor,
@@ -683,8 +703,18 @@ class AdvancedPixelBufferFiller:
         `"triangle_id"` / `"barycentrics"` in `want` (or a tensor passed as `triangle_id_out` / `barycentrics_out`) adds the id
         outputs of every view: int32 [V,rows,w], the index of the visible triangle in the base mesh (-1: none), and float32
         [V,rows,w,3], its screen-space barycentrics (crb_render_views_ids).
-        Returns a dict of the produced tensors."""
+        `supersample=2 | 4`: an anti-aliased uint8 image -- the filler's h x w are samples, and each s x s block of them is
+        resolved into one pixel of color_u8 [V, rows/s, w/s, 3] inside the rasterizer (CRB_SS2 / CRB_SS4, DESIGN 2).  The
+        uint8 image is then the only output: `want` names none (its default is then empty) and color_u8_out is True or such a
+        tensor.
+        `want` defaults to ("z", "color", "normals").  Returns a dict of the produced tensors."""
         torch = self._torch
+        ss = _check_supersample(supersample)
+        if want is None:
+            want = ("z", "color", "normals") if ss == 1 else ()
+        if ss > 1:
+            self._check_supersampled_views(ss, want, color_u8_out, u8_exchange,
+                                           (z_out, color_out, normals_out, triangle_id_out, barycentrics_out))
         if texture is not None:
             texture = _check_texture(texture)
             c = self._uv_array(c, True)
@@ -714,10 +744,14 @@ class AdvancedPixelBufferFiller:
         triangle_id_out = slab("triangle_id", triangle_id_out, (V, rows, self.w), torch.int32)
         barycentrics_out = slab("barycentrics", barycentrics_out, (V, rows, self.w, 3), torch.float32)
         if color_u8_out is True:
-            color_u8_out = torch.empty((V, rows, self.w, 3), dtype=torch.uint8, device=self._dev)
+            color_u8_out = torch.empty((V, rows // ss, self.w // ss, 3), dtype=torch.uint8, device=self._dev)
+        elif ss > 1 and not (color_u8_out.is_cuda and color_u8_out.is_contiguous() and color_u8_out.dtype == torch.uint8
+                             and tuple(color_u8_out.shape) == (V, rows // ss, self.w // ss, 3)):
+            raise ValueError(f"supersample={ss}: color_u8_out must be a contiguous CUDA uint8 tensor [{V}, {rows // ss}, "
+                             f"{self.w // ss}, 3]")
         if color_u8_out is not None:
             out["color_u8"] = color_u8_out
-        flags, light = 0, None
+        flags, light = SS_FLAGS[ss], None
         if texture is not None:
             self._bind_texture(texture)
             flags |= self._tex_flags
@@ -746,6 +780,21 @@ class AdvancedPixelBufferFiller:
         finally:
             if u8_exchange is not None:
                 check(self._L.crb_set_u8_exchange(self._handle, 0, 0, None))
+
+    def _check_supersampled_views(self, ss, want, color_u8_out, u8_exchange, outputs):
+        """What crb_render_views refuses with CRB_SS2 / CRB_SS4, raised as ValueError before anything is queued."""
+        if want:
+            raise ValueError(f"supersample={ss} gives the uint8 image only: want must name no output, got {tuple(want)!r}")
+        if any(t is not None for t in outputs):
+            raise ValueError(f"supersample={ss} gives the uint8 image only: no float32 or id output tensor can be passed")
+        if color_u8_out is not True and not isinstance(color_u8_out, self._torch.Tensor):
+            raise ValueError(f"supersample={ss} needs color_u8_out=True or a uint8 tensor [V, rows/{ss}, w/{ss}, 3]")
+        if u8_exchange is not None:
+            raise ValueError(f"supersample={ss} does not combine with u8_exchange")
+        if self.row0 != 0 or self.row1 != self.h:
+            raise ValueError(f"supersample={ss} is not available for band fillers")
+        if self.h % ss or self.w % ss:
+            raise ValueError(f"supersample={ss} needs a filler size that is a multiple of {ss}, got {self.h} x {self.w}")
 
     def _render_views_loop(self, v, c, n, T, views, V, z_out, color_out, normals_out, color_u8_out, flags, light, check_status,
                            out, ptr, tri_id_out=None, bary_out=None):

@@ -115,6 +115,28 @@ extern "C" {
      with its own level's (th_l, tw_l).  Where fr == 0 the second level is still not read.
    - Both bits are independent of CRB_TEX_PERSPECTIVE and combine with every filter; one mode applies to both axes.
    - Both bits together, or either without CRB_TEXTURE: CRB_ERR_INVALID on every render entry point. */
+#define CRB_SS2 65536u             /* crb_render_views / crb_render_image_host: the uint8 image anti-aliased by 2 x 2 supersampling */
+#define CRB_SS4 131072u            /* ... by 4 x 4 supersampling.
+   The rule of both (DESIGN 2 states it word for word the same):
+   - A supersampled image is defined by composition: the frame is rendered at the filler's resolution (rows x w samples), exactly
+     as without the bit, CRB_GURO and texturing included; then each s x s block of samples is resolved into one output pixel.
+     s = 2 (CRB_SS2) or 4 (CRB_SS4).  Neither bit means today's image, bit for bit.
+   - The output is uint8 [rows/s, w/s, 3] per view, rows flipped as run.py:26 flips them.  Let C be the float32 colour the frame
+     would have at sample (row, col), lit if CRB_GURO, with background 0.  Output pixel (r, x), r counted from the bottom like the
+     buffers, reads the samples C[s*r + i, s*x + j], i, j in [0, s).
+   - Per channel the samples are summed as a fixed pairwise tree, first along each sample row, then across the rows: for s = 2
+     (a+b), for s = 4 ((a+b)+(c+d)).  Each operation is one binary32 rounding with no FMA.  The sum is multiplied by F(1/s^2), which
+     scales exactly, then truncated by run.py's .astype('uint8') rule (NaN and values outside int range give 0), then the rows are
+     flipped.  NaN and inf propagate through the sum as IEEE says.
+   - Sample coordinates are the reference's, on the s-times grid: the projection of an (s*h, s*w) filler puts every sample at
+     exactly s times its 1x screen coordinate (xs and ys scale by a power of two, and (float)(h/w) is the same quotient).  The box
+     of output pixel x therefore covers [x, x + (s-1)/s] of the 1x grid; it is not shifted to be centred on x.
+   - Texturing composes unchanged.  Trilinear derivatives are per sample, so the level of detail drops by log2 s.
+   - crb_render_views / crb_render_views_ids accept the bits for image-only frames only: color_u8_out non-NULL and every float32
+     and id output NULL.  crb_render_image_host writes (rows/s) * (w/s) * 3 bytes.
+   - CRB_ERR_INVALID: both bits set; a float32 or id output passed; rows % s or w % s non-zero; a band filler (crb_set_band other
+     than [0, h)); a row exchange set (crb_set_u8_exchange); crb_render / crb_render_host given either bit.
+   - A frame that overflows the pair list leaves the image untouched, like every output. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u
@@ -294,7 +316,8 @@ int crb_sync(crb_filler *f, void *stream);
  * Each view is rendered with fresh-filler semantics into its own slab of z_out [n_views,rows,w], color_out /
  * normals_out [n_views,rows,w,3] (DEVICE).  Any of the three output pointers may be NULL (buffer not wanted).
  * color_u8_out, if not NULL, additionally receives run.py:26's output stage on device: [n_views,rows,w,3] uint8,
- * rows flipped (image[::-1]) and truncated like .astype('uint8'). */
+ * rows flipped (image[::-1]) and truncated like .astype('uint8').  With CRB_SS2 / CRB_SS4 it is the only output, the
+ * supersampled image [n_views,rows/s,w/s,3] (rule above). */
 int crb_render_views(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views /* NULL: one untransformed view */,
                      int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
                      unsigned flags, const float light[3], void *stream);
@@ -342,6 +365,11 @@ int crb_guro(crb_filler *f, const float light[3], void *stream);
 
 /* run.py:26: image[::-1].astype('uint8') of the colour buffer -> out_u8 DEVICE [rows,w,3]. */
 int crb_color_u8_flipped(crb_filler *f, uint8_t *out_u8, void *stream);
+
+/* The resolve of CRB_SS2 / CRB_SS4 (rule above) applied to the bound colour buffer, whose h x w are the samples -> out_u8 DEVICE
+ * [h/s, w/s, 3].  s = 1 is crb_color_u8_flipped.  CRB_ERR_INVALID for s not in {1, 2, 4}, and for s > 1 on a band filler or
+ * with h % s or w % s non-zero. */
+int crb_color_u8_resolved(crb_filler *f, int s, uint8_t *out_u8, void *stream);
 
 /* ---- transfers and status ------------------------------------------------------------------------------------- */
 int crb_download(crb_filler *f, unsigned mask, float *z_host, float *color_host, float *normals_host, void *stream);
