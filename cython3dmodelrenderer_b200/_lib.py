@@ -22,6 +22,7 @@ CRB_CLEAR_FIRST, CRB_PATH_ATOMIC, CRB_GURO, CRB_NO_SYNC, CRB_DL_SPARSE, CRB_DEFE
 CRB_TEXTURE, CRB_TEX_PERSPECTIVE, CRB_TEX_BILINEAR, CRB_TEX_TRILINEAR = 1024, 2048, 4096, 8192
 CRB_TEX_REPEAT, CRB_TEX_MIRROR = 16384, 32768
 CRB_SS2, CRB_SS4 = 65536, 131072
+CRB_CLIP_NEAR = 262144
 CRB_OPT_CHUNK_PIPELINE, CRB_OPT_TMA = 1, 2
 CRB_OPT_BAND_PREPASS, CRB_OPT_RASTER_CTAS, CRB_OPT_SPLIT_HEAVY, CRB_OPT_WIDE_KERNEL, CRB_OPT_RASTER_SHAPE = 4, 5, 6, 7, 8
 CRB_BUF_Z, CRB_BUF_COLOR, CRB_BUF_NORMALS, CRB_BUF_ALL = 1, 2, 4, 7

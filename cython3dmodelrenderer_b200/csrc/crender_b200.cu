@@ -143,7 +143,8 @@ struct Frame {
 struct FrameIds : Frame {
     int32_t *triId;
     float *bary;
-    int idBase;          // tri_id = idBase + the winner's index in the call's [T,3,3] arrays
+    int idBase;          // tri_id = idBase + (the winner's index >> idShift): its index in the call's [T,3,3] arrays
+    int idShift;         // 1 in a CRB_CLIP_NEAR frame (the winner is piece index & 1 of triangle index >> 1), else 0
 };
 // What the shading pass of k_raster / k_shade_atomic writes, fixed at compile time: the float32 buffers and the uint8 image
 // (OUT_PLAIN), those plus the id outputs (OUT_IDS), or only the supersampled uint8 image, each s x s block of samples resolved
@@ -850,6 +851,179 @@ __global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
         __syncthreads();                                // everybody is done with the stage (and with sM / slist / wsum)
         const long long w2 = w + (long long)SETUP_STAGES * gridDim.x;
         if (threadIdx.x == 0 && w2 < nItems) issue(w2, s);
+    }
+}
+
+// ---- CRB_CLIP_NEAR (crender_b200.h, DESIGN 2) ---------------------------------------------------------------------------
+// A clip frame is a frame of F.T = 2T virtual triangles: virtual triangle j is piece j & 1 of real triangle j >> 1.  The setup
+// below writes for each virtual triangle exactly what setup_chunk writes for a triangle (shade record, recE entry, per-tile
+// counts), so every kernel behind it runs unchanged, and the visibility key's index is the rule's tie order 2t + h.
+
+// Corner k of real triangle r (staged in shared memory) in camera space: position (view_point), normal (view_normal), colour.
+__device__ __forceinline__ void clip_corner(const Frame &F, const float *sM, const float *sv, const float *sn, const float *sc, int r,
+                                            int k, float a[9])
+{
+    const int o = r * 9 + k * 3;
+    a[0] = sv[o]; a[1] = sv[o + 1]; a[2] = sv[o + 2];
+    a[3] = sn[o]; a[4] = sn[o + 1]; a[5] = sn[o + 2];
+    a[6] = sc[o]; a[7] = sc[o + 1]; a[8] = sc[o + 2];
+    if (F.views) {
+        view_point(sM, a[0], a[1], a[2]);
+        view_normal(sM, a[3], a[4], a[5]);
+    }
+}
+
+// Item `chunk` of view `view`: NT virtual triangles = NT / 2 real ones, staged by the threads (stage_floats).
+template <bool PERSP>
+__device__ __forceinline__ void setup_chunk_clip(const Frame &F, const float zn, const int view, const long long chunk,
+                                                 const long long chunksPerView, float *sv, float *sn, float *sc, float *sM, unsigned *wsum)
+{
+    const long long first = chunk * NT;                       // first virtual triangle (F.T is even, so cnt is too)
+    const long long cnt = min((long long)NT, F.T - first);
+    stage_floats(F.v, first / 2 * 9, cnt / 2 * 9, sv);
+    stage_floats(F.n, first / 2 * 9, cnt / 2 * 9, sn);
+    stage_floats(F.c, first / 2 * 9, cnt / 2 * 9, sc);
+    if (F.views && threadIdx.x < 16) sM[threadIdx.x] = F.views[view * 16 + threadIdx.x];
+    __syncthreads();
+    const int me = (int)threadIdx.x;
+    const bool valid = me < cnt;
+    const int r = valid ? me >> 1 : 0, h = me & 1;
+
+    // The polygon, corner j in bits 4j..4j+3 as (i | o << 2): corner i itself if o == i, else the crossing point I(i, o)
+    bool in[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const int o = r * 9 + k * 3;
+        float x = sv[o], y = sv[o + 1], z = sv[o + 2];
+        if (F.views) view_point(sM, x, y, z);
+        in[k] = z >= zn;                                      // NaN: outside
+    }
+    unsigned poly = 0;
+    int np = 0;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const int b = a == 2 ? 0 : a + 1;
+        if (in[a]) { poly |= (unsigned)(a | a << 2) << (4 * np); ++np; }
+        if (in[a] != in[b]) {
+            const int i = in[a] ? a : b, o = in[a] ? b : a;
+            poly |= (unsigned)(i | o << 2) << (4 * np); ++np;
+        }
+    }
+    // piece 0 = (p0, p1, p2), piece 1 = (p0, p2, p3), present with 3 or 4 corners (piece 1: 4 only)
+    const bool present = valid && (h == 0 ? np >= 3 : np == 4);
+    float x[3], y[3], z[3], zc[3], nx[3], ny[3], nz[3], q[9];
+#pragma unroll
+    for (int m = 0; m < 3; ++m) {
+        const int j = (m == 0 || h == 0) ? m : m + 1;
+        const int i = (poly >> (4 * j)) & 3u, o = (poly >> (4 * j + 2)) & 3u;
+        float A[9];
+        clip_corner(F, sM, sv, sn, sc, r, i, A);
+        if (o != i) {
+            float B[9];
+            clip_corner(F, sM, sv, sn, sc, r, o, B);
+            const float s = (zn - A[2]) / (B[2] - A[2]);
+#pragma unroll
+            for (int k = 0; k < 9; ++k) A[k] = A[k] + s * (B[k] - A[k]);
+            A[2] = zn;
+        }
+        x[m] = A[0]; y[m] = A[1]; z[m] = A[2]; zc[m] = A[2];
+        nx[m] = A[3]; ny[m] = A[4]; nz[m] = A[5];
+        q[3 * m] = A[6]; q[3 * m + 1] = A[7]; q[3 * m + 2] = A[8];
+        project_vertex(F.proj, x[m], y[m], z[m]);
+    }
+
+    // from here on setup_chunk's code for one triangle: cull (pyx:202-204), rectangle, denominators and flags
+    float fxl = (float)F.W, fxr = 0.0f, fyt = (float)F.H, fyb = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        if (x[k] < fxl) fxl = x[k];
+        if (x[k] > fxr) fxr = x[k];
+        if (y[k] < fyt) fyt = y[k];
+        if (y[k] > fyb) fyb = y[k];
+    }
+    int xl = clipi(ceil_to_int_ref(fxl), 0, F.W), xr = clipi(ceil_to_int_ref(fxr), 0, F.W);
+    int yt = clipi(ceil_to_int_ref(fyt), 0, F.H), yb = clipi(ceil_to_int_ref(fyb), 0, F.H);
+    yt = max(yt, F.row0);
+    yb = min(yb, F.row1);
+    const bool drawn = present && !(((nz[0] + nz[1]) + nz[2]) >= 0.0f) && (xl < xr) && (yt < yb);
+    const unsigned bx = drawn ? ((unsigned)xl | ((unsigned)xr << 16)) : 0u;
+    const unsigned by = drawn ? ((unsigned)yt | ((unsigned)yb << 16)) : 0u;
+    float l03 = 0.f, l13 = 0.f, l23 = 0.f;
+    unsigned fl = 0;
+    if (drawn) {
+        l03 = (x[1] - x[2]) * (y[0] - y[2]) - (y[1] - y[2]) * (x[0] - x[2]);
+        l13 = (x[2] - x[0]) * (y[1] - y[0]) - (y[2] - y[0]) * (x[1] - x[0]);
+        l23 = (x[0] - x[1]) * (y[2] - y[1]) - (y[0] - y[1]) * (x[2] - x[1]);
+        const float a03 = fabsf(l03), a13 = fabsf(l13), a23 = fabsf(l23);
+        if (a03 >= L3_MIN && a03 <= L3_MAX) fl |= (FL_REJ << 0) | (l03 < 0.f ? (FL_NEG << 0) : 0u);
+        if (a13 >= L3_MIN && a13 <= L3_MAX) fl |= (FL_REJ << 1) | (l13 < 0.f ? (FL_NEG << 1) : 0u);
+        if (a23 >= L3_MIN && a23 <= L3_MAX) fl |= (FL_REJ << 2) | (l23 < 0.f ? (FL_NEG << 2) : 0u);
+        float cmax = 0.0f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) cmax = fmaxf(cmax, fmaxf(fabsf(x[k]), fabsf(y[k])));
+        const bool finite_xy = (x[0] - x[0] == 0.f) && (x[1] - x[1] == 0.f) && (x[2] - x[2] == 0.f) && (y[0] - y[0] == 0.f) &&
+                               (y[1] - y[1] == 0.f) && (y[2] - y[2] == 0.f);
+        if ((fl & (7u * FL_REJ)) == 7u * FL_REJ && finite_xy && cmax <= SPAN_COORD_MAX) fl |= FL_SPAN;
+        if (fminf(fminf(a03, a13), a23) >= FDIV_LO && fmaxf(fmaxf(a03, a13), a23) <= FDIV_HI) fl |= FL_FDIV;
+    }
+    // the drawn pieces' entries, densely at the head of the item's recE block, as a band-sharded setup_chunk lists them
+    unsigned n_entries;
+    const unsigned dpos = block_compact(drawn, wsum, n_entries);
+    if (drawn) F.recE[(long long)view * F.T + first + dpos] = make_float4(__uint_as_float(bx), __uint_as_float(by), __uint_as_float((unsigned)me), __uint_as_float(fl));
+    if (threadIdx.x == 0) F.alive[(long long)view * chunksPerView + chunk] = (unsigned short)n_entries;
+    if (drawn) {
+        float4 *R = F.shrec + ((long long)view * F.T + first + me) * SREC;
+        R[S_A] = make_float4(x[0], y[0], x[1], y[1]);
+        R[S_B] = make_float4(x[2], y[2], z[0], z[1]);
+        R[S_C] = make_float4(z[2], l03, l13, l23);
+        R[S_N0] = make_float4(nx[0], ny[0], nz[0], nx[1]);
+        R[S_N1] = make_float4(ny[1], nz[1], nx[2], ny[2]);
+        if (PERSP) {   // CRB_TEX_PERSPECTIVE: (u*w, v*w, w), w = 1 / the piece corner's camera z (zn for a crossing point)
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                const float w = 1.0f / zc[k];
+                q[3 * k] = q[3 * k] * w; q[3 * k + 1] = q[3 * k + 1] * w; q[3 * k + 2] = w;
+            }
+        }
+        R[S_X] = make_float4(nz[2], q[0], q[1], q[2]);
+        R[S_C1] = make_float4(q[3], q[4], q[5], q[6]);
+        R[S_C2] = make_float4(q[7], q[8], __uint_as_float(fl), 0.0f);
+    }
+    if (F.flags & CRB_PATH_ATOMIC) return;
+    int tx0 = 0, tx1 = -1, ty0 = 0, ty1 = -1;
+    if (drawn) tile_span(F, bx, by, tx0, tx1, ty0, ty1);
+    unsigned *cnt_view = F.count + (long long)view * F.nTiles;
+    const int nt = drawn ? (tx1 - tx0 + 1) * (ty1 - ty0 + 1) : 0;
+    if (nt <= WIDE_TILES)
+        for (int ty = ty0; ty <= ty1; ++ty)
+            for (int tx = tx0; tx <= tx1; ++tx) atomicAdd(cnt_view + ty * F.tilesX + tx, 1u);
+    for (unsigned wide = __ballot_sync(0xFFFFFFFFu, nt > WIDE_TILES); wide; wide &= wide - 1u) {
+        const int src = __ffs(wide) - 1;
+        const int sx0 = __shfl_sync(0xFFFFFFFFu, tx0, src), sx1 = __shfl_sync(0xFFFFFFFFu, tx1, src);
+        const int sy0 = __shfl_sync(0xFFFFFFFFu, ty0, src), n = __shfl_sync(0xFFFFFFFFu, nt, src);
+        const int wx = sx1 - sx0 + 1;
+        for (int i = (int)(threadIdx.x & 31u); i < n; i += 32) atomicAdd(cnt_view + (sy0 + i / wx) * F.tilesX + sx0 + i % wx, 1u);
+    }
+}
+
+// The clip instantiations of k_setup: a few CTAs per SM walk the (view, item) work items.  zn = F(z_near) is a parameter of its
+// own, so that Frame, every kernel's parameter block, does not grow.
+template <bool PERSP>
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_clip(const Frame F, const float zn)
+{
+    __shared__ __align__(16) float sv[NT / 2 * 9];
+    __shared__ __align__(16) float sn[NT / 2 * 9];
+    __shared__ __align__(16) float sc[NT / 2 * 9];
+    __shared__ float sM[16];
+    __shared__ unsigned wsum[NT / 32];
+    if (blockIdx.x == 0 && threadIdx.x == 0) {  // k_alloc (next launch) accumulates
+        F.total[0] = 0ull; F.total[2] = 0ull; F.total[3] = 0ull; F.total[4] = 0ull; F.total[5] = 0ull;
+    }
+    const long long chunksPerView = (F.T + NT - 1) / NT;
+    const long long nItems = chunksPerView * F.nViews;
+    for (long long w = blockIdx.x; w < nItems; w += gridDim.x) {
+        setup_chunk_clip<PERSP>(F, zn, (int)(w / chunksPerView), w % chunksPerView, chunksPerView, sv, sn, sc, sM, wsum);
+        __syncthreads();                                // everybody is done with the staged arrays (and with sM / wsum)
     }
 }
 
@@ -1698,7 +1872,7 @@ __device__ __forceinline__ void raster_tile(const FrameOf<OUT> &F, TileSmem<C> &
                 const float zold = clear ? Z_INIT : F.z[pix];
                 if (!(fz > zold)) {  // pyx:223: drawn unless new_z > z_buffer (equal depth overwrites)
                     z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
-                    if constexpr (IDS) { id = F.idBase + (int)tri; b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
+                    if constexpr (IDS) { id = F.idBase + (int)(tri >> F.idShift); b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
                     write = true;
                 }
             }
@@ -1918,7 +2092,7 @@ __global__ void __launch_bounds__(NT) k_shade_atomic(const FrameOf<OUT> F, unsig
             const float zold = clear ? Z_INIT : F.z[pix];
             if (!(fz > zold)) {
                 z = fz; c[0] = fc[0]; c[1] = fc[1]; c[2] = fc[2]; nn[0] = fn[0]; nn[1] = fn[1]; nn[2] = fn[2];
-                if constexpr (IDS) { id = F.idBase + (int)tri; b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
+                if constexpr (IDS) { id = F.idBase + (int)(tri >> F.idShift); b[0] = fb[0]; b[1] = fb[1]; b[2] = fb[2]; }
                 write = true;
             }
         }
@@ -2330,11 +2504,18 @@ int check_filler(const crb_filler *f)
 
 // Shared by every render entry point: triangle indices are packed into 32 bits (the ~tri half of the visibility key, the
 // staged triangle's index word), so a larger T would silently alias winners.
-int check_triangles(const crb_filler *f, int64_t T, const float *v, const float *c, const float *n)
+// CRB_CLIP_NEAR: a call of T triangles is a frame of 2T pieces, with z_near finite and > 0.
+int check_triangles(const crb_filler *f, int64_t T, const float *v, const float *c, const float *n, unsigned flags)
 {
     if (T < 0) return fail(CRB_ERR_INVALID, "T < 0");
     if (T > 0 && (!v || !c || !n)) return fail(CRB_ERR_INVALID, "NULL triangle array");
     if (!f->ws) return fail(CRB_ERR_STATE, "workspace not bound");
+    const bool clip = (flags & CRB_CLIP_NEAR) != 0;
+    if (clip && !(std::isfinite(f->z_near) && f->z_near > 0.0f))
+        return fail(CRB_ERR_INVALID, "CRB_CLIP_NEAR needs a finite z_near > 0 (got %g)", (double)f->z_near);
+    if (clip && T > 0x7FFFFFF8ll) return fail(CRB_ERR_INVALID, "CRB_CLIP_NEAR: 2T exceeds 32-bit triangle indices");
+    if (clip && 2 * T > f->maxT)
+        return fail(CRB_ERR_STATE, "CRB_CLIP_NEAR: 2T=%lld exceeds the workspace's max_triangles=%lld", 2 * (long long)T, f->maxT);
     if (T > f->maxT) return fail(CRB_ERR_STATE, "T=%lld exceeds the workspace's max_triangles=%lld", (long long)T, f->maxT);
     if (T > 0xFFFFFFF0ll) return fail(CRB_ERR_INVALID, "T exceeds 32-bit triangle indices");
     return CRB_OK;
@@ -2394,6 +2575,7 @@ void fill_ids(const crb_filler *f, FrameIds *F)
     F->triId = f->tri_id;
     F->bary = f->bary;
     F->idBase = f->id_base;
+    F->idShift = 0;
 }
 
 // tri_id = base + t must fit int32 for every t < T (-1 is reserved: base >= 0 is checked where it is bound)
@@ -2490,10 +2672,15 @@ int setup_smem_attr(int device)
     return CRB_OK;
 }
 
-// k_setup with `grid` CTAs; CRB_TEX_PERSPECTIVE frames write the perspective-correct texture coordinates into the records
-void launch_setup(const Frame &F, unsigned grid, cudaStream_t st)
+// k_setup with `grid` CTAs; CRB_TEX_PERSPECTIVE frames write the perspective-correct texture coordinates into the records,
+// CRB_CLIP_NEAR frames (F.T = 2T pieces) clip at zn = F(z_near) first
+void launch_setup(const crb_filler *f, const Frame &F, unsigned grid, cudaStream_t st)
 {
-    if (F.flags & CRB_TEX_PERSPECTIVE) k_setup<true><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
+    const bool persp = (F.flags & CRB_TEX_PERSPECTIVE) != 0;
+    if (F.flags & CRB_CLIP_NEAR) {
+        if (persp) k_setup_clip<true><<<grid, NT, 0, st>>>(F, f->z_near);
+        else k_setup_clip<false><<<grid, NT, 0, st>>>(F, f->z_near);
+    } else if (persp) k_setup<true><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
     else k_setup<false><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
 }
 
@@ -2514,13 +2701,14 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     }
     F.wideCap = wide_kernel && !(F.flags & CRB_PATH_ATOMIC) ? (unsigned)(f->wideCap > 0xFFFFFFF0ll ? 0xFFFFFFF0ll : f->wideCap) : 0u;
     unsigned gT = (unsigned)((F.T + NT - 1) / NT);
-    // band-sharded single view: list the chunks that can reach the band first, then walk only those (persistent grids)
+    // band-sharded single view: list the chunks that can reach the band first, then walk only those (persistent grids).  Not for
+    // clip frames: the pre-pass projects unclipped corners (their setup still clamps every piece to the band's rows).
     const bool banded = F.row0 > 0 || F.row1 < F.H;
     F.chunks = nullptr;
     // (it reads the vertex array once more than k_setup alone would: it pays when many chunks miss the band -- measured on the
     // 10 M-triangle sphere with the persistent k_setup that walks the listed chunks through its bulk-copy ring: half-frame bands
     // 1.14 -> 1.06 ms; round 1, with one-chunk CTAs: half 1.16 -> 1.22 ms, quarter 0.84 -> 0.82, eighth 0.59 -> 0.51)
-    if (banded && f->band_prepass && 8ll * (F.row1 - F.row0) <= (long long)PREPASS_EIGHTHS * F.H && F.nViews == 1 && !F.views && F.T >= 8 * NT && !(F.flags & CRB_PATH_ATOMIC) &&
+    if (banded && f->band_prepass && 8ll * (F.row1 - F.row0) <= (long long)PREPASS_EIGHTHS * F.H && F.nViews == 1 && !F.views && F.T >= 8 * NT && !(F.flags & (CRB_PATH_ATOMIC | CRB_CLIP_NEAR)) &&
         !(reinterpret_cast<uintptr_t>(F.v) & 15u)) {
         const size_t so = (size_t)(reinterpret_cast<const char *>(F.alive) - reinterpret_cast<const char *>(f->alive));   // workspace set in use
         F.chunks = reinterpret_cast<unsigned *>(reinterpret_cast<char *>(f->chunks) + so);
@@ -2534,7 +2722,7 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
         const long long items = F.chunks ? (long long)gT : (long long)gT * F.nViews;
-        launch_setup(F, (unsigned)min(items, (long long)f->sm_count * SETUP_MIN_CTAS), st);
+        launch_setup(f, F, (unsigned)min(items, (long long)f->sm_count * SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
     } else {
         CU(cudaMemsetAsync(F.total, 0, 8, st));
@@ -2691,7 +2879,7 @@ int run_atomic(crb_filler *f, FrameIds &F, cudaStream_t st)
     }
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
-        launch_setup(F, (unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * SETUP_MIN_CTAS), st);
+        launch_setup(f, F, (unsigned)min((F.T + NT - 1) / NT, (long long)f->sm_count * SETUP_MIN_CTAS), st);
         if ((rc = launch_check(f, "k_setup"))) return rc;
         k_raster_atomic<<<(unsigned)((F.T * 32 + NT - 1) / NT), NT, 0, st>>>(F, f->keybuf);
         if ((rc = launch_check(f, "k_raster_atomic"))) return rc;
@@ -3087,8 +3275,9 @@ int crb_render(crb_filler *f, const float *v, const float *c, const float *n, in
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (flags & CRB_SS_FLAGS) return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: supersampled images come from crb_render_views only");
     if (!f->z || !f->color || !f->normals) return fail(CRB_ERR_STATE, "buffers not bound");
-    { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int trc = check_triangles(f, T, v, c, n, flags); if (trc) return trc; }
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
+    if ((flags & CRB_CLIP_NEAR) && f->bary) return fail(CRB_ERR_INVALID, "CRB_CLIP_NEAR: no barycentric output (a piece's are not the parent's)");
     if (f->tri_id) { int irc = check_id_range(f->id_base, T); if (irc) return irc; }
     CU(cudaSetDevice(f->device));
     { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
@@ -3096,7 +3285,9 @@ int crb_render(crb_filler *f, const float *v, const float *c, const float *n, in
     FrameIds F;
     fill_frame(f, &F);
     fill_ids(f, &F);
-    F.T = T; F.nViews = 1; F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEX_FLAGS);
+    F.flags = flags & (CRB_CLEAR_FIRST | CRB_PATH_ATOMIC | CRB_TEX_FLAGS | CRB_CLIP_NEAR);
+    F.idShift = (flags & CRB_CLIP_NEAR) ? 1 : 0;
+    F.T = T << F.idShift; F.nViews = 1;
     F.v = v; F.c = c; F.n = n;
     F.z = f->z; F.color = f->color; F.normals = f->normals;
     return (flags & CRB_PATH_ATOMIC) ? run_atomic(f, F, (cudaStream_t)stream) : run_tiled(f, F, (cudaStream_t)stream);
@@ -3286,8 +3477,9 @@ static int render_host_once(crb_filler *f, const float *v, const float *c, const
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (flags & CRB_SS_FLAGS) return fail(CRB_ERR_INVALID, "CRB_SS2 / CRB_SS4: supersampled images come from crb_render_views only");
-    { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int trc = check_triangles(f, T, v, c, n, flags); if (trc) return trc; }
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
+    if ((flags & CRB_CLIP_NEAR) && f->bary) return fail(CRB_ERR_INVALID, "CRB_CLIP_NEAR: no barycentric output (a piece's are not the parent's)");
     CU(cudaSetDevice(f->device));
     { int jrc = join_pending(f, (cudaStream_t)stream); if (jrc) return jrc; }
     cudaStream_t st = (cudaStream_t)stream;
@@ -3422,7 +3614,7 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (n_views < 0) return fail(CRB_ERR_INVALID, "negative size");
-    { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int trc = check_triangles(f, T, v, c, n, flags); if (trc) return trc; }
     if (n_views > 0 && !views && n_views != 1) return fail(CRB_ERR_INVALID, "views is NULL (allowed for one untransformed view only)");
     if (flags & CRB_PATH_ATOMIC) return fail(CRB_ERR_INVALID, "CRB_PATH_ATOMIC supports single-view renders only");
     if ((flags & CRB_GURO) && !light) return fail(CRB_ERR_INVALID, "CRB_GURO needs a light direction");
@@ -3430,6 +3622,7 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
     if ((reinterpret_cast<uintptr_t>(z_out) | reinterpret_cast<uintptr_t>(color_out) | reinterpret_cast<uintptr_t>(normals_out) |
          reinterpret_cast<uintptr_t>(tri_id_out) | reinterpret_cast<uintptr_t>(bary_out)) & 15u)
         return fail(CRB_ERR_INVALID, "output slabs must be 16-byte aligned");
+    if ((flags & CRB_CLIP_NEAR) && bary_out) return fail(CRB_ERR_INVALID, "CRB_CLIP_NEAR: no barycentric output (a piece's are not the parent's)");
     if (tri_id_out) { int irc = check_id_range(0, T); if (irc) return irc; }
     if (f->u8x_n && color_u8_out) return fail(CRB_ERR_INVALID, "color_u8_out must be NULL while a row exchange is set (crb_set_u8_exchange)");
     if (f->u8x_n && f->u8x_n * f->u8x_rows != f->row1 - f->row0) return fail(CRB_ERR_STATE, "row exchange bands do not cover the filler's rows");
@@ -3469,8 +3662,9 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
         F.triId = tri_id_out ? tri_id_out + (size_t)v0 * slab : nullptr;    // views index the base mesh: base 0
         F.bary = bary_out ? bary_out + (size_t)v0 * slab * 3 : nullptr;
         F.idBase = 0;
-        F.T = T; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
-        F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS)) | CRB_CLEAR_FIRST;
+        F.idShift = (flags & CRB_CLIP_NEAR) ? 1 : 0;
+        F.T = T << F.idShift; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
+        F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS | CRB_CLIP_NEAR)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;
         F.views = views ? views + (size_t)v0 * 16 : nullptr;
         F.z = z_out ? z_out + (size_t)v0 * slab : nullptr;
@@ -3529,7 +3723,7 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
                           const float light[3], uint8_t *image_dev, uint8_t *image_host, uint64_t status_pinned[4], void *stream)
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
-    { int trc = check_triangles(f, T, v, c, n); if (trc) return trc; }
+    { int trc = check_triangles(f, T, v, c, n, flags); if (trc) return trc; }
     if (!image_dev || !image_host) return fail(CRB_ERR_INVALID, "NULL image buffer");
     { int xrc = check_texture(f, flags); if (xrc) return xrc; }
     CU(cudaSetDevice(f->device));
@@ -3539,7 +3733,7 @@ int crb_render_image_host(crb_filler *f, const float *v, const float *c, const f
     if (rc) return rc;
     // one untransformed view, no float32 output: the rasterizer writes the flipped uint8 image itself
     rc = crb_render_views(f, f->stage_v, f->stage_c, f->stage_n, T, nullptr, 1, nullptr, nullptr, nullptr, image_dev,
-                          flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS), light, stream);
+                          flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS | CRB_CLIP_NEAR), light, stream);
     if (rc) return rc;
     const int s = (flags & CRB_SS4) ? 4 : (flags & CRB_SS2) ? 2 : 1;
     const size_t bytes = (size_t)((f->row1 - f->row0) / s) * (f->w / s) * 3;

@@ -26,11 +26,12 @@ class _Slot:
 
 class HostFramePipeline:
     def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, depth=2, device=None, want=("z", "color", "normals"),
-                 sparse=True):
+                 sparse=True, near_clip=False):
         """sparse=True: CRB_DL_SPARSE read-back -- each slot's pinned host arrays persist between its frames, so only the
         tiles that are busy in the new frame or were busy in the frame the arrays still show are copied (by a kernel that
         writes into the mapped host memory); the arrays are bit-identical to a full download but READ-ONLY for the caller.
-        sparse=False: plain cudaMemcpy of the whole buffers every frame."""
+        sparse=False: plain cudaMemcpy of the whole buffers every frame.  near_clip=True: triangles are clipped at z_near
+        (CRB_CLIP_NEAR, see AdvancedPixelBufferFiller)."""
         if depth < 1:
             raise ValueError("depth must be >= 1")
         self.sparse = bool(sparse)
@@ -41,7 +42,7 @@ class HostFramePipeline:
         self.slots = []
         for _ in range(depth):
             s = _Slot()
-            s.filler = AdvancedPixelBufferFiller(h, w, fov=fov, z_near=z_near, z_far=z_far, device=device)
+            s.filler = AdvancedPixelBufferFiller(h, w, fov=fov, z_near=z_near, z_far=z_far, device=device, near_clip=near_clip)
             torch = s.filler._torch
             s.stream = torch.cuda.Stream(device=s.filler._dev)
             s.out = {name: s.filler._mirror(name) for name in self.want}      # pinned host tensors
@@ -95,7 +96,8 @@ class HostFramePipeline:
 
     def _launch(self, s):
         pv, pc, pn, T = s.args
-        check(self._L.crb_render_host(s.filler._handle, pv, pc, pn, T, _lib.CRB_CLEAR_FIRST | _lib.CRB_NO_SYNC | (_lib.CRB_DL_SPARSE if self.sparse else 0), self.mask,
+        check(self._L.crb_render_host(s.filler._handle, pv, pc, pn, T, _lib.CRB_CLEAR_FIRST | _lib.CRB_NO_SYNC | (_lib.CRB_DL_SPARSE if self.sparse else 0) |
+                                      s.filler._clip_flags, self.mask,
                                       self._ptr(s, "z"), self._ptr(s, "color"), self._ptr(s, "normals"),
                                       ctypes.c_void_p(s.stream.cuda_stream)))
 
@@ -144,10 +146,12 @@ class HostImagePipeline:
     status words.  `depth` frames are in flight.  Inputs: a pinned float32 tensor [3,T,3,3] = (vertices, colours, normals)
     by triangles, not to be modified before `result`.  `supersample=2 | 4`: the image is anti-aliased -- its fillers render
     (s*h, s*w) samples and the rasterizer resolves each s x s block into one pixel of the [h,w,3] image (CRB_SS2 / CRB_SS4).
+    `near_clip=True`: triangles are clipped at z_near (CRB_CLIP_NEAR, see AdvancedPixelBufferFiller).
     (The per-frame host work matters: at 10 k images/s the submitting thread is the bottleneck if a frame costs it more than
     a few dozen microseconds.)"""
 
-    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, depth=3, device=None, light=None, supersample=1):
+    def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, depth=3, device=None, light=None, supersample=1,
+                 near_clip=False):
         if depth < 1:
             raise ValueError("depth must be >= 1")
         ss = _check_supersample(supersample)
@@ -161,7 +165,8 @@ class HostImagePipeline:
         self.slots = []
         for _ in range(depth):
             s = _Slot()
-            s.filler = AdvancedPixelBufferFiller(ss * h, ss * w, fov=fov, z_near=z_near, z_far=z_far, device=device)
+            s.filler = AdvancedPixelBufferFiller(ss * h, ss * w, fov=fov, z_near=z_near, z_far=z_far, device=device,
+                                                 near_clip=near_clip)
             torch = s.filler._torch
             dev = s.filler._dev
             s.stream = torch.cuda.Stream(device=dev)
@@ -175,6 +180,7 @@ class HostImagePipeline:
             s.done = torch.cuda.Event()
             s.busy = False
             self.slots.append(s)
+        self._flags |= self.slots[0].filler._clip_flags
         self._torch = torch
         self._L = self.slots[0].filler._L
         self._next = 0
@@ -190,7 +196,7 @@ class HostImagePipeline:
         if s.busy:
             self.result(i)
         T = int(block.shape[1])
-        if T > s.filler._ws_T or s.filler._ws is None:
+        if s.filler._frame_triangles(T) > s.filler._ws_T or s.filler._ws is None:
             with torch.cuda.stream(s.stream):
                 s.filler._ensure_workspace(T, views=1)
         s.T = T

@@ -144,6 +144,11 @@ class AdvancedPixelBufferFiller:
     pixel (`id_base` of the render call + its index in the call's arrays; -1 where nothing was drawn) and a float32 [rows,w,3]
     buffer of its screen-space barycentrics there (crb_bind_id_buffers, DESIGN 2); read them with get_triangle_id_buffer() /
     get_barycentric_buffer() or device_id_buffers().  With `out_ptrs` these two buffers are the filler's own.
+    `near_clip=True` -- every render of this filler clips its triangles at `z_near` in camera space before projecting them
+    (CRB_CLIP_NEAR, DESIGN 2), so that geometry behind the camera draws nothing and cameras may stand inside a scene.  Each
+    triangle becomes at most two pieces, so the workspace is sized for twice the triangles; the triangle-id buffer still names
+    the parent triangle, and barycentrics are not available.  Without it (the default) triangles behind the camera project
+    through, as in the reference.
     """
 
     PAGEABLE_MIN_BYTES = 8 << 20      # host arrays of at least this size go up through the library's threaded staging ring
@@ -156,7 +161,7 @@ class AdvancedPixelBufferFiller:
 
     def __init__(self, h, w, fov=90.0, z_near=0.1, z_far=1000.0, n_threads=1, device=None, band=None, out_ptrs=None,
                  texturing="vertex", texture_filter="nearest", perspective_correct=False, texture_wrap="clamp",
-                 triangle_ids=False, barycentrics=False):
+                 triangle_ids=False, barycentrics=False, near_clip=False):
         if texturing not in ("vertex", "pixel"):
             raise ValueError(f"texturing must be 'vertex' or 'pixel', got {texturing!r}")
         if not isinstance(texture_filter, str) or texture_filter not in ("nearest", "bilinear", "trilinear"):
@@ -165,9 +170,15 @@ class AdvancedPixelBufferFiller:
             raise ValueError(f"perspective_correct must be True or False, got {perspective_correct!r}")
         if not isinstance(texture_wrap, str) or texture_wrap not in ("clamp", "repeat", "mirror"):
             raise ValueError(f"texture_wrap must be 'clamp', 'repeat' or 'mirror', got {texture_wrap!r}")
-        for name, val in (("triangle_ids", triangle_ids), ("barycentrics", barycentrics)):
+        for name, val in (("triangle_ids", triangle_ids), ("barycentrics", barycentrics), ("near_clip", near_clip)):
             if not isinstance(val, (bool, np.bool_)):
                 raise ValueError(f"{name} must be True or False, got {val!r}")
+        if near_clip and barycentrics:
+            raise ValueError("near_clip=True does not combine with barycentrics=True (a piece's barycentrics are not its triangle's)")
+        if near_clip and not (np.isfinite(np.float32(z_near)) and np.float32(z_near) > 0):
+            raise ValueError(f"near_clip=True needs a finite z_near > 0, got {z_near!r}")
+        # render flags of every frame: clipping at z_near (CRB_CLIP_NEAR), which makes a call of T triangles a frame of 2T pieces
+        self._clip_flags = _lib.CRB_CLIP_NEAR if near_clip else 0
         self._texturing = texturing
         # render flags of every textured frame (kept in the arguments of a frame, so a redraw of it samples the same way)
         self._tex_flags = (_lib.CRB_TEXTURE | (_lib.CRB_TEX_BILINEAR if texture_filter == "bilinear" else 0)
@@ -270,7 +281,13 @@ class AdvancedPixelBufferFiller:
     def _stream(self):
         return ctypes.c_void_p(self._torch.cuda.current_stream(self._dev).cuda_stream)
 
+    def _frame_triangles(self, T):
+        """Triangles of the frame a call of T triangles makes (the workspace's unit): 2T with near_clip, else T."""
+        return 2 * int(T) if self._clip_flags else int(T)
+
     def _ensure_workspace(self, T, views=1, pair_cap=0):
+        """Workspace for calls of T triangles (2T pieces with near_clip), `views` views per launch, `pair_cap` pairs."""
+        T = self._frame_triangles(T)
         if self._ws is not None and T <= self._ws_T and views <= self._ws_views and pair_cap <= self._pair_cap:
             return
         torch = self._torch
@@ -545,7 +562,7 @@ class AdvancedPixelBufferFiller:
         [T,3,2], and every pixel takes the texel they name (CRB_TEXTURE), sampled as the constructor's `texture_filter`,
         `perspective_correct` and `texture_wrap` say.  `id_base`: added to the triangle index in the triangle-id buffer."""
         torch = self._torch
-        flags = _lib.CRB_PATH_ATOMIC if path == "atomic" else 0
+        flags = (_lib.CRB_PATH_ATOMIC if path == "atomic" else 0) | self._clip_flags
         if texture is not None:
             texture = _check_texture(texture)
             # one residence for all three: on the device if any of them is a CUDA tensor
@@ -712,6 +729,8 @@ class AdvancedPixelBufferFiller:
         ss = _check_supersample(supersample)
         if want is None:
             want = ("z", "color", "normals") if ss == 1 else ()
+        if self._clip_flags and ("barycentrics" in want or barycentrics_out is not None):
+            raise ValueError("near_clip=True gives no barycentrics (a piece's barycentrics are not its triangle's)")
         if ss > 1:
             self._check_supersampled_views(ss, want, color_u8_out, u8_exchange,
                                            (z_out, color_out, normals_out, triangle_id_out, barycentrics_out))
@@ -751,7 +770,7 @@ class AdvancedPixelBufferFiller:
                              f"{self.w // ss}, 3]")
         if color_u8_out is not None:
             out["color_u8"] = color_u8_out
-        flags, light = SS_FLAGS[ss], None
+        flags, light = SS_FLAGS[ss] | self._clip_flags, None
         if texture is not None:
             self._bind_texture(texture)
             flags |= self._tex_flags

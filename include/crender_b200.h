@@ -137,6 +137,31 @@ extern "C" {
    - CRB_ERR_INVALID: both bits set; a float32 or id output passed; rows % s or w % s non-zero; a band filler (crb_set_band other
      than [0, h)); a row exchange set (crb_set_u8_exchange); crb_render / crb_render_host given either bit.
    - A frame that overflows the pair list leaves the image untouched, like every output. */
+#define CRB_CLIP_NEAR 262144u      /* every render entry point: clip triangles at z_near in camera space before projection.
+   The rule (DESIGN 2 states it word for word the same).  F() is float32; every operation is one binary32 rounding with no FMA.
+   - Without the bit every output is bit for bit what it is without clipping: triangles behind the camera project through.
+   - Definition by composition.  Each triangle t of a call is replaced by at most two pieces, (t, 0) and (t, 1), computed in camera
+     space.  The pieces are then rendered exactly as the triangles of a call without the bit, in the order (0,0), (0,1), (1,0),
+     (1,1), ...  So the tie rule's "higher index wins" reads the index 2t + h.  An absent piece draws nothing.  Camera space for
+     crb_render* and crb_render_image_host is the arrays as passed; for batched views it is the output of the view transform:
+     positions through view_point, normals through view_normal.  Colours and texture coordinates are used as passed.
+   - Plane: zn = F(z_near) of the filler.  A corner is inside iff z >= zn.  A NaN z is outside.
+   - Polygon: walk the edges (0,1), (1,2), (2,0).  For edge (a, b): if a is inside, emit a; if exactly one of a and b is
+     inside, emit I(i, o), where i is the inside end and o the outside end.
+   - Crossing point I(i, o): s = (zn - z_i) / (z_o - z_i); x = x_i + s*(x_o - x_i), and y the same way; z = zn exactly; every
+     colour (or texture-coordinate) component and every normal component a = a_i + s*(a_o - a_i).
+   - Pieces: the polygon has 0, 3 or 4 corners p0...  0 corners: no piece.  3 corners: piece 0 = (p0, p1, p2); piece 1 is
+     absent.  4 corners: piece 0 = (p0, p1, p2) and piece 1 = (p0, p2, p3).  With all three corners inside, piece 0 is the
+     triangle itself, bit for bit, so a call whose corners all lie at z >= zn renders exactly as without the bit, in every output.
+   - A piece is an ordinary triangle: it is culled by pyx:202-204 on its own normals, then projected, bounded and rasterized.
+   - CRB_TEX_PERSPECTIVE: w of a piece corner is 1 / its camera z, which is zn for the new corners.
+   - Composes with CRB_GURO, every texture filter, interpolation and wrap mode, CRB_SS2 / CRB_SS4, band fillers, the row
+     exchange, CRB_DEFER_JOIN, the launch pipeline, CRB_DL_SPARSE and CRB_HOST_PAGEABLE.
+   - Id outputs: tri_id = base + t, the parent triangle.  A bary output with the bit returns CRB_ERR_INVALID (a piece's
+     screen-space barycentrics are not barycentrics of the parent).
+   - Workspace: a call of T triangles counts as 2T: max_triangles must be at least 2T, otherwise CRB_ERR_STATE; 2T > 0xFFFFFFF0
+     returns CRB_ERR_INVALID.  So does a filler z_near that is not finite or is <= 0.
+   - A frame that overflows the pair list leaves every output untouched.  There is no far-plane or side clipping. */
 
 /* which-buffer masks for crb_download / crb_render_host */
 #define CRB_BUF_Z 1u
