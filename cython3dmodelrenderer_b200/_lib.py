@@ -54,6 +54,7 @@ SIGNATURES = {
     "crb_render_host": (_i, [_vp, _vp, _vp, _vp, _i64, _u, _u, _vp, _vp, _vp, _vp]),
     "crb_render_views": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i, _vp, _vp, _vp, _vp, _u, _fp, _vp]),
     "crb_render_views_ids": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _u, _fp, _vp]),
+    "crb_render_scene_views": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _u, _fp, _vp]),
     "crb_bind_id_buffers": (_i, [_vp, _vp, _vp, ctypes.c_int32]),
     "crb_set_option": (_i, [_vp, _i, _i]),
     "crb_join": (_i, [_vp, _vp]),

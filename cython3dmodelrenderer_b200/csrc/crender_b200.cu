@@ -192,6 +192,19 @@ __device__ __forceinline__ void view_normal(const float *M, float &x, float &y, 
     z = (M[6] * nx + M[7] * ny) + M[8] * nz;
 }
 
+// Scene frames (crb_render_scene_views): F.views is [nViews, K, 16], and triangle `tri` of view `view` takes the transform of its
+// object, F.views[view, triObj[tri]].  `shown` is false for an object index outside [0, K) and for a hidden object (pad neither
+// +0 nor -0, NaN included); the pointer then names a transform that exists, so that the caller may read it and drop the result.
+__device__ __forceinline__ const float *scene_transform(const Frame &F, const int *triObj, const int K, const int view,
+                                                        const long long tri, bool &shown)
+{
+    const int k = triObj[tri];
+    const bool in = k >= 0 && k < K;
+    const float *M = F.views + ((long long)view * K + (in ? k : 0)) * 16;
+    shown = in && M[15] == 0.0f;
+    return M;
+}
+
 // (int)ceil(x) as the reference binary performs it (pyx:165-166): x86-64 cvttsd2si yields INT_MIN for anything
 // outside int range (the C cast is undefined there); CUDA's cvt would saturate instead, so the range test is explicit.
 __device__ __forceinline__ int ceil_to_int_ref(float x)
@@ -578,11 +591,12 @@ __device__ __forceinline__ unsigned block_compact(const bool flag, unsigned *wsu
 
 // One chunk of NT consecutive triangles of one view.  Every early exit below is taken by the whole CTA or lies behind
 // the last barrier, so the function can be called in a loop (chunk-list mode).  PERSP: the colour slots of the record get
-// the perspective-correct texture coordinates of CRB_TEX_PERSPECTIVE.
-template <bool PERSP>
+// the perspective-correct texture coordinates of CRB_TEX_PERSPECTIVE.  SCENE: each thread reads its triangle's own transform
+// (scene_transform) where the other frames use the view's, sM; a hidden triangle is treated like a culled one.
+template <bool PERSP, bool SCENE>
 __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, const long long chunk, const long long chunksPerView,
                                             float *sv, float *sn, float *sc, float *sM, unsigned char *slist, unsigned *wsum,
-                                            const bool staged)
+                                            const bool staged, const int *triObj, const int K)
 {
     const long long first = chunk * NT;
     const long long cnt = min((long long)NT, F.T - first);
@@ -597,7 +611,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
         stage_floats(F.v, first * 9, cnt * 9, sv);
         if (!banded) stage_floats(F.n, first * 9, cnt * 9, sn);
     }
-    if (F.views && threadIdx.x < 16) sM[threadIdx.x] = F.views[view * 16 + threadIdx.x];
+    if (!SCENE && F.views && threadIdx.x < 16) sM[threadIdx.x] = F.views[view * 16 + threadIdx.x];
     __syncthreads();
     // `me`: the triangle of the chunk this thread sets up (-1: none).  A full-frame filler culls first (pyx:202-204 needs only
     // the z of the three view-space normals) and hands the survivors to the first threads, so that the projection, the
@@ -610,12 +624,14 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
         if (me >= 0) {
             const float *q = sn + me * 9;
             float z0 = q[2], z1 = q[5], z2 = q[8];
-            if (F.views) {   // view_normal, z row only
-                z0 = (sM[6] * q[0] + sM[7] * q[1]) + sM[8] * q[2];
-                z1 = (sM[6] * q[3] + sM[7] * q[4]) + sM[8] * q[5];
-                z2 = (sM[6] * q[6] + sM[7] * q[7]) + sM[8] * q[8];
+            bool shown = true;
+            const float *M = SCENE ? scene_transform(F, triObj, K, view, first + me, shown) : sM;
+            if (SCENE || F.views) {   // view_normal, z row only
+                z0 = (M[6] * q[0] + M[7] * q[1]) + M[8] * q[2];
+                z1 = (M[6] * q[3] + M[7] * q[4]) + M[8] * q[5];
+                z2 = (M[6] * q[6] + M[7] * q[7]) + M[8] * q[8];
             }
-            keep = !(((z0 + z1) + z2) >= 0.0f);
+            keep = shown && !(((z0 + z1) + z2) >= 0.0f);
         }
         const unsigned pos = block_compact(keep, wsum, kept);
         if (kept == 0) {
@@ -630,6 +646,8 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
     const int mi = valid ? me : 0;
     const long long tri = first + mi;
     const long long ridx = (long long)view * F.T + tri;
+    bool shown = true;
+    const float *M = SCENE ? scene_transform(F, triObj, K, view, tri, shown) : sM;
     float x[3], y[3], z[3];
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
@@ -637,7 +655,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
         x[k] = sv[mi * 9 + k * 3 + 0];
         y[k] = sv[mi * 9 + k * 3 + 1];
         z[k] = sv[mi * 9 + k * 3 + 2];
-        if (F.views) view_point(sM, x[k], y[k], z[k]);
+        if (SCENE || F.views) view_point(M, x[k], y[k], z[k]);
         project_vertex(F.proj, x[k], y[k], z[k]);
     }
 
@@ -654,7 +672,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
     int yt = clipi(ceil_to_int_ref(fyt), 0, F.H), yb = clipi(ceil_to_int_ref(fyb), 0, F.H);
     yt = max(yt, F.row0);  // band sharding: rows outside [row0,row1) belong to another filler
     yb = min(yb, F.row1);
-    bool drawn = valid && (xl < xr) && (yt < yb);  // pyx:209-211 and the empty range() cases
+    bool drawn = valid && shown && (xl < xr) && (yt < yb);  // pyx:209-211 and the empty range() cases
     if (banded) {
         if (!__syncthreads_or(drawn ? 1 : 0)) {
             if (threadIdx.x == 0) *alive = 0;
@@ -671,10 +689,10 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
     if (banded && valid) {
         const float *q = sn + mi * 9;
         float z0 = q[2], z1 = q[5], z2 = q[8];
-        if (F.views) {
-            z0 = (sM[6] * q[0] + sM[7] * q[1]) + sM[8] * q[2];
-            z1 = (sM[6] * q[3] + sM[7] * q[4]) + sM[8] * q[5];
-            z2 = (sM[6] * q[6] + sM[7] * q[7]) + sM[8] * q[8];
+        if (SCENE || F.views) {
+            z0 = (M[6] * q[0] + M[7] * q[1]) + M[8] * q[2];
+            z1 = (M[6] * q[3] + M[7] * q[4]) + M[8] * q[5];
+            z2 = (M[6] * q[6] + M[7] * q[7]) + M[8] * q[8];
         }
         drawn = drawn && !(((z0 + z1) + z2) >= 0.0f);
     }
@@ -740,7 +758,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
         nx[k] = sn[mi * 9 + k * 3 + 0];
         ny[k] = sn[mi * 9 + k * 3 + 1];
         nz[k] = sn[mi * 9 + k * 3 + 2];
-        if (F.views) view_normal(sM, nx[k], ny[k], nz[k]);
+        if (SCENE || F.views) view_normal(M, nx[k], ny[k], nz[k]);
     }
     R[S_N0] = make_float4(nx[0], ny[0], nz[0], nx[1]);
     R[S_N1] = make_float4(ny[1], nz[1], nx[2], ny[2]);
@@ -751,7 +769,7 @@ __device__ __forceinline__ void setup_chunk(const Frame &F, const int view, cons
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             const float *p = sv + mi * 9 + k * 3;
-            const float zc = F.views ? ((sM[6] * (p[0] - sM[9]) + sM[7] * (p[1] - sM[10])) + sM[8] * (p[2] - sM[11])) + sM[14] : p[2];
+            const float zc = (SCENE || F.views) ? ((M[6] * (p[0] - M[9]) + M[7] * (p[1] - M[10])) + M[8] * (p[2] - M[11])) + M[14] : p[2];
             const float w = 1.0f / zc;
             t[3 * k] = q[3 * k] * w; t[3 * k + 1] = q[3 * k + 1] * w; t[3 * k + 2] = w;
         }
@@ -796,8 +814,8 @@ constexpr int SETUP_MIN_CTAS = 3;
 constexpr int SETUP_STAGES = 2;
 constexpr size_t SETUP_STAGE_FLOATS = 3 * (size_t)NT * 9;
 constexpr size_t SETUP_DYN_SMEM = SETUP_STAGES * SETUP_STAGE_FLOATS * sizeof(float);
-template <bool PERSP>
-__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
+template <bool PERSP, bool SCENE>
+__device__ __forceinline__ void setup_items(const Frame &F, const int *triObj, const int K)
 {
     extern __shared__ __align__(128) float stg[];          // [SETUP_STAGES][3][NT * 9]
     __shared__ __align__(8) unsigned long long bar[SETUP_STAGES];
@@ -835,8 +853,8 @@ __global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
             if ((long long)blockIdx.x + (long long)s * gridDim.x < nItems) issue((long long)blockIdx.x + (long long)s * gridDim.x, s);
     }
     __syncthreads();
-    unsigned uses = 0;                                  // bit s: parity of the bulk-loaded items stage s has delivered so far
     int i = 0;
+    unsigned uses = 0;                                  // bit s: parity of the bulk-loaded items stage s has delivered so far
     for (long long w = blockIdx.x; w < nItems; w += gridDim.x, ++i) {
         const int s = i % SETUP_STAGES;
         int view;
@@ -847,11 +865,23 @@ __global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
             uses ^= 1u << s;
         }
         float *d = stg + (size_t)s * SETUP_STAGE_FLOATS;
-        setup_chunk<PERSP>(F, view, chunk, chunksPerView, d, d + NT * 9, d + 2 * NT * 9, sM, slist, wsum, staged);
+        setup_chunk<PERSP, SCENE>(F, view, chunk, chunksPerView, d, d + NT * 9, d + 2 * NT * 9, sM, slist, wsum, staged, triObj, K);
         __syncthreads();                                // everybody is done with the stage (and with sM / slist / wsum)
         const long long w2 = w + (long long)SETUP_STAGES * gridDim.x;
         if (threadIdx.x == 0 && w2 < nItems) issue(w2, s);
     }
+}
+template <bool PERSP>
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
+{
+    setup_items<PERSP, false>(F, nullptr, 0);
+}
+// The scene instantiations (crb_render_scene_views): F.views is [nViews, K, 16], triObj [T] names each triangle's object.  Both
+// are parameters of their own, so that Frame, every kernel's parameter block, does not grow.
+template <bool PERSP>
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_scene(const Frame F, const int *triObj, const int K)
+{
+    setup_items<PERSP, true>(F, triObj, K);
 }
 
 // ---- CRB_CLIP_NEAR (crender_b200.h, DESIGN 2) ---------------------------------------------------------------------------
@@ -860,34 +890,40 @@ __global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup(const Frame F)
 // counts), so every kernel behind it runs unchanged, and the visibility key's index is the rule's tie order 2t + h.
 
 // Corner k of real triangle r (staged in shared memory) in camera space: position (view_point), normal (view_normal), colour.
-__device__ __forceinline__ void clip_corner(const Frame &F, const float *sM, const float *sv, const float *sn, const float *sc, int r,
+// M: the view's transform (staged in shared memory), or in a scene frame the triangle's own (scene_transform).
+template <bool SCENE>
+__device__ __forceinline__ void clip_corner(const Frame &F, const float *M, const float *sv, const float *sn, const float *sc, int r,
                                             int k, float a[9])
 {
     const int o = r * 9 + k * 3;
     a[0] = sv[o]; a[1] = sv[o + 1]; a[2] = sv[o + 2];
     a[3] = sn[o]; a[4] = sn[o + 1]; a[5] = sn[o + 2];
     a[6] = sc[o]; a[7] = sc[o + 1]; a[8] = sc[o + 2];
-    if (F.views) {
-        view_point(sM, a[0], a[1], a[2]);
-        view_normal(sM, a[3], a[4], a[5]);
+    if (SCENE || F.views) {
+        view_point(M, a[0], a[1], a[2]);
+        view_normal(M, a[3], a[4], a[5]);
     }
 }
 
-// Item `chunk` of view `view`: NT virtual triangles = NT / 2 real ones, staged by the threads (stage_floats).
-template <bool PERSP>
+// Item `chunk` of view `view`: NT virtual triangles = NT / 2 real ones, staged by the threads (stage_floats).  SCENE: as in
+// setup_chunk, each thread's real triangle takes its own transform, and a hidden one has no pieces.
+template <bool PERSP, bool SCENE>
 __device__ __forceinline__ void setup_chunk_clip(const Frame &F, const float zn, const int view, const long long chunk,
-                                                 const long long chunksPerView, float *sv, float *sn, float *sc, float *sM, unsigned *wsum)
+                                                 const long long chunksPerView, float *sv, float *sn, float *sc, float *sM, unsigned *wsum,
+                                                 const int *triObj, const int K)
 {
     const long long first = chunk * NT;                       // first virtual triangle (F.T is even, so cnt is too)
     const long long cnt = min((long long)NT, F.T - first);
     stage_floats(F.v, first / 2 * 9, cnt / 2 * 9, sv);
     stage_floats(F.n, first / 2 * 9, cnt / 2 * 9, sn);
     stage_floats(F.c, first / 2 * 9, cnt / 2 * 9, sc);
-    if (F.views && threadIdx.x < 16) sM[threadIdx.x] = F.views[view * 16 + threadIdx.x];
+    if (!SCENE && F.views && threadIdx.x < 16) sM[threadIdx.x] = F.views[view * 16 + threadIdx.x];
     __syncthreads();
     const int me = (int)threadIdx.x;
     const bool valid = me < cnt;
     const int r = valid ? me >> 1 : 0, h = me & 1;
+    bool shown = true;
+    const float *M = SCENE ? scene_transform(F, triObj, K, view, first / 2 + r, shown) : sM;
 
     // The polygon, corner j in bits 4j..4j+3 as (i | o << 2): corner i itself if o == i, else the crossing point I(i, o)
     bool in[3];
@@ -895,7 +931,7 @@ __device__ __forceinline__ void setup_chunk_clip(const Frame &F, const float zn,
     for (int k = 0; k < 3; ++k) {
         const int o = r * 9 + k * 3;
         float x = sv[o], y = sv[o + 1], z = sv[o + 2];
-        if (F.views) view_point(sM, x, y, z);
+        if (SCENE || F.views) view_point(M, x, y, z);
         in[k] = z >= zn;                                      // NaN: outside
     }
     unsigned poly = 0;
@@ -910,17 +946,17 @@ __device__ __forceinline__ void setup_chunk_clip(const Frame &F, const float zn,
         }
     }
     // piece 0 = (p0, p1, p2), piece 1 = (p0, p2, p3), present with 3 or 4 corners (piece 1: 4 only)
-    const bool present = valid && (h == 0 ? np >= 3 : np == 4);
+    const bool present = valid && shown && (h == 0 ? np >= 3 : np == 4);
     float x[3], y[3], z[3], zc[3], nx[3], ny[3], nz[3], q[9];
 #pragma unroll
     for (int m = 0; m < 3; ++m) {
         const int j = (m == 0 || h == 0) ? m : m + 1;
         const int i = (poly >> (4 * j)) & 3u, o = (poly >> (4 * j + 2)) & 3u;
         float A[9];
-        clip_corner(F, sM, sv, sn, sc, r, i, A);
+        clip_corner<SCENE>(F, M, sv, sn, sc, r, i, A);
         if (o != i) {
             float B[9];
-            clip_corner(F, sM, sv, sn, sc, r, o, B);
+            clip_corner<SCENE>(F, M, sv, sn, sc, r, o, B);
             const float s = (zn - A[2]) / (B[2] - A[2]);
 #pragma unroll
             for (int k = 0; k < 9; ++k) A[k] = A[k] + s * (B[k] - A[k]);
@@ -1008,8 +1044,8 @@ __device__ __forceinline__ void setup_chunk_clip(const Frame &F, const float zn,
 
 // The clip instantiations of k_setup: a few CTAs per SM walk the (view, item) work items.  zn = F(z_near) is a parameter of its
 // own, so that Frame, every kernel's parameter block, does not grow.
-template <bool PERSP>
-__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_clip(const Frame F, const float zn)
+template <bool PERSP, bool SCENE>
+__device__ __forceinline__ void setup_items_clip(const Frame &F, const float zn, const int *triObj, const int K)
 {
     __shared__ __align__(16) float sv[NT / 2 * 9];
     __shared__ __align__(16) float sn[NT / 2 * 9];
@@ -1022,9 +1058,19 @@ __global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_clip(const Frame F
     const long long chunksPerView = (F.T + NT - 1) / NT;
     const long long nItems = chunksPerView * F.nViews;
     for (long long w = blockIdx.x; w < nItems; w += gridDim.x) {
-        setup_chunk_clip<PERSP>(F, zn, (int)(w / chunksPerView), w % chunksPerView, chunksPerView, sv, sn, sc, sM, wsum);
+        setup_chunk_clip<PERSP, SCENE>(F, zn, (int)(w / chunksPerView), w % chunksPerView, chunksPerView, sv, sn, sc, sM, wsum, triObj, K);
         __syncthreads();                                // everybody is done with the staged arrays (and with sM / wsum)
     }
+}
+template <bool PERSP>
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_clip(const Frame F, const float zn)
+{
+    setup_items_clip<PERSP, false>(F, zn, nullptr, 0);
+}
+template <bool PERSP>
+__global__ void __launch_bounds__(NT, SETUP_MIN_CTAS) k_setup_clip_scene(const Frame F, const float zn, const int *triObj, const int K)
+{
+    setup_items_clip<PERSP, true>(F, zn, triObj, K);
 }
 
 // Band-sharded fillers (SURVEY 8e) see every triangle of the frame but draw only those that reach their rows.  This
@@ -2668,18 +2714,32 @@ int setup_smem_attr(int device)
     if (device >= 0 && device < 64 && done[device]) return CRB_OK;
     CU(cudaFuncSetAttribute(k_setup<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
     CU(cudaFuncSetAttribute(k_setup<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
+    CU(cudaFuncSetAttribute(k_setup_scene<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
+    CU(cudaFuncSetAttribute(k_setup_scene<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SETUP_DYN_SMEM));
     if (device >= 0 && device < 64) done[device] = true;
     return CRB_OK;
 }
 
+// The objects of a scene frame (crb_render_scene_views): triObj [T] on the device and K >= 1 of them.  K = 0 in every other frame.
+struct Scene {
+    const int *triObj = nullptr;
+    int K = 0;
+};
+
 // k_setup with `grid` CTAs; CRB_TEX_PERSPECTIVE frames write the perspective-correct texture coordinates into the records,
-// CRB_CLIP_NEAR frames (F.T = 2T pieces) clip at zn = F(z_near) first
-void launch_setup(const crb_filler *f, const Frame &F, unsigned grid, cudaStream_t st)
+// CRB_CLIP_NEAR frames (F.T = 2T pieces) clip at zn = F(z_near) first, scene frames take each triangle's object transform
+void launch_setup(const crb_filler *f, const Frame &F, unsigned grid, cudaStream_t st, const Scene &sc = Scene())
 {
     const bool persp = (F.flags & CRB_TEX_PERSPECTIVE) != 0;
     if (F.flags & CRB_CLIP_NEAR) {
-        if (persp) k_setup_clip<true><<<grid, NT, 0, st>>>(F, f->z_near);
+        if (sc.K) {
+            if (persp) k_setup_clip_scene<true><<<grid, NT, 0, st>>>(F, f->z_near, sc.triObj, sc.K);
+            else k_setup_clip_scene<false><<<grid, NT, 0, st>>>(F, f->z_near, sc.triObj, sc.K);
+        } else if (persp) k_setup_clip<true><<<grid, NT, 0, st>>>(F, f->z_near);
         else k_setup_clip<false><<<grid, NT, 0, st>>>(F, f->z_near);
+    } else if (sc.K) {
+        if (persp) k_setup_scene<true><<<grid, NT, SETUP_DYN_SMEM, st>>>(F, sc.triObj, sc.K);
+        else k_setup_scene<false><<<grid, NT, SETUP_DYN_SMEM, st>>>(F, sc.triObj, sc.K);
     } else if (persp) k_setup<true><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
     else k_setup<false><<<grid, NT, SETUP_DYN_SMEM, st>>>(F);
 }
@@ -2687,7 +2747,7 @@ void launch_setup(const crb_filler *f, const Frame &F, unsigned grid, cudaStream
 constexpr int PREPASS_EIGHTHS = 5;  // the band pre-pass runs for bands of at most this many eighths of the frame (half-frame bands gain
                                     // 7 %; a cut balanced by measurement lands a few strips off the middle, which must not switch it off)
 // project/setup/count -> alloc -> fill for up to maxViews views
-int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
+int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0, const Scene &sc = Scene())
 {
     int rc;
     // Triangles that span many tiles get a kernel of their own (k_fill_wide) -- but only where there are any: the launch is
@@ -2722,7 +2782,7 @@ int run_prep(crb_filler *f, Frame &F, cudaStream_t st, int slot = 0)
     if (F.T > 0) {
         if ((rc = setup_smem_attr(f->device))) return rc;
         const long long items = F.chunks ? (long long)gT : (long long)gT * F.nViews;
-        launch_setup(f, F, (unsigned)min(items, (long long)f->sm_count * SETUP_MIN_CTAS), st);
+        launch_setup(f, F, (unsigned)min(items, (long long)f->sm_count * SETUP_MIN_CTAS), st, sc);
         if ((rc = launch_check(f, "k_setup"))) return rc;
     } else {
         CU(cudaMemsetAsync(F.total, 0, 8, st));
@@ -2858,9 +2918,9 @@ int run_raster(crb_filler *f, FrameIds &F, cudaStream_t st, int slot)
     return CRB_OK;
 }
 
-int run_tiled(crb_filler *f, FrameIds &F, cudaStream_t st, int slot = 0)
+int run_tiled(crb_filler *f, FrameIds &F, cudaStream_t st, int slot = 0, const Scene &sc = Scene())
 {
-    int rc = run_prep(f, F, st, slot);
+    int rc = run_prep(f, F, st, slot, sc);
     return rc ? rc : run_raster(f, F, st, slot);
 }
 
@@ -3608,9 +3668,10 @@ int crb_render_views(crb_filler *f, const float *v, const float *c, const float 
                                 flags, light, stream);
 }
 
-int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views,
-                         int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
-                         int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream)
+// crb_render_views_ids (sc.K == 0: views [n_views,16]) and crb_render_scene_views (views [n_views,K,16], one per object)
+static int render_views(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views,
+                        int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
+                        int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream, const Scene &sc)
 {
     if (check_filler(f)) return CRB_ERR_INVALID;
     if (n_views < 0) return fail(CRB_ERR_INVALID, "negative size");
@@ -3666,7 +3727,7 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
         F.T = T << F.idShift; F.nViews = (n_views - v0 < f->maxViews) ? n_views - v0 : f->maxViews;
         F.flags = (flags & (CRB_GURO | CRB_TEX_FLAGS | CRB_SS_FLAGS | CRB_CLIP_NEAR)) | CRB_CLEAR_FIRST;
         F.v = v; F.c = c; F.n = n;
-        F.views = views ? views + (size_t)v0 * 16 : nullptr;
+        F.views = views ? views + (size_t)v0 * (sc.K ? sc.K : 1) * 16 : nullptr;
         F.z = z_out ? z_out + (size_t)v0 * slab : nullptr;
         F.color = color_out ? color_out + (size_t)v0 * slab * 3 : nullptr;
         F.normals = normals_out ? normals_out + (size_t)v0 * slab * 3 : nullptr;
@@ -3679,12 +3740,12 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
         if (light) { F.light[0] = light[0]; F.light[1] = light[1]; F.light[2] = light[2]; }
         int rc;
         if (!pipe) {
-            rc = run_tiled(f, F, user, i);
+            rc = run_tiled(f, F, user, i, sc);
             if (rc) return rc;
             continue;
         }
         if (f->set_used[set]) CU(cudaStreamWaitEvent(f->s_prep, f->ev_raster[set], 0));   // the set's previous frame has been rasterized
-        if ((rc = run_prep(f, F, f->s_prep, i))) return rc;
+        if ((rc = run_prep(f, F, f->s_prep, i, sc))) return rc;
         CU(cudaEventRecord(f->ev_fill[set], f->s_prep));
         CU(cudaStreamWaitEvent(f->s_raster, f->ev_fill[set], 0));
         if ((rc = run_raster(f, F, f->s_raster, i))) return rc;
@@ -3697,6 +3758,34 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
         if (!defer) return join_pending(f, user);
     }
     return CRB_OK;
+}
+
+int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const float *views,
+                         int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
+                         int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream)
+{
+    return render_views(f, v, c, n, T, views, n_views, z_out, color_out, normals_out, color_u8_out, tri_id_out, bary_out, flags,
+                        light, stream, Scene());
+}
+
+int crb_render_scene_views(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const int32_t *tri_obj,
+                           int n_objects, const float *views, int n_views, float *z_out, float *color_out, float *normals_out,
+                           uint8_t *color_u8_out, int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3],
+                           void *stream)
+{
+    if (check_filler(f)) return CRB_ERR_INVALID;
+    if (n_objects < 1) return fail(CRB_ERR_INVALID, "n_objects must be >= 1, got %d", n_objects);
+    if (!views || !tri_obj) return fail(CRB_ERR_INVALID, "a scene needs views and tri_obj");
+    if ((reinterpret_cast<uintptr_t>(views) | reinterpret_cast<uintptr_t>(tri_obj)) & 3u)
+        return fail(CRB_ERR_INVALID, "views and tri_obj must be 4-byte aligned");
+    if (flags & CRB_PATH_ATOMIC) return fail(CRB_ERR_INVALID, "CRB_PATH_ATOMIC supports single-view renders only");
+    if (n_views > 0 && (uint64_t)n_objects > (uint64_t)(PTRDIFF_MAX / 64) / (uint64_t)n_views)
+        return fail(CRB_ERR_INVALID, "views of %d x %d transforms are not addressable", n_views, n_objects);
+    Scene sc;
+    sc.triObj = tri_obj;
+    sc.K = n_objects;
+    return render_views(f, v, c, n, T, views, n_views, z_out, color_out, normals_out, color_u8_out, tri_id_out, bary_out, flags,
+                        light, stream, sc);
 }
 
 int crb_set_u8_exchange(crb_filler *f, int n_bands, int rows_per_band, void *const *band_base)

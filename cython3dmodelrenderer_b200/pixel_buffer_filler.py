@@ -703,7 +703,7 @@ class AdvancedPixelBufferFiller:
 
     def render_views(self, v, c, n, views, z_out=None, color_out=None, normals_out=None, color_u8_out=None,
                      want=None, guro_light=None, chunk=32, check_status=True, defer_join=False,
-                     u8_exchange=None, texture=None, triangle_id_out=None, barycentrics_out=None, supersample=1):
+                     u8_exchange=None, texture=None, triangle_id_out=None, barycentrics_out=None, supersample=1, objects=None):
         """Batched multi-view render (config C5): every view gets fresh-filler buffers in its own slab.
 
         v, c, n: torch CUDA float32 [T,3,3] (device-resident base mesh);  views: [V,16] float32 (numpy or CUDA tensor,
@@ -724,8 +724,14 @@ class AdvancedPixelBufferFiller:
         resolved into one pixel of color_u8 [V, rows/s, w/s, 3] inside the rasterizer (CRB_SS2 / CRB_SS4, DESIGN 2).  The
         uint8 image is then the only output: `want` names none (its default is then empty) and color_u8_out is True or such a
         tensor.
+        `objects` (int32 [T], NumPy or torch): a scene whose objects move independently (crb_render_scene_views, DESIGN 2).
+        Triangle t belongs to object objects[t], and `views` is then [V,K,16]: entry [v,k] is object k's transform in view v
+        (views.scene_views composes a camera with object poses).  A non-zero pad (entry 15) hides the object in that view; a
+        triangle whose object is outside [0, K) draws nothing.  Every other keyword composes; tri_id still indexes the base
+        mesh, so objects[tri_id] is the object of a pixel.
         `want` defaults to ("z", "color", "normals").  Returns a dict of the produced tensors."""
         torch = self._torch
+        objects = self._check_scene(views, objects)
         ss = _check_supersample(supersample)
         if want is None:
             want = ("z", "color", "normals") if ss == 1 else ()
@@ -742,6 +748,10 @@ class AdvancedPixelBufferFiller:
                 raise ValueError("render_views needs CUDA float32 tensors of shape [T,3,3]")
         v, c, n = v.contiguous(), c.contiguous(), n.contiguous()
         T = v.shape[0]
+        if objects is not None:
+            if tuple(objects.shape) != (T,):
+                raise ValueError(f"objects must have one entry per triangle, [{T}], got {list(objects.shape)}")
+            objects = (objects if isinstance(objects, torch.Tensor) else torch.from_numpy(objects)).to(self._dev).contiguous()
         if not isinstance(views, torch.Tensor):
             views = torch.from_numpy(np.ascontiguousarray(views, dtype=np.float32)).to(self._dev)
         views = views.contiguous()
@@ -784,7 +794,7 @@ class AdvancedPixelBufferFiller:
             flags |= _lib.CRB_DEFER_JOIN
             # the front end may still be queued on the filler's internal stream when this call returns: torch's allocator orders
             # the reuse of freed memory on the CALLER's stream only, so temporaries made above stay referenced until join()
-            self._deferred_keep = (views, v, c, n)
+            self._deferred_keep = (views, v, c, n, objects)
         self._ensure_workspace(T, views=min(int(chunk), max(V, 1)))
         ptr = lambda t: None if t is None else t.data_ptr()
         if u8_exchange is not None:
@@ -795,10 +805,27 @@ class AdvancedPixelBufferFiller:
             check(self._L.crb_set_u8_exchange(self._handle, len(bases), int(hb), arr))
         try:
             return self._render_views_loop(v, c, n, T, views, V, z_out, color_out, normals_out, color_u8_out, flags, light,
-                                           check_status, out, ptr, triangle_id_out, barycentrics_out)
+                                           check_status, out, ptr, triangle_id_out, barycentrics_out, objects)
         finally:
             if u8_exchange is not None:
                 check(self._L.crb_set_u8_exchange(self._handle, 0, 0, None))
+
+    def _check_scene(self, views, objects):
+        """render_views' `views` and `objects`: [V,16] without objects, [V,K,16] (K >= 1) with an int32 [T] array or tensor
+        (returned as given, a NumPy array if it was not a tensor); misuse raises ValueError before anything is queued.  (The
+        length of objects is checked against T by the caller.)"""
+        torch = self._torch
+        if objects is not None:
+            if not isinstance(objects, torch.Tensor):
+                objects = np.asarray(objects)
+            if objects.dtype not in (np.int32, torch.int32) or len(objects.shape) != 1:
+                raise ValueError(f"objects must be an int32 [T] array or tensor, got {objects.dtype} {list(objects.shape)}")
+        shape = tuple(views.shape) if isinstance(views, torch.Tensor) else np.shape(views)
+        if objects is not None and (len(shape) != 3 or shape[2] != 16 or shape[1] < 1):
+            raise ValueError(f"with objects, views must be [V,K,16] with K >= 1, got {list(shape)}")
+        if objects is None and len(shape) == 3:
+            raise ValueError(f"views of shape {list(shape)} are per object: pass objects= (the object of each triangle)")
+        return objects
 
     def _check_supersampled_views(self, ss, want, color_u8_out, u8_exchange, outputs):
         """What crb_render_views refuses with CRB_SS2 / CRB_SS4, raised as ValueError before anything is queued."""
@@ -816,9 +843,14 @@ class AdvancedPixelBufferFiller:
             raise ValueError(f"supersample={ss} needs a filler size that is a multiple of {ss}, got {self.h} x {self.w}")
 
     def _render_views_loop(self, v, c, n, T, views, V, z_out, color_out, normals_out, color_u8_out, flags, light, check_status,
-                           out, ptr, tri_id_out=None, bary_out=None):
+                           out, ptr, tri_id_out=None, bary_out=None, objects=None):
         while True:
-            if tri_id_out is None and bary_out is None:
+            if objects is not None:
+                check(self._L.crb_render_scene_views(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, objects.data_ptr(),
+                                                     views.shape[1], views.data_ptr(), V, ptr(z_out), ptr(color_out),
+                                                     ptr(normals_out), ptr(color_u8_out), ptr(tri_id_out), ptr(bary_out), flags,
+                                                     light, self._stream()))
+            elif tri_id_out is None and bary_out is None:
                 check(self._L.crb_render_views(self._handle, v.data_ptr(), c.data_ptr(), n.data_ptr(), T, views.data_ptr(), V,
                                                ptr(z_out), ptr(color_out), ptr(normals_out), ptr(color_u8_out), flags, light,
                                                self._stream()))

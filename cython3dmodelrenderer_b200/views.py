@@ -49,3 +49,35 @@ def transform_arrays_host(view, v, n):
         vo[..., r] = ((M[3 * r] * d[0] + M[3 * r + 1] * d[1]) + M[3 * r + 2] * d[2]) + M[12 + r]
         no[..., r] = (M[3 * r] * n[..., 0] + M[3 * r + 1] * n[..., 1]) + M[3 * r + 2] * n[..., 2]
     return vo, no
+
+
+def scene_views(camera, poses):
+    """Per-object transforms of a scene (render_views(objects=...)): [V,K,16] float32, entry [v,k] = camera[v] after pose k.
+
+    camera: [V,16] views, poses: [K,16] (the same poses in every view) or [V,K,16], both in the {R, p, q, pad} format.  A pose
+    x -> Ro (x - po) + qo followed by the camera y -> Rc (y - pc) + qc is x -> Rc Ro (x - po) + (Rc (qo - pc) + qc), so the
+    composition is R = Rc Ro, p = po, q = Rc (qo - pc) + qc, computed in float64 and rounded to float32 once.  The pose's pad is
+    carried through: a pose with a non-zero pad hides its object in that view."""
+    cam = np.asarray(camera, dtype=np.float64).reshape(-1, 16)
+    V = cam.shape[0]
+    pos = np.asarray(poses, dtype=np.float64)
+    pos = np.broadcast_to(pos.reshape(1, -1, 16) if pos.ndim == 2 else pos, (V, pos.shape[-2], 16))
+    Rc = cam[:, None, :9].reshape(V, 1, 3, 3)
+    Ro = pos[..., :9].reshape(V, -1, 3, 3)
+    out = np.empty(pos.shape, np.float64)
+    out[..., :9] = (Rc @ Ro).reshape(V, -1, 9)
+    out[..., 9:12] = pos[..., 9:12]
+    out[..., 12:15] = (Rc @ (pos[..., 12:15] - cam[:, None, 9:12])[..., None])[..., 0] + cam[:, None, 12:15]
+    out[..., 15] = pos[..., 15]
+    return out.astype(np.float32)
+
+
+def concat_meshes(meshes):
+    """One base mesh of several objects: [(v, c, n), ...] of [T_k,3,3] float32 arrays -> (v, c, n, tri_obj), the arrays
+    concatenated in the given order and tri_obj int32 [sum T_k], k for the triangles of mesh k."""
+    if not meshes:
+        raise ValueError("concat_meshes needs at least one mesh")
+    v, c, n = (np.ascontiguousarray(np.concatenate([np.asarray(m[i], np.float32).reshape(-1, 3, 3) for m in meshes]))
+               for i in range(3))
+    tri_obj = np.concatenate([np.full(len(np.asarray(m[0]).reshape(-1, 9)), k, np.int32) for k, m in enumerate(meshes)])
+    return v, c, n, tri_obj

@@ -354,6 +354,35 @@ int crb_render_views_ids(crb_filler *f, const float *v, const float *c, const fl
                          int n_views, float *z_out, float *color_out, float *normals_out, uint8_t *color_u8_out,
                          int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3], void *stream);
 
+/* ---- scenes in batched views: a pose per object and view (an extension) ---------------------------------------------------
+ * The rule (DESIGN 2 states it word for word the same):
+ *   - Inputs: the base mesh v, c, n [T,3,3] as crb_render_views takes it; tri_obj: DEVICE int32 [T], the object of each
+ *     triangle; n_objects = K >= 1; views: DEVICE float32 [n_views, K, 16].  Entry [v, k] has crb_render_views' format
+ *     {R (9), p (3), q (3), pad}.
+ *   - Definition by composition.  In view v, triangle t with k = tri_obj[t] is transformed by views[v, k] exactly as
+ *     crb_render_views transforms it by views[v]: positions through view_point, normals through view_normal, the same float32
+ *     expressions, one rounding per operation, no FMA.  The camera-space triangles are then rendered exactly as in
+ *     crb_render_views, in base-mesh order, so the tie rule's "higher index wins" still reads t.  This covers the cull of
+ *     pyx:202-204 on the transformed normals, CRB_TEX_PERSPECTIVE's w = 1 / (camera z of the object's transform), the
+ *     CRB_CLIP_NEAR pieces 2t + h, CRB_GURO, every texture filter, interpolation and wrap mode, CRB_SS2 / CRB_SS4, band
+ *     fillers, the row exchange, the launch pipeline and CRB_DEFER_JOIN.
+ *   - Hidden objects.  If views[v, k, 15] (the pad) is neither +0 nor -0, object k is hidden in view v and its triangles draw
+ *     nothing there; NaN also hides.  A triangle whose tri_obj lies outside [0, K) draws nothing in any view.  Dropping
+ *     triangles does not change the relative order of the others.
+ *   - Id outputs: tri_id is the base-mesh index t (base 0), as for crb_render_views_ids.  The object of a pixel is
+ *     tri_obj[tri_id].
+ *   - Equivalences: with K = 1 and tri_obj all 0 a scene call is crb_render_views_ids bit for bit, in every output; with every
+ *     views[v, k] equal to one views[v] it is crb_render_views_ids of the same mesh.
+ *   - Normals go through R with no inverse-transpose; a non-rigid R is treated exactly as crb_render_views treats it.
+ *   - CRB_ERR_INVALID: K < 1; views or tri_obj NULL or not 4-byte aligned; CRB_PATH_ATOMIC; n_views * K * 16 floats not
+ *     addressable; and every refusal of crb_render_views_ids.
+ *   - Workspace: as crb_render_views with T triangles (2T with CRB_CLIP_NEAR).  A frame that overflows the pair list leaves
+ *     every output untouched. */
+int crb_render_scene_views(crb_filler *f, const float *v, const float *c, const float *n, int64_t T, const int32_t *tri_obj,
+                           int n_objects, const float *views, int n_views, float *z_out, float *color_out, float *normals_out,
+                           uint8_t *color_u8_out, int32_t *tri_id_out, float *bary_out, unsigned flags, const float light[3],
+                           void *stream);
+
 /* Row exchange of the uint8 image (SURVEY 8e, config C5 "view-sharded ... with NCCL gather"; no reference counterpart --
  * run.py is one process).  While n_bands > 0, crb_render_views writes run.py:26's flipped uint8 image of its views NOT into
  * color_u8_out (pass NULL there) but row band by row band into other GPUs' memory, from inside the rasterizer: image row r
